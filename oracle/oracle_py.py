@@ -178,7 +178,13 @@ class Oracle:
         return self._solve(self.L.aar_oracle_track_port, z0, max_trace)
 
     def track_ref(self, z0, max_trace=64):
+        """MultiCamMapper::track() driving the unmodified reference sparselevmarq.h (ref build only)."""
+        if not self.is_ref:
+            raise RuntimeError("reference SLM build (oracle/_ref) not available")
         return self._solve(self.L.aar_oracle_track_ref, z0, max_trace)
+
+    def track(self, z0, max_trace=64):
+        return self.track_ref(z0, max_trace) if self.is_ref else self.track_port(z0, max_trace)
 
     def time_ref_steps(self, z0, iters):
         z = np.ascontiguousarray(z0, dtype=np.float64)
