@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstring>
 #include <dlfcn.h>
+#include <limits>
 #include <unistd.h>
 #include <map>
 #include <memory>
@@ -24,6 +25,7 @@
 #include "../../include/aar_cuda.h"
 #include "aar_host_math.h"
 #include "aar_kernels.cuh"
+#include "aar_report.cuh"
 
 using namespace aar;
 
@@ -88,6 +90,7 @@ struct aar_problem {
     // ---- row map (global, a1 order) and shard
     long long N = 0;                               // global observations
     std::vector<int> g_frame, g_cam, g_marker, g_hasjac; // indices per global observation
+    long long num_det = 0; std::vector<long long> g_det;  // desc->num_detections; index into desc->det_* of every global observation (aar_error_report)
     int f_begin = 0, f_end = 0;                    // this rank's frame index range
     long long o_begin = 0, o_end = 0;              // this rank's observation range
     int nrc = 0, nrm = 0, nri = 0, n_r = 0; bool opt_i = false;   // nri: 2 C intrinsics pseudo-blocks (aar_intrinsics.cuh)
@@ -133,6 +136,8 @@ struct aar_problem {
     cudaGraph_t lm_graph = nullptr; cudaGraphExec_t lm_exec = nullptr; cudaGraphConditionalHandle lm_outer = 0, lm_inner = 0; cudaStream_t lm_side = nullptr;
     bool lm_graph_tried = false, lm_graph_ok = false, capturing = false; long long lm_graph_launches = 0, lm_graph_iters = 0; int lm_body_launches = 0, lm_try_launches = 0;
     DevBuf<LmTraceDev> d_trace;
+    // aar_error_report (aar_report.cuh): observation errors, entity statistics [C + M + F], select state [2 nq], digit histograms [nq][SEL_BINS]
+    DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
     // sharded handles: every rank's reduced system and decision scalars mapped through cudaIpc (aar_kernels.cuh: PeerDev)
     PeerDev pd; bool peer_ok = false; DevBuf<double> d_peer_small, d_Br_sum; DevBuf<int> d_peer_flags; std::vector<void *> ipc_opened;
     cudaEvent_t ev[16] = {}; double phase_ms[AAR_NUM_PHASES] = {};
@@ -207,14 +212,17 @@ int allreduce(aar_problem *p, double *buf, size_t n, ncclRedOp_t op) {
     return AAR_OK;
 }
 
-// residual sum of squares at dz into d_red3[0] (must be zeroed by the caller); optional residual vector
-int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_out) {
+// residual sum of squares at dz into d_red3[0] (must be zeroed by the caller); optional residual vector.
+// unweighted: without the Huber weights whatever the handle's setting (aar_error_report)
+int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_out, bool unweighted = false) {
+    DevProblem dq = p->dp;
+    if (unweighted) { dq.huber = 0; dq.st_dev = nullptr; }
     LAUNCH(p, k_expand_trial, cdiv((long long)p->C + p->M + p->dp.F, 128), 128, 0, p->dp, dz);
     if (p->opt_i) LAUNCH(p, k_expand_intr, cdiv(p->C, 64), 64, 0, p->dp, dz, p->d_intr_tr.p);
     if (p->dp.N > 0 && p->analytic)
-        LAUNCH(p, k_residual_an, cdiv(p->dp.N, 256), 256, 0, p->dp, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
+        LAUNCH(p, k_residual_an, cdiv(p->dp.N, 256), 256, 0, dq, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
     else if (p->dp.N > 0)
-        LAUNCH(p, k_residual, cdiv(p->dp.N, 256), 256, 0, p->dp, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
+        LAUNCH(p, k_residual, cdiv(p->dp.N, 256), 256, 0, dq, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
     return AAR_OK;
 }
 
@@ -763,6 +771,7 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
     CU(cudaStreamSynchronize(p->stream));
     cmark("undistortion, attributes, sync");
     aar_lm_default_params(&p->params);
+    p->num_det = nd; p->g_det = std::move(keep);
     guard.release();
     *out = p;
     return AAR_OK;
@@ -954,6 +963,88 @@ int aar_eval_residual(aar_problem *p, const double *z, float huber_delta, double
     CU(cudaStreamSynchronize(p->stream));
     CU(cudaGetLastError());
     if (sum_sq) *sum_sq = p->h_red3[0];
+    return AAR_OK;
+}
+
+int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out) {
+    if (!p || !z || !out) return AAR_ERR_INVALID;
+    if (p->world != 1) { set_err("aar_error_report: single-rank handles only"); return AAR_ERR_INVALID; }
+    if (p->lm_active) { set_err("aar_error_report between aar_lm_begin and aar_lm_end would overwrite the trial buffers of the resident loop"); return AAR_ERR_INVALID; }
+    const int nq = out->num_q;
+    if (nq < 0 || nq > SEL_MAX_Q || (nq > 0 && (!out->q || !out->q_value))) { set_err("aar_error_report: num_q must be in [0, %d] with q and q_value given", SEL_MAX_Q); return AAR_ERR_INVALID; }
+    for (int t = 0; t < nq; t++) if (!(out->q[t] >= 0.0 && out->q[t] <= 1.0)) { set_err("aar_error_report: q[%d] = %g is not in [0, 1]", t, out->q[t]); return AAR_ERR_INVALID; }
+    CU(cudaSetDevice(p->device));
+    const long long N = p->dp.N;
+    const size_t ne = (size_t)p->C + p->M + p->F;
+    int rc = upload_z(p, z, p->d_zt.p); if (rc) return rc;
+    if (p->d_r.n < 8 * (size_t)N) CU(p->d_r.alloc(std::max<size_t>(8 * (size_t)N, 8)));
+    if (p->d_rep_err.n < (size_t)N) CU(p->d_rep_err.alloc(std::max<size_t>((size_t)N, 1)));
+    if (p->d_rep_cnt.n < ne) { CU(p->d_rep_cnt.alloc(ne)); CU(p->d_rep_sum.alloc(ne)); CU(p->d_rep_max.alloc(ne)); }
+    CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
+    CU(cudaMemsetAsync(p->d_rep_cnt.p, 0, ne * sizeof(unsigned long long), p->stream));
+    CU(cudaMemsetAsync(p->d_rep_sum.p, 0, ne * sizeof(double), p->stream));
+    CU(cudaMemsetAsync(p->d_rep_max.p, 0, ne * sizeof(unsigned long long), p->stream));
+    if ((rc = residual(p, p->d_zt.p, 0.f, p->d_r.p, true))) return rc;
+    if (N > 0) {
+        const size_t msm = (size_t)p->M * 20;
+        const int marker_smem = msm + 4096 <= p->smem_optin;
+        if (marker_smem) CU(cudaFuncSetAttribute(k_report_obs, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
+        int per_sm = 1; CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_report_obs, REP_THREADS, marker_smem ? msm : 0));
+        const int grid = (int)std::min<long long>((long long)std::max(per_sm, 1) * p->num_sms, cdiv(N, REP_THREADS));
+        LAUNCH(p, k_report_obs, grid, REP_THREADS, marker_smem ? msm : 0, N, p->d_r.p, p->dp.obs_f, p->dp.obs_cm, p->C, p->M, p->f_begin, marker_smem,
+               p->d_rep_err.p, p->d_rep_cnt.p, p->d_rep_sum.p, p->d_rep_max.p);
+    }
+    // exact order statistics: ranks floor(q (n - 1)), ascending, share the digit passes
+    std::vector<int> order((size_t)nq);
+    std::vector<unsigned long long> sel(2 * (size_t)nq, 0);      // [prefix | rank] in rank order
+    if (nq > 0 && N > 0) {
+        std::iota(order.begin(), order.end(), 0);
+        auto rank_of_q = [&](int t) { return (unsigned long long)std::floor(out->q[t] * (double)(N - 1)); };
+        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return rank_of_q(a) < rank_of_q(b); });
+        for (int t = 0; t < nq; t++) sel[(size_t)nq + t] = rank_of_q(order[(size_t)t]);
+        if (p->d_sel.n < 2 * (size_t)nq) CU(p->d_sel.alloc(2 * (size_t)nq));
+        if (p->d_sel_hist.n < (size_t)nq * SEL_BINS) CU(p->d_sel_hist.alloc((size_t)nq * SEL_BINS));
+        CU(cudaMemcpyAsync(p->d_sel.p, sel.data(), sel.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaFuncSetAttribute(k_sel_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SEL_BINS * sizeof(unsigned))));
+        const auto *keys = reinterpret_cast<const unsigned long long *>(p->d_rep_err.p);
+        for (int pass = 0; pass < SEL_PASSES; pass++) {
+            const int smem_hist = pass == 0;                       // one histogram, most contended digit (sign, exponent)
+            CU(cudaMemsetAsync(p->d_sel_hist.p, 0, (size_t)(smem_hist ? 1 : nq) * SEL_BINS * sizeof(unsigned), p->stream));
+            int per_sm = 1; CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sel_hist, REP_THREADS, smem_hist ? SEL_BINS * sizeof(unsigned) : 0));
+            const int grid = (int)std::min<long long>((long long)std::max(per_sm, 1) * p->num_sms, cdiv(N, REP_THREADS));
+            LAUNCH(p, k_sel_hist, grid, REP_THREADS, smem_hist ? SEL_BINS * sizeof(unsigned) : 0, N, keys, pass, nq, p->d_sel.p, smem_hist, p->d_sel_hist.p);
+            LAUNCH(p, k_sel_pick, 1, REP_THREADS, 0, pass, nq, p->d_sel.p, p->d_sel.p + nq, p->d_sel_hist.p);
+        }
+        CU(cudaMemcpyAsync(sel.data(), p->d_sel.p, (size_t)nq * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    }
+    std::vector<unsigned long long> cnt(ne), mx(ne); std::vector<double> sum(ne), err(out->det_err ? (size_t)N : 0);
+    CU(cudaMemcpyAsync(cnt.data(), p->d_rep_cnt.p, ne * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CU(cudaMemcpyAsync(sum.data(), p->d_rep_sum.p, ne * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    CU(cudaMemcpyAsync(mx.data(), p->d_rep_max.p, ne * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    if (!err.empty()) CU(cudaMemcpyAsync(err.data(), p->d_rep_err.p, err.size() * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    CU(cudaMemcpyAsync(p->h_red3, p->d_red3.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    CU(cudaStreamSynchronize(p->stream));
+    CU(cudaGetLastError());
+    for (int t = 0; t < nq; t++) {
+        double v = std::numeric_limits<double>::quiet_NaN();
+        if (N > 0) std::memcpy(&v, &sel[(size_t)t], sizeof v);
+        out->q_value[order.empty() ? t : order[(size_t)t]] = v;
+    }
+    auto put = [&](size_t e0, size_t n, int64_t *c, double *s, double *m) {
+        for (size_t i = 0; i < n; i++) {
+            if (c) c[i] = (int64_t)cnt[e0 + i];
+            if (s) s[i] = sum[e0 + i];
+            if (m) std::memcpy(&m[i], &mx[e0 + i], sizeof(double));
+        }
+    };
+    put(0, (size_t)p->C, out->cam_count, out->cam_sum_sq, out->cam_max);
+    put((size_t)p->C, (size_t)p->M, out->marker_count, out->marker_sum_sq, out->marker_max);
+    put((size_t)p->C + p->M, (size_t)p->F, out->frame_count, out->frame_sum_sq, out->frame_max);
+    if (out->det_err) {
+        std::fill(out->det_err, out->det_err + p->num_det, std::numeric_limits<double>::quiet_NaN());
+        for (long long o = 0; o < N; o++) out->det_err[p->g_det[(size_t)o]] = err[(size_t)o];
+    }
+    out->num_observations = N; out->num_not_in_problem = p->num_det - N; out->sum_sq = p->h_red3[0];
     return AAR_OK;
 }
 

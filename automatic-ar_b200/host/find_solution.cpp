@@ -1,11 +1,13 @@
 // find_solution — the reference's app (/root/reference/apps/find_solution.cpp:28-181) on the CUDA path, OpenCV-free:
 //   find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>]
-//                 [-consensus-max <k>] [-init <initial.solution>] [-analytic]
+//                 [-consensus-max <k>] [-init <initial.solution>] [-analytic] [-reject-outliers <px>]
 // Reads <folder>/<cam>/calib.yml and <folder>/aruco.detections, builds the starting point with the Initializer (device: IPPE per
 // detection + consensus; include/aar_init.h), writes initial<suffix>.solution(.yaml), solves on the GPU (include/aar_cuda.h) and
 // writes final<suffix>.solution(.yaml) — the file names of find_solution.cpp:76-100.  Two additions: -consensus-max (SURVEY 8(f) row 3,
 // the reference's exhaustive consensus is O(n^2) in the number of co-observations) and -init (start from an existing .solution
-// instead of the detections) and -analytic (analytic Jacobian, residuals in double: include/aar_analytic.h; not the reference's arithmetic).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
+// instead of the detections) and -analytic (analytic Jacobian, residuals in double: include/aar_analytic.h; not the reference's arithmetic),
+// -reject-outliers <px> (after the solve, remove the detections whose reprojection error is above px and solve again with the same settings;
+// the final file holds the second solve).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -17,14 +19,14 @@
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic]" << std::endl;
+        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>]" << std::endl;
         return -1;
     }
     const std::string folder = argv[1];
     const double marker_size = std::stod(argv[2]);
-    bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0;
+    bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
     std::set<int> excluded_cams; std::string init_path;
-    enum { NONE, EXCLUDE, THRESH, CMAX, INIT } flag = NONE;
+    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT } flag = NONE;
     for (int i = 3; i < argc; i++) {
         const std::string a = argv[i];
         if (a == "-subseqs") { use_subseqs = true; flag = NONE; }
@@ -34,10 +36,12 @@ int main(int argc, char **argv) {
         else if (a == "-thresh") { set_threshold = true; flag = THRESH; }
         else if (a == "-consensus-max") flag = CMAX;
         else if (a == "-init") flag = INIT;
+        else if (a == "-reject-outliers") flag = REJECT;
         else if (flag == EXCLUDE) excluded_cams.insert(std::stoi(a));
         else if (flag == THRESH) { threshold = std::stod(a); flag = NONE; }
         else if (flag == CMAX) { consensus_max = std::stoi(a); flag = NONE; }
         else if (flag == INIT) { init_path = a; flag = NONE; }
+        else if (flag == REJECT) { reject_px = std::stod(a); flag = NONE; }
     }
     std::string suffix;                                         // find_solution.cpp:76-100
     if (use_subseqs) suffix += "_subseqs";
@@ -80,6 +84,15 @@ int main(int argc, char **argv) {
         mcm.solve();
         d += std::chrono::system_clock::now() - start;
         std::cout.precision(17); std::cout << "final_error: " << mcm.final_error << " iterations: " << mcm.iterations << std::endl;
+        if (reject_px >= 0) {
+            start = std::chrono::system_clock::now();
+            aar::MultiCamMapper::Rejection rj;
+            mcm.remove_outliers(reject_px, &rj);
+            std::printf("removed %lld of %lld detections above %.17g px\n", rj.removed, rj.observations, reject_px); std::fflush(stdout);
+            mcm.solve();
+            d += std::chrono::system_clock::now() - start;
+            std::cout << "final_error: " << mcm.final_error << " iterations: " << mcm.iterations << std::endl;
+        }
         mcm.write_solution_file(final_path);
         mcm.write_text_solution_file(final_path + ".yaml");
         const int minutes = (int)(d.count() / 60); const long seconds = std::lround(d.count() - minutes * 60);

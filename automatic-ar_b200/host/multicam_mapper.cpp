@@ -254,6 +254,79 @@ void MultiCamMapper::solve() {
     }
 }
 
+MultiCamMapper::ErrorReport MultiCamMapper::error_report(const std::vector<double> &q) {
+    if (!handle) make_handle(corners_undistorted);
+    if (io_vec.size() != (size_t)aar_num_vars(handle)) mats2eVec(config, io_vec);
+    ErrorReport r;
+    const size_t C = transforms_to_root_cam.size(), M = transforms_to_root_marker.size(), F = object_to_global.size();
+    size_t nd = 0;
+    for (auto &f : (raw_frame_cam_markers.empty() ? frame_cam_markers : raw_frame_cam_markers)) for (auto &c : f.second) nd += c.second.size();
+    r.det_err.assign(nd, 0.0); r.q = q; r.q_value.assign(q.size(), 0.0);
+    std::vector<int64_t> cnt(C + M + F); std::vector<double> sum(C + M + F), mx(C + M + F);
+    aar_error_report_out o; std::memset(&o, 0, sizeof o);
+    o.det_err = r.det_err.data();
+    o.cam_count = cnt.data(); o.marker_count = cnt.data() + C; o.frame_count = cnt.data() + C + M;
+    o.cam_sum_sq = sum.data(); o.marker_sum_sq = sum.data() + C; o.frame_sum_sq = sum.data() + C + M;
+    o.cam_max = mx.data(); o.marker_max = mx.data() + C; o.frame_max = mx.data() + C + M;
+    o.num_q = (int32_t)q.size(); o.q = r.q.data(); o.q_value = r.q_value.data();
+    check(aar_error_report(handle, io_vec.data(), &o), "aar_error_report");
+    r.observations = o.num_observations; r.not_in_problem = o.num_not_in_problem; r.sum_sq = o.sum_sq;
+    size_t i = 0;
+    auto fill = [&](const std::map<int, Mat44> &ids, std::map<int, EntityError> &dst) {
+        for (auto &p : ids) { EntityError &e = dst[p.first]; e.observations = cnt[i]; e.sum_sq = sum[i]; e.max = mx[i]; i++; }
+    };
+    fill(transforms_to_root_cam, r.cams); fill(transforms_to_root_marker, r.markers); fill(object_to_global, r.frames);
+    return r;
+}
+
+long long MultiCamMapper::remove_outliers(double max_px, Rejection *out) {
+    const ErrorReport rep = error_report({});
+    // det_err follows make_handle's flatten order: the raw detections when present (frame_cam_markers then holds the undistorted copy of
+    // exactly those that are in the problem, in the same order), else frame_cam_markers
+    const bool from_raw = !raw_frame_cam_markers.empty();
+    auto in_problem = [&](int f, int c, int id) { return object_to_global.count(f) && transforms_to_root_cam.count(c) && transforms_to_root_marker.count(id); };
+    Rejection rj; rj.observations = rep.observations;
+    std::map<int, long long> left;                               // frame -> observations kept
+    std::map<int, long long> cam_left, marker_left;
+    size_t i = 0;
+    for (auto &f : (from_raw ? raw_frame_cam_markers : frame_cam_markers)) {
+        for (auto &c : f.second) {
+            std::vector<Marker> &v = c.second;
+            std::vector<Marker> *u = nullptr;
+            if (from_raw) { auto fi = frame_cam_markers.find(f.first); if (fi != frame_cam_markers.end()) { auto ci = fi->second.find(c.first); if (ci != fi->second.end()) u = &ci->second; } }
+            size_t w = 0, ui = 0, uw = 0;
+            for (size_t k = 0; k < v.size(); k++) {
+                const bool inp = in_problem(f.first, c.first, v[k].id);
+                const bool drop = rep.det_err[i++] > max_px;         // NaN (not in the problem) is never above
+                if (!drop) v[w++] = v[k];
+                if (from_raw && inp && u) { if (!drop) (*u)[uw++] = (*u)[ui]; ui++; }
+                if (drop) rj.removed++;
+                else if (inp) { left[f.first]++; cam_left[c.first]++; marker_left[v[k].id]++; }
+            }
+            v.resize(w);
+            if (u) u->resize(uw);
+        }
+    }
+    auto prune = [](FrameCamMarkers &fcm) {                      // no empty camera lists, no empty frames
+        for (auto f = fcm.begin(); f != fcm.end();) {
+            for (auto c = f->second.begin(); c != f->second.end();) c = c->second.empty() ? f->second.erase(c) : std::next(c);
+            f = f->second.empty() ? fcm.erase(f) : std::next(f);
+        }
+    };
+    for (auto f = object_to_global.begin(); f != object_to_global.end();) {
+        if (left.count(f->first)) { ++f; continue; }
+        rj.dropped_frames.push_back(f->first);
+        frame_cam_markers.erase(f->first); raw_frame_cam_markers.erase(f->first);
+        f = object_to_global.erase(f);
+    }
+    prune(frame_cam_markers); prune(raw_frame_cam_markers);
+    for (auto &p : transforms_to_root_cam) if (!cam_left.count(p.first)) rj.unobserved_cams.push_back(p.first);
+    for (auto &p : transforms_to_root_marker) if (!marker_left.count(p.first)) rj.unobserved_markers.push_back(p.first);
+    drop_handle(); io_vec.clear();
+    if (out) *out = rj;
+    return rj.removed;
+}
+
 void MultiCamMapper::track() {
     // track() optimises the object pose only (apps/track.cpp:95-97 sets the flags; forced here like the 6-variable io_vec of :272-279)
     Config keep = config;

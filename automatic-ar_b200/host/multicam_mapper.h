@@ -3,6 +3,8 @@
 // aar::Mat44, the optimisation itself forwarded to the CUDA path through the C ABI of include/aar_cuda.h.
 // What is NOT here: overlays / visualisation (GUI).
 #pragma once
+#include <cmath>
+#include <map>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -55,6 +57,22 @@ public:
     size_t get_num_vars(const Config &conf) const;
 
     void solve();     // multicam_mapper.cpp:419-428: device-resident SparseLevMarq::solve(io_vec, error_function, jacobian_function)
+
+    // not in the reference: reprojection errors of the current state (aar_error_report, include/aar_cuda.h), Huber weights off
+    struct EntityError { long long observations = 0; double sum_sq = 0, max = 0; double rms() const { return std::sqrt(sum_sq / (4.0 * (double)observations)); } };
+    struct ErrorReport {
+        long long observations = 0, not_in_problem = 0; double sum_sq = 0;
+        std::map<int, EntityError> cams, markers, frames;       // by id
+        std::vector<double> q, q_value;                          // exact percentiles of the observation errors
+        std::vector<double> det_err;                             // per detection of the handle (raw_frame_cam_markers when present, else frame_cam_markers,
+                                                                 // frame / camera / detection order); NaN when not in the problem
+    };
+    // at io_vec when it belongs to the current Config (after solve()), else at the current transforms
+    ErrorReport error_report(const std::vector<double> &q = {0.5, 0.9, 0.99});
+    // removes every detection whose error is above max_px and the frames left without an observation; cameras and markers that lose
+    // all their observations stay (listed in `out`).  The handle is dropped: the next solve() creates it anew.  Returns the number removed.
+    struct Rejection { long long removed = 0, observations = 0; std::vector<int> dropped_frames, unobserved_cams, unobserved_markers; };
+    long long remove_outliers(double max_px, Rejection *out = nullptr);
     void track();     // multicam_mapper.cpp:430-443: per-frame 6-dof solve against the fixed rig, every frame of the object at once
 
     bool write_solution_file(const std::string &path);         // byte-exact .solution (multicam_mapper.cpp:1053-1099)

@@ -24,7 +24,7 @@ NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a",
 # declared by include/aar_cuda.h — tests check that the library exports every one of them
 EXPORTS = ["aar_lm_default_params", "aar_problem_create", "aar_problem_destroy", "aar_last_error", "aar_num_vars",
            "aar_num_observations", "aar_num_local_observations", "aar_jacobian_nnz", "aar_index_maps", "aar_get_observations",
-           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_eval_jacobian", "aar_reduced_system", "aar_lm_solve",
+           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_lm_solve",
            "aar_lm_begin", "aar_lm_iterate", "aar_lm_end", "aar_track_batch", "aar_track_upload", "aar_track_run", "aar_track_download", "aar_track_ms", "aar_shard_plan", "aar_row_map", "aar_comm_unique_id", "aar_comm_init",
            "aar_kernel_launches", "aar_set_profiling", "aar_get_phase_ms", "aar_problem_stats"]
 
@@ -72,6 +72,14 @@ class LmTrace(C.Structure):
 class LmReport(C.Structure):
     _fields_ = [("initial_cost", C.c_double), ("final_cost", C.c_double), ("iterations", C.c_int32), ("exit_code", C.c_int32),
                 ("total_tries", C.c_int64), ("trace", C.POINTER(LmTrace)), ("trace_capacity", C.c_int32), ("trace_len", C.c_int32)]
+
+
+class ErrorReportOut(C.Structure):
+    _fields_ = [("det_err", C.c_void_p), ("cam_count", C.c_void_p), ("marker_count", C.c_void_p), ("frame_count", C.c_void_p),
+                ("cam_sum_sq", C.c_void_p), ("marker_sum_sq", C.c_void_p), ("frame_sum_sq", C.c_void_p),
+                ("cam_max", C.c_void_p), ("marker_max", C.c_void_p), ("frame_max", C.c_void_p),
+                ("num_q", C.c_int32), ("reserved", C.c_int32), ("q", C.c_void_p), ("q_value", C.c_void_p),
+                ("num_observations", C.c_int64), ("num_not_in_problem", C.c_int64), ("sum_sq", C.c_double)]
 
 
 _lib = None
@@ -201,6 +209,24 @@ class Problem:
         ss = C.c_double(0)
         _chk(lib().aar_eval_residual(self.h, _vp(z), C.c_float(huber_delta), _vp(r) if want_vector else None, C.byref(ss)), "aar_eval_residual")
         return r, ss.value
+
+    def error_report(self, z, q=(0.5, 0.9, 0.99)):
+        """aar_error_report: reprojection error per detection (indexed like the rig's det_* arrays, NaN when not in the problem), count /
+        sum of squares / max error per camera, marker and frame, exact percentiles q -> q_value, totals."""
+        z = np.ascontiguousarray(z, np.float64)
+        qa = np.ascontiguousarray(q, np.float64).reshape(-1)
+        n_det = len(self._keep["det_frame"])
+        r = dict(det_err=np.zeros(n_det), q=qa, q_value=np.zeros(len(qa)))
+        out = ErrorReportOut()
+        out.det_err = _vp(r["det_err"])
+        for ent, n in (("cam", self.nC), ("marker", self.nM), ("frame", self.nF)):
+            r[ent + "_count"] = np.zeros(n, np.int64); r[ent + "_sum_sq"] = np.zeros(n); r[ent + "_max"] = np.zeros(n)
+            for k in ("count", "sum_sq", "max"):
+                setattr(out, f"{ent}_{k}", _vp(r[f"{ent}_{k}"]))
+        out.num_q = len(qa); out.q = _vp(qa); out.q_value = _vp(r["q_value"])
+        _chk(lib().aar_error_report(self.h, _vp(z), C.byref(out)), "aar_error_report")
+        r.update(observations=out.num_observations, not_in_problem=out.num_not_in_problem, sum_sq=out.sum_sq)
+        return r
 
     def jacobian(self, z):
         z = np.ascontiguousarray(z, np.float64)

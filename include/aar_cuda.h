@@ -125,6 +125,32 @@ int aar_evec2mats(aar_problem *p, const double *z, double *cam_T, double *marker
 
 /* MultiCamMapper::error_function (multicam_mapper.cpp:731-737): r has 8*n_local entries */
 int aar_eval_residual(aar_problem *p, const double *z, float huber_delta, double *r, double *sum_sq);
+/* Reprojection-error report at z (not in the reference).  The residual of an observation is r[0..7] of the handle's own residual
+ * evaluation (the one aar_eval_residual runs) with the Huber weights OFF; its error is e = sqrt(s / 4), s = r0^2 + ... + r7^2 summed
+ * left to right without FMA: the RMS corner distance in pixels.  Every pointer may be NULL except q / q_value when num_q > 0.
+ * Entity arrays are indexed by rank of the id (ascending ids); an entity without observations has count 0, sum_sq 0, max 0.
+ * Duplicates erased by "last duplicate wins" still have residual rows, so they count like any other observation. */
+typedef struct {
+    double *det_err;                                  /* [desc num_detections], indexed like desc->det_*: e, NaN for a detection not in
+                                                       * the problem (unknown camera / marker id, frame without a pose) */
+    int64_t *cam_count, *marker_count, *frame_count;  /* observations */
+    double *cam_sum_sq, *marker_sum_sq, *frame_sum_sq;/* sum of s; RMS = sqrt(sum_sq / (4 count)) */
+    double *cam_max, *marker_max, *frame_max;         /* max e */
+    int32_t num_q;                                    /* in: number of percentiles, <= 256 */
+    int32_t reserved;
+    const double *q;                                  /* in: [num_q] in [0, 1] */
+    double *q_value;                                  /* out: [num_q] exact order statistic sorted(e)[floor(q (n - 1))]; NaN when n = 0 */
+    int64_t num_observations;                         /* out: n */
+    int64_t num_not_in_problem;                       /* out: detections of the description that are not observations */
+    double sum_sq;                                    /* out: Huber-off cost (sum of s over all observations) */
+} aar_error_report_out;
+#ifdef __cplusplus
+static_assert(sizeof(aar_error_report_out) == 128, "aar_error_report_out layout");
+#else
+_Static_assert(sizeof(aar_error_report_out) == 128, "aar_error_report_out layout");
+#endif
+/* Single-rank handles only, and not between aar_lm_begin and aar_lm_end (AAR_ERR_INVALID). */
+int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out);
 /* MultiCamMapper::jacobian_function (multicam_mapper.cpp:739-801) in the compressed-column form
  * Eigen's setFromTriplets produces: colptr[num_vars+1], rowidx[nnz], vals[nnz].  Single-rank handles only. */
 int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t *rowidx, double *vals);
