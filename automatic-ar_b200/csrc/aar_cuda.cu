@@ -49,7 +49,6 @@ struct Nccl {
     ncclResult_t (*GetUniqueId)(ncclUniqueId *) = nullptr;
     ncclResult_t (*CommInitRank)(ncclComm_t *, int, ncclUniqueId, int) = nullptr;
     ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
     const char *(*GetErrorString)(ncclResult_t) = nullptr;
     bool load() {
@@ -60,7 +59,6 @@ struct Nccl {
         GetUniqueId = (decltype(GetUniqueId))dlsym(lib, "ncclGetUniqueId");
         CommInitRank = (decltype(CommInitRank))dlsym(lib, "ncclCommInitRank");
         AllReduce = (decltype(AllReduce))dlsym(lib, "ncclAllReduce");
-        AllGather = (decltype(AllGather))dlsym(lib, "ncclAllGather");
         CommDestroy = (decltype(CommDestroy))dlsym(lib, "ncclCommDestroy");
         GetErrorString = (decltype(GetErrorString))dlsym(lib, "ncclGetErrorString");
         if (!GetUniqueId || !CommInitRank || !AllReduce || !CommDestroy) { set_err("NCCL: missing symbols"); return false; }
@@ -106,7 +104,6 @@ struct aar_problem {
     DevBuf<int> d_frame_cs_cum, d_slot_frame, d_frame_block_slot, d_frame_obs_ptr, d_trk_iters, d_obs_pair;
     DevBuf<int2> d_pair_fc; DevBuf<double> d_pair_tab; int npairs = 0;
     DevBuf<int4> d_pair_info, d_mrun_info; DevBuf<int> d_perm_fm, d_pair_cam; DevBuf<double> d_cm_rep; int nmruns = 0;     // visiting orders of the tensor-core assembly (aar_assemble.cuh)
-    bool legacy_acc = false;                                                          // AAR_ASM=legacy: round-1 lane-per-observation kernel (A/B aid)
     bool analytic = false; DevBuf<double> d_cam_an, d_mk_an, d_fr_an;                 // analytic-Jacobian / full-FP64 variant (aar_analytic.cuh)
     DevBuf<double> d_trk_cam_inv, d_trk_Y, d_trk_z, d_trk_z0, d_trk_cost; bool trk_have_z0 = false; double track_ms = 0; long long track_runs = 0;
     DevBuf<double> d_fc, d_E, d_xinv;
@@ -116,7 +113,7 @@ struct aar_problem {
     DevBuf<LmState> d_st;
     DevBuf<int> d_flag;
     LmState *h_st = nullptr; double *h_red3 = nullptr; int *h_flags = nullptr; // pinned
-    // ---- staged central-difference numerators ([144][N] float32, or float64 in the exact fallback) and residuals ([8][N])
+    // ---- staged rows of central-difference numerators ([N][JROW] float32, or float64 in the exact fallback) and Huber weights ([N][4])
     DevBuf<float> d_Jn32; DevBuf<double> d_Jn64, d_Rv;
     int max_ms = 0, num_sms = 148; size_t smem_optin = 227 * 1024;
     bool use_cluster_solve = true;
@@ -138,8 +135,6 @@ struct aar_problem {
     DevBuf<LmTraceDev> d_trace;
     // aar_error_report (aar_report.cuh): observation errors, entity statistics [C + M + F], select state [2 nq], digit histograms [nq][SEL_BINS]
     DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
-    // sharded handles: every rank's reduced system and decision scalars mapped through cudaIpc (aar_kernels.cuh: PeerDev)
-    PeerDev pd; bool peer_ok = false; DevBuf<double> d_peer_small, d_Br_sum; DevBuf<int> d_peer_flags; std::vector<void *> ipc_opened;
     cudaEvent_t ev[16] = {}; double phase_ms[AAR_NUM_PHASES] = {};
 };
 
@@ -229,7 +224,7 @@ int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_ou
 void prof_mark(aar_problem *p, int i) { if (p->profiling) cudaEventRecord(p->ev[i], p->stream); }
 
 // Launches the Jacobian kernels: k_jac_project (numerators + residual at z, one row per observation) and the tensor-core assembly
-// k_asm_pairs + k_asm_mruns (aar_assemble.cuh).  AAR_ASM=legacy selects the round-1 lane-per-observation kernel instead.
+// k_asm_pairs + k_asm_mruns (aar_assemble.cuh).
 template <typename JT>
 int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
     const size_t tab_bytes = (size_t)((p->M * MK_TAB_S + 1) & ~1) * sizeof(double);
@@ -240,26 +235,7 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
     const double s1 = p->analytic ? 1.0 : 1.0 / (2 * p->J_delta), s2 = s1 * s1;
     const int grid1 = (int)std::max<long long>(1, std::min<long long>((long long)AAR_PROJ_MINBLOCKS * p->num_sms, (N + PROJ_THREADS - 1) / PROJ_THREADS));
     prof_mark(p, 7);
-    if (p->legacy_acc) {
-        if (p->opt_i) { set_err("AAR_ASM=legacy has no intrinsics block"); return AAR_ERR_UNSUPPORTED; }
-        constexpr int AW = 8;
-        auto k1 = k_jac_project<JT, false>; auto k2 = k_jac_accumulate<JT, AW>;
-        const size_t scr = (size_t)AW * SCR_DOUBLES * sizeof(double), fix = (size_t)(p->nrc + p->nrm) * 27 * sizeof(double);
-        AccPlan pl; pl.s1 = s1; pl.s2 = s2; pl.skip = 0;
-        const size_t avail = p->smem_optin - 2048;
-        if (fix + scr > avail) { set_err("too many cameras + markers (%d) for the shared accumulators of k_jac_accumulate", p->nrc + p->nrm); return AAR_ERR_UNSUPPORTED; }
-        pl.hcm_smem = (int)std::min<size_t>((size_t)p->nrc * p->nrm, (avail - fix - scr) / 288);
-        const size_t smem2 = fix + (size_t)pl.hcm_smem * 288 + scr;
-        CU(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem1, 1024)));
-        CU(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-        const int grid2 = (int)std::max<long long>(1, std::min<long long>((long long)p->num_sms, (N + AW * 32 - 1) / (AW * 32)));
-        LAUNCH(p, k1, grid1, PROJ_THREADS, smem1, p->dp, huber_eval, Jn, p->d_Rv.p, tabs_smem, p->d_flag.p, 0LL, N);
-        prof_mark(p, 9);
-        LAUNCH(p, k2, grid2, AW * 32, smem2, p->dp, pl, Jn, p->d_Rv.p, p->d_Hf.p, p->d_W.p, p->d_Hrr.p, p->d_gr.p, 0LL, N);
-        prof_mark(p, 8);
-        return AAR_OK;
-    }
-    auto k1 = k_jac_project<JT, true>; auto k2 = k_asm_pairs<JT>; auto k3 = k_asm_mruns<JT>;
+    auto k1 = k_jac_project<JT>; auto k2 = k_asm_pairs<JT>; auto k3 = k_asm_mruns<JT>;
     AsmPlan pl; pl.pair_info = p->d_pair_info.p; pl.pair_cam = p->d_pair_cam.p; pl.npairs = p->npairs; pl.mrun_info = p->d_mrun_info.p; pl.perm_fm = p->d_perm_fm.p;
     pl.nmruns = p->nmruns; pl.nperm = (int)p->d_perm_fm.n;
     pl.s1 = s1; pl.s2 = s2;
@@ -330,11 +306,9 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, double *Jdump, bool de
         if (p->d_Hrr.n) CU(cudaMemsetAsync(p->d_Hrr.p, 0, p->d_Hrr.n * sizeof(double), p->stream));
         if (p->d_gr.n) CU(cudaMemsetAsync(p->d_gr.p, 0, p->d_gr.n * sizeof(double), p->stream));
         if (p->d_Hf.n) CU(cudaMemsetAsync(p->d_Hf.p, 0, p->d_Hf.n * sizeof(double), p->stream));
-        // the tensor-core assembly stores every W block (each slot is owned by one run); the legacy kernel accumulates into them
-        if (p->legacy_acc && p->d_W.n) CU(cudaMemsetAsync(p->d_W.p, 0, p->d_W.n * sizeof(double), p->stream));
         if (N == 0) return AAR_OK;
-        const size_t Np = (N + 31) / 32 * 32;      // whole tiles of 32 observations
-        if (p->d_Rv.n < 8 * Np) CU(p->d_Rv.alloc(8 * Np));          // legacy: residuals [N/32][8][32]; assembly path: Huber weights [N][4]
+        const size_t Np = (N + 31) / 32 * 32;      // rounded up to a multiple of 32 observations
+        if (p->d_Rv.n < 4 * Np) CU(p->d_Rv.alloc(4 * Np));          // Huber weights [N][4]
         int rc;
         if (exact) { if (p->d_Jn64.n < JROW * Np) CU(p->d_Jn64.alloc(JROW * Np)); rc = launch_jacobian<double>(p, huber_eval, p->d_Jn64.p); }
         else { if (p->d_Jn32.n < JROW * Np) CU(p->d_Jn32.alloc(JROW * Np)); rc = launch_jacobian<float>(p, huber_eval, p->d_Jn32.p); }
@@ -352,8 +326,6 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, double *Jdump, bool de
     }
     return AAR_OK;
 }
-
-int zero_normal_equations(aar_problem *) { return AAR_OK; }   // zeroing is part of jacobian_accumulate
 
 __global__ void k_prepare_reduced(int n_r, const double *__restrict__ Hrr, const double *__restrict__ gr, double *__restrict__ red) {
     // red = [S (n_r*n_r) | b (n_r) | Br (n_r)]
@@ -385,11 +357,10 @@ int schur_eliminate(aar_problem *p, double *S, double *b) {
 int build_and_solve_reduced(aar_problem *p) {
     const int n_r = p->n_r;
     double *S = p->d_red.p, *b = S + (size_t)n_r * n_r;     // [S | b | Br]: Br = -gr is kept for the gain denominator
-    if (p->peer_ok) LAUNCH(p, k_peer_begin_try, 1, 1, 0, p->pd);      // nobody reads this rank's S of the previous try any more
     if (n_r > 0) LAUNCH(p, k_prepare_reduced, cdiv((long long)n_r * n_r + n_r, 256), 256, 0, n_r, p->d_Hrr.p, p->d_gr.p, S);
     { int rc = schur_eliminate(p, S, b); if (rc) return rc; }
     if (n_r > 0) {
-        if (!p->peer_ok) { int rc = allreduce(p, S, (size_t)n_r * n_r + 2 * n_r, ncclSum); if (rc) return rc; }
+        { int rc = allreduce(p, S, (size_t)n_r * n_r + 2 * n_r, ncclSum); if (rc) return rc; }
         const int nblk = (n_r + CH_NB - 1) / CH_NB;
         bool done = false;
         if (nblk <= 16 && p->use_cluster_solve) {
@@ -399,7 +370,7 @@ int build_and_solve_reduced(aar_problem *p) {
             cudaLaunchAttribute at[1]; at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = nblk; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
             cfg.attrs = at; cfg.numAttrs = 1;
             const double *bc = b; const LmState *stp = p->d_st.p;
-            cudaError_t e = cudaLaunchKernelEx(&cfg, k_reduced_solve_cluster2, n_r, S, bc, p->d_dr.p, stp, p->d_flag.p, p->d_xinv.p, p->pd);
+            cudaError_t e = cudaLaunchKernelEx(&cfg, k_reduced_solve_cluster2, n_r, S, bc, p->d_dr.p, stp, p->d_flag.p, p->d_xinv.p);
             if (e == cudaSuccess) { done = true; p->launches++; }
             else { cudaGetLastError(); p->use_cluster_solve = false; }      // e.g. the cluster cannot be scheduled: fall back for good
         }
@@ -706,7 +677,6 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
         }
         p->nmruns = (int)mrun_info.size();
         UP(p->d_perm_fm, perm_fm); UP(p->d_mrun_info, mrun_info);
-        { const char *e = getenv("AAR_ASM"); p->legacy_acc = e && !strcmp(e, "legacy") && !p->analytic; }
     }
 
     UP(p->d_raw_a, raw_a); UP(p->d_raw_b, raw_b); UP(p->d_obs_pair, obs_pair); UP(p->d_pair_fc, pair_fc);
@@ -735,7 +705,6 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
     dp.opt_c = p->opt_c; dp.opt_m = p->opt_m; dp.opt_f = p->opt_f; dp.huber = p->huber;
     dp.nrc = p->nrc; dp.nrm = p->nrm; dp.n_r = p->n_r; dp.col_frame0 = p->n_r + 6 * p->f_begin;
     dp.opt_i = p->opt_i; dp.nri = p->nri; dp.col_intr0 = 6 * (p->nrc + p->nrm); dp.st_dev = nullptr;
-    std::memset(&p->pd, 0, sizeof p->pd); p->pd.world = 1;
     dp.h = (double)(p->marker_size / 2.f); // aruco::Marker::get3DPoints: half size in float (marker.cpp:358-369)
     dp.J_delta = p->J_delta;
     dp.obs_f = p->d_obs_f.p; dp.obs_cm = p->d_obs_cm.p; dp.obs_slot_c = p->d_slot_c.p; dp.obs_slot_m = p->d_slot_m.p;
@@ -810,7 +779,6 @@ void aar_problem_destroy(aar_problem *p) {
     if (p->h_st) cudaFreeHost(p->h_st);
     if (p->h_red3) cudaFreeHost(p->h_red3);
     if (p->h_flags) cudaFreeHost(p->h_flags);
-    for (void *q : p->ipc_opened) cudaIpcCloseMemHandle(q);
     if (p->lm_exec) cudaGraphExecDestroy(p->lm_exec);
     if (p->lm_graph) cudaGraphDestroy(p->lm_graph);
     if (p->lm_side) cudaStreamDestroy(p->lm_side);
@@ -1095,7 +1063,6 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
     if (p->lm_active) { set_err("aar_reduced_system between aar_lm_begin and aar_lm_end would replace the resident iterate and LM state"); return AAR_ERR_INVALID; }
     CU(cudaSetDevice(p->device));
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
-    if ((rc = zero_normal_equations(p))) return rc;
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
     residual(p, p->d_z.p, p->huber_eval, nullptr);
     if ((rc = jacobian_accumulate(p, p->huber_eval, nullptr))) return rc;
@@ -1183,7 +1150,7 @@ static bool lm_graph_build(aar_problem *p) {
     p->capturing = true; p->dp.st_dev = p->d_st.p;
     GR(cudaStreamBeginCaptureToGraph(main_stream, body_outer, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed)); cap_outer = true;
     if (jacobian_accumulate(p, 0.f, nullptr)) { ok = false; goto done; }
-    k_lm_begin_iter_g<<<1, 1, 0, main_stream>>>(p->d_st.p, p->d_flag.p, p->lm_inner, p->comm ? 1 : 0); p->launches++;
+    k_lm_begin_iter_g<<<1, 1, 0, main_stream>>>(p->d_st.p, p->d_flag.p, p->lm_inner); p->launches++;
     // the inner WHILE node goes in by hand, behind everything captured so far; the capture continues behind it
     GR(cudaStreamGetCaptureInfo_v2(main_stream, &cs, nullptr, &cg, &deps, &ndeps));
     std::memset(&ni, 0, sizeof ni);
@@ -1203,7 +1170,7 @@ static bool lm_graph_build(aar_problem *p) {
         p->launches++;
     }
     residual(p, p->d_zt.p, 0.f, nullptr);
-    k_lm_decide_g<<<1, 1, 0, p->stream>>>(p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->lm_inner, p->d_flag.p, p->pd); p->launches++;
+    k_lm_decide_g<<<1, 1, 0, p->stream>>>(p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->lm_inner); p->launches++;
     k_lm_commit<<<std::max(1, std::min(2 * p->num_sms, (int)cdiv(p->n_vars, 256))), 256, 0, p->stream>>>(p->d_st.p, p->n_vars, p->d_zt.p, p->d_z.p); p->launches++;
     GR(cudaStreamEndCapture(p->lm_side, &tmp)); cap_inner = false;
     p->stream = main_stream;
@@ -1264,7 +1231,7 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
     if (rep) { rep->trace_len = 0; rep->initial_cost = p->initial_cost; }
     double *S = p->d_red.p, *b = S + (size_t)n_r * n_r, *Br = b + n_r;
     const char *no_graph = getenv("AAR_NO_GRAPH");           // development aid: host-driven loop only
-    const bool graph_eligible = (!p->comm || p->peer_ok) && !p->profiling && !P.verbose && !p->legacy_acc && !p->force_exact_staging && !p->analytic && !(no_graph && *no_graph == '1') && p->dp.N > 0;
+    const bool graph_eligible = !p->comm && !p->profiling && !P.verbose && !p->force_exact_staging && !p->analytic && !(no_graph && *no_graph == '1') && p->dp.N > 0;
     for (int it = 0; it < max_iters && !mustExit; it++) {
         if (graph_eligible && p->h_st->mu >= 0 && (p->lm_graph_ok || !p->lm_graph_tried)) {
             // every iteration but the first of a solve: inside the graph, without the host (see lm_graph_build)
@@ -1274,7 +1241,6 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
                 const int want = std::min(max_iters - it, LM_TRACE_DEV_CAP);
                 if ((rc = lm_graph_run(p, want, rep, &gd, &gx))) { p->lm_active = false; return rc; }
                 done_iters += gd;
-                if (p->h_flags[3]) { set_err("a peer rank did not answer within the time-out of the peer-memory reduction"); p->lm_active = false; return AAR_ERR_COMM; }
                 if (gx == -1) {
                     int flags[4];
                     CU(cudaMemcpy(flags, p->d_flag.p, sizeof flags, cudaMemcpyDeviceToHost));
@@ -1294,8 +1260,7 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
         }
         // ---- J, JtJ blocks, B (sparselevmarq.h:353-367)
         prof_mark(p, 0);
-        if ((rc = zero_normal_equations(p))) return rc;
-        if ((rc = jacobian_accumulate(p, p->huber_eval, nullptr, true))) { p->lm_active = false; return rc; }
+            if ((rc = jacobian_accumulate(p, p->huber_eval, nullptr, true))) { p->lm_active = false; return rc; }
         prof_mark(p, 1);
         if (p->h_st->mu < 0) { // first iteration: mu = tau * max diag(JtJ) (sparselevmarq.h:369-377)
             p->h_st->maxdiag = -1e300; push_state(p);
@@ -1325,8 +1290,8 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
             prof_mark(p, 4);
             residual(p, p->d_zt.p, p->huber_cur, nullptr);
             prof_mark(p, 5);
-            if (!p->peer_ok && (rc = allreduce(p, p->d_red3.p, 3, ncclSum))) return rc;
-            LAUNCH(p, k_lm_decide, 1, 1, 0, p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->d_flag.p, p->pd);
+            if ((rc = allreduce(p, p->d_red3.p, 3, ncclSum))) return rc;
+            LAUNCH(p, k_lm_decide, 1, 1, 0, p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->d_flag.p);
             // an accepted trial point becomes the iterate by a device copy (a pointer swap would invalidate the captured graph of the resident loop)
             LAUNCH(p, k_lm_commit, std::max(1, std::min(2 * p->num_sms, (int)cdiv(p->n_vars, 256))), 256, 0, p->d_st.p, p->n_vars, p->d_zt.p, p->d_z.p);
             if ((rc = fetch_state(p))) return rc;
@@ -1344,7 +1309,7 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
                     cudaEventElapsedTime(&ms, p->ev[0], p->ev[1]); p->phase_ms[0] += ms;
                     cudaEventElapsedTime(&ms, p->ev[7], p->ev[9]); p->phase_ms[5] += ms; p->phase_ms[6] += 1;
                     cudaEventElapsedTime(&ms, p->ev[9], p->ev[8]); p->phase_ms[7] += ms;
-                    if (!p->legacy_acc && p->npairs > 0) { cudaEventElapsedTime(&ms, p->ev[9], p->ev[12]); p->phase_ms[10] += ms; cudaEventElapsedTime(&ms, p->ev[12], p->ev[8]); p->phase_ms[11] += ms; }
+                    if (p->npairs > 0) { cudaEventElapsedTime(&ms, p->ev[9], p->ev[12]); p->phase_ms[10] += ms; cudaEventElapsedTime(&ms, p->ev[12], p->ev[8]); p->phase_ms[11] += ms; }
                 }
                 if (p->opt_f && p->dp.F > 0 && p->n_r > 0 && p->nslots > 0) { cudaEventElapsedTime(&ms, p->ev[10], p->ev[11]); p->phase_ms[8] += ms; p->phase_ms[9] += 1; }
                 cudaEventElapsedTime(&ms, p->ev[2], p->ev[3]); p->phase_ms[1] += ms;
@@ -1361,7 +1326,6 @@ int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
             it--; continue;
         }
         const int *flags = p->h_flags;                    // fetched with the state of the last try
-        if (flags[3]) { set_err("a peer rank did not answer within the time-out of the peer-memory reduction"); p->lm_active = false; return AAR_ERR_COMM; }
         if (!std::isfinite(p->h_st->trial_cost)) { set_err("non-finite cost at iteration %d", p->iter); p->lm_active = false; return AAR_ERR_NUMERIC; }
         if (flags[0] || flags[2]) {
             // flags[0]: a non-positive pivot in a frame block or in the reduced system (the kernels substituted 1 to keep going):
@@ -1513,69 +1477,13 @@ int aar_comm_init(aar_problem *p, const void *id128) {
     ncclUniqueId id; std::memcpy(&id, id128, sizeof id);
     ncclResult_t r = g_nccl.CommInitRank(&p->comm, p->world, id, p->rank);
     if (r != ncclSuccess) { set_err("ncclCommInitRank: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "error"); p->comm = nullptr; return AAR_ERR_COMM; }
-    // ---- peer-memory reduction of the LM try (aar_kernels.cuh: PeerDev): map every rank's reduced system, decision scalars and flag arrays
-    // through cudaIpc; the handles travel by one ncclAllGather.  Any failure, on any rank, keeps the NCCL all-reduces for all of them.
-    {
-        // Opt-in (AAR_PEER=1): measured on 8 x B200 at cfg 4, the peer-memory sums + graph-resident loop take 4.06 ms per LM iteration against
-        // 3.94 ms for ncclAllReduce + host-driven tries (profiles/r2_bench_cfg4_n8*.json): 15 CTAs pulling 14 MB over NVLink with 8-byte loads
-        // and three flag round trips per try cost more than the two NCCL calls they replace.
-        const char *e = getenv("AAR_PEER");
-        int want = (p->world <= PEER_MAX && p->n_r > 0 && p->use_cluster_solve && g_nccl.AllGather && e && *e == '1') ? 1 : 0;
-        struct Handles { cudaIpcMemHandle_t red, small, flags; };
-        Handles mine; std::memset(&mine, 0, sizeof mine);
-        if (want) {
-            if (p->d_peer_small.alloc(8) != cudaSuccess || p->d_peer_flags.alloc(4 * PEER_MAX) != cudaSuccess || p->d_Br_sum.alloc((size_t)p->n_r) != cudaSuccess) want = 0;
-            else {
-                CU(cudaMemsetAsync(p->d_peer_small.p, 0, 8 * sizeof(double), p->stream)); CU(cudaMemsetAsync(p->d_peer_flags.p, 0, 4 * PEER_MAX * sizeof(int), p->stream));
-                if (cudaIpcGetMemHandle(&mine.red, p->d_red.p) != cudaSuccess || cudaIpcGetMemHandle(&mine.small, p->d_peer_small.p) != cudaSuccess ||
-                    cudaIpcGetMemHandle(&mine.flags, p->d_peer_flags.p) != cudaSuccess) { cudaGetLastError(); want = 0; }
-            }
-        }
-        DevBuf<unsigned char> d_send, d_recv; DevBuf<double> d_ok;
-        CU(d_send.alloc(sizeof(Handles))); CU(d_recv.alloc(sizeof(Handles) * (size_t)p->world)); CU(d_ok.alloc(1));
-        CU(cudaMemcpyAsync(d_send.p, &mine, sizeof mine, cudaMemcpyHostToDevice, p->stream));
-        std::vector<Handles> all((size_t)p->world);
-        if (g_nccl.AllGather) {
-            r = g_nccl.AllGather(d_send.p, d_recv.p, sizeof(Handles), ncclChar, p->comm, p->stream);
-            if (r != ncclSuccess) { set_err("ncclAllGather: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "error"); return AAR_ERR_COMM; }
-            CU(cudaMemcpyAsync(all.data(), d_recv.p, sizeof(Handles) * (size_t)p->world, cudaMemcpyDeviceToHost, p->stream));
-            CU(cudaStreamSynchronize(p->stream));
-        }
-        PeerDev pd; std::memset(&pd, 0, sizeof pd);
-        pd.world = p->world; pd.rank = p->rank;
-        if (want) {
-            for (int j = 0; j < p->world && want; j++) {
-                void *q_red = p->d_red.p, *q_small = p->d_peer_small.p, *q_flags = p->d_peer_flags.p;
-                if (j != p->rank) {
-                    if (cudaIpcOpenMemHandle(&q_red, all[(size_t)j].red, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { cudaGetLastError(); want = 0; break; }
-                    p->ipc_opened.push_back(q_red);
-                    if (cudaIpcOpenMemHandle(&q_small, all[(size_t)j].small, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { cudaGetLastError(); want = 0; break; }
-                    p->ipc_opened.push_back(q_small);
-                    if (cudaIpcOpenMemHandle(&q_flags, all[(size_t)j].flags, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { cudaGetLastError(); want = 0; break; }
-                    p->ipc_opened.push_back(q_flags);
-                }
-                pd.red[j] = (const double *)q_red; pd.small[j] = (double *)q_small;
-                pd.flagA[j] = (int *)q_flags; pd.flagB[j] = (int *)q_flags + PEER_MAX; pd.flagC[j] = (int *)q_flags + 2 * PEER_MAX;
-            }
-            pd.epoch = p->d_peer_flags.p + 3 * PEER_MAX; pd.Br_sum = p->d_Br_sum.p; pd.err = p->d_flag.p + 3;
-        }
-        // all ranks or none
-        double okv = want ? 1.0 : 0.0;
-        CU(cudaMemcpyAsync(d_ok.p, &okv, sizeof okv, cudaMemcpyHostToDevice, p->stream));
-        r = g_nccl.AllReduce(d_ok.p, d_ok.p, 1, ncclFloat64, ncclMin, p->comm, p->stream);
-        if (r != ncclSuccess) { set_err("ncclAllReduce: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "error"); return AAR_ERR_COMM; }
-        CU(cudaMemcpyAsync(&okv, d_ok.p, sizeof okv, cudaMemcpyDeviceToHost, p->stream));
-        CU(cudaStreamSynchronize(p->stream));
-        p->peer_ok = okv > 0.5;
-        if (p->peer_ok) p->pd = pd; else { p->pd.world = 1; p->pd.rank = 0; }
-    }
     return AAR_OK;
 }
 
 int64_t aar_kernel_launches(const aar_problem *p) { return p ? p->launches : 0; }
 int aar_problem_stats(const aar_problem *p, int64_t *out) {
     if (!p || !out) return AAR_ERR_INVALID;
-    out[0] = p->nslots; out[1] = p->npairs; out[2] = p->nmruns; out[3] = p->schur_fma; out[4] = (p->peer_ok ? 1 : 0) | (p->lm_graph_ok ? 2 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
+    out[0] = p->nslots; out[1] = p->npairs; out[2] = p->nmruns; out[3] = p->schur_fma; out[4] = (p->lm_graph_ok ? 2 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
     return AAR_OK;
 }
 int aar_set_profiling(aar_problem *p, int32_t on) { if (!p) return AAR_ERR_INVALID; p->profiling = on != 0; for (double &m : p->phase_ms) m = 0; p->track_ms = 0; p->track_runs = 0; return AAR_OK; }

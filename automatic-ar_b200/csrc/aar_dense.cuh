@@ -234,7 +234,7 @@ __device__ __forceinline__ void stage_tiles(double *dst, int ldd, const double *
 }
 
 __global__ void __launch_bounds__(CH_THREADS) k_reduced_solve_cluster2(int n /* even */, double *__restrict__ S, const double *__restrict__ b, double *__restrict__ x, const LmState *__restrict__ st,
-                                                                       int *__restrict__ chol_fail, double *__restrict__ Xinv /* [nblk][32][32] */, PeerDev pd) {
+                                                                       int *__restrict__ chol_fail, double *__restrict__ Xinv /* [nblk][32][32] */) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) double sm[];
     const int nblk = (n + CH_NB - 1) / CH_NB, LD = nblk * CH_NB + 2;
@@ -252,34 +252,17 @@ __global__ void __launch_bounds__(CH_THREADS) k_reduced_solve_cluster2(int n /* 
 #ifdef AAR_SOLVE_TIMING
     long long t_last = clock64(), tt[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 #endif
-    if (pd.world > 1) {
-        // sharded handle: the all-reduce of [S | b | Br] is this load phase — every rank's piece is read through NVLink peer memory and
-        // summed in rank order.  A: my piece is complete (the kernels before this one ran) -> wait until everybody's is.
-        if (tid == 0) { const int epoch = *pd.epoch; if (me == 0) peer_signal(pd.flagA, pd, epoch); peer_wait(pd.flagA[pd.rank], pd, epoch); }
-        __syncthreads();
-    }
-    const size_t nn = (size_t)n * n;
     for (int e = tid; e < CH_NB * nblk * CH_NB; e += CH_THREADS) {
         const int r = e % CH_NB, c = e / CH_NB, gr = me * CH_NB + r;
         double v = 0.0;
-        if (gr < n && c <= gr) {
-            if (pd.world > 1) { for (int j = 0; j < pd.world; j++) v += __ldcg(pd.red[j] + (size_t)c * n + gr); }
-            else v = S[(size_t)c * n + gr];
-            v += (c == gr ? mu : 0.0);
-        } else if (gr >= n && c == gr) v = 1.0;
+        if (gr < n && c <= gr) v = S[(size_t)c * n + gr] + (c == gr ? mu : 0.0);
+        else if (gr >= n && c == gr) v = 1.0;
         sRow[r * LD + c] = v;
     }
-    for (int e = tid; e < nblk * CH_NB; e += CH_THREADS) {
-        double v = 0.0;
-        if (e < n) { if (pd.world > 1) { for (int j = 0; j < pd.world; j++) v += __ldcg(pd.red[j] + nn + e); } else v = b[e]; }
-        sy[e] = v;
-    }
-    if (pd.world > 1 && me == 0)                          // the summed Br for the gain denominator (k_lm_decide)
-        for (int e = tid; e < n; e += CH_THREADS) { double v = 0.0; for (int j = 0; j < pd.world; j++) v += __ldcg(pd.red[j] + nn + n + e); pd.Br_sum[e] = v; }
+    for (int e = tid; e < nblk * CH_NB; e += CH_THREADS) sy[e] = e < n ? b[e] : 0.0;
     if (tid < CH_NB) ss[tid] = 0.0;
     SOLVE_T(0);
     cluster.sync();
-    if (pd.world > 1 && me == 0 && tid == 0) peer_signal(pd.flagB, pd, *pd.epoch);      // B: every CTA of this rank has read everybody's piece
     SOLVE_T(1);
     double acc0[2] = {0, 0}, acc1[2] = {0, 0};           // this warp's share of the update of tile (me, k + 1), carried across the barriers of step k
     for (int k = 0; k < nblk; k++) {

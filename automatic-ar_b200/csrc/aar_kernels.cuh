@@ -355,42 +355,6 @@ __global__ void k_maxdiag_frames(DevProblem p, const double *__restrict__ Hf, Lm
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// Sharded solves without a collective library inside the LM try: the per-rank pieces of the reduced system [S | b | Br] and of the
-// three scalars of the decision stay where their kernels left them and every rank SUMS ALL RANKS' COPIES ITSELF, through NVLink
-// peer memory (cudaIpc mappings of every rank's buffers), in rank order — so every rank holds bit-identical sums and takes the
-// same decisions.  The sum of S is the load phase of the reduced Cholesky (k_reduced_solve_cluster2), the sum of the scalars the
-// first lines of k_lm_decide: the all-reduce is fused into its consumers.  Ordering is three monotonic flag arrays per rank
-// (A: my S is complete, B: I have finished reading everybody's S, C: my scalars are published), written into the peers' memory and
-// spun on locally, with one epoch counter per LM try.
-constexpr int PEER_MAX = 8;
-struct PeerDev {
-    int world, rank;
-    const double *red[PEER_MAX];       // every rank's [S | b | Br]
-    double *small[PEER_MAX];           // every rank's scalars: [2 parities][4]  (trial cost, dd_f, dB_f, inexact-staging flag)
-    int *flagA[PEER_MAX], *flagB[PEER_MAX], *flagC[PEER_MAX];   // every rank's flag arrays [PEER_MAX]; index = WRITER's rank
-    int *epoch;                        // local: number of the current LM try
-    double *Br_sum;                    // local [n_r]: the summed Br for k_lm_decide
-    int *err;                          // local: set when a wait timed out (a peer died)
-};
-__device__ __forceinline__ void peer_signal(int *const *flags, const PeerDev &pd, int value) {      // one thread
-    __threadfence_system();
-    for (int j = 0; j < pd.world; j++) *reinterpret_cast<volatile int *>(flags[j] + pd.rank) = value;
-}
-__device__ __forceinline__ void peer_wait(const int *mine, const PeerDev &pd, int value) {          // one thread; mine = this rank's flag array
-    const long long t0 = clock64();
-    for (int j = 0; j < pd.world; j++)
-        while (*reinterpret_cast<const volatile int *>(mine + j) < value)
-            if (clock64() - t0 > 20000000000LL) { atomicExch(pd.err, 1); return; }                    // ~10 s: a peer is gone; the host reports AAR_ERR_COMM
-    __threadfence_system();
-}
-// start of an LM try on a sharded handle: nobody may still be reading this rank's S of the previous try
-__global__ void k_peer_begin_try(PeerDev pd) {
-    if (threadIdx.x || blockIdx.x) return;
-    peer_wait(pd.flagB[pd.rank], pd, *pd.epoch);
-    *pd.epoch += 1;
-}
-
 // One-thread control kernels -----------------------------------------------------------------
 // after the (all-reduced) normal equations of a new iteration are available
 __global__ void k_lm_begin_iter(LmState *st, int n_r, const double *__restrict__ Hrr_diag_src, int ld, double tau, double frames_maxdiag_global) {
@@ -402,34 +366,17 @@ __global__ void k_lm_begin_iter(LmState *st, int n_r, const double *__restrict__
     }
     st->tries = 0; st->accepted = 0; st->gain = 0;
 }
-// gain / accept / reject (sparselevmarq.h:402-419). red = [trial_cost, dd_f, dB_f] (all-reduced);
-// delta_r.delta_r and delta_r.Br are added here (identical on every rank).
-// the three scalars of the decision summed over the ranks through peer memory (rank order: identical on every rank)
-__device__ __forceinline__ void peer_sum_scalars(const PeerDev &pd, const double *red, int inexact, double &err, double &dd, double &dB, int &any_inexact) {
-    const int epoch = *pd.epoch, par = epoch & 1;
-    double *mine = pd.small[pd.rank] + 4 * par;
-    mine[0] = red[0]; mine[1] = red[1]; mine[2] = red[2]; mine[3] = inexact ? 1.0 : 0.0;
-    peer_signal(pd.flagC, pd, epoch);
-    peer_wait(pd.flagC[pd.rank], pd, epoch);
-    err = 0; dd = 0; dB = 0; double fl = 0;
-    for (int j = 0; j < pd.world; j++) {
-        const volatile double *v = pd.small[j] + 4 * par;
-        err += v[0]; dd += v[1]; dB += v[2]; fl += v[3];
-    }
-    any_inexact = fl != 0.0;
-}
-__global__ void k_lm_decide(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, const int *__restrict__ flags, PeerDev pd) {
-    if (threadIdx.x || blockIdx.x) return;
-    double err0 = red[0], dd = red[1], dB = red[2]; int inexact = flags[1];
-    if (pd.world > 1) { peer_sum_scalars(pd, red, flags[1], err0, dd, dB, inexact); Br = pd.Br_sum; }
-    if (inexact) { st->must_exit = -2; st->accepted = 0; return; }       // inexact float32 staging of this Jacobian (on any rank): decide nothing, the host redoes the iteration
-    st->trial_cost = err0;
+// gain / accept / reject of one try (sparselevmarq.h:402-419). red = [trial_cost, dd_f, dB_f] (all-reduced);
+// delta_r.delta_r and delta_r.Br are added here (identical on every rank).  Returns whether the trial point was accepted.
+__device__ __forceinline__ bool lm_decide_try(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br) {
+    double dd = red[1], dB = red[2];
     for (int i = 0; i < n_r; i++) { dd = fma(dr[i], dr[i], dd); dB = fma(dr[i], Br[i], dB); }
-    const double err = err0, mu = st->mu;
+    const double err = red[0], mu = st->mu;
     const double L = 0.5 * (mu * dd - dB);
     const double gain = (err - st->prev_cost) / L;
     st->L = L; st->gain = gain; st->trial_cost = err;
-    if (gain > 0 && ((err - st->prev_cost) < 0)) {
+    const bool accept = gain > 0 && ((err - st->prev_cost) < 0);
+    if (accept) {
         double t = 2 * gain - 1;
         st->mu = mu * fmax(0.33, 1. - t * t * t);
         st->v = 2.;
@@ -437,40 +384,30 @@ __global__ void k_lm_decide(LmState *st, const double *__restrict__ red, int n_r
         st->accepted = 1;
     } else { st->mu = mu * st->v; st->v = st->v * 5; }
     st->tries += 1;
+    return accept;
+}
+__global__ void k_lm_decide(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, const int *__restrict__ flags) {
+    if (threadIdx.x || blockIdx.x) return;
+    if (flags[1]) { st->must_exit = -2; st->accepted = 0; return; }       // inexact float32 staging of this Jacobian: decide nothing, the host redoes the iteration
+    lm_decide_try(st, red, n_r, dr, Br);
 }
 
 // ---- the same decisions without a host in the loop: CUDA-graph WHILE nodes whose conditions these kernels set -------------
 // start of an iteration (after J^T J): mu0 never needs computing here (the first iteration runs on the host path); an inexact
 // float32 staging (flags[1]) hands the iteration back to the host loop before any step is tried
-__global__ void k_lm_begin_iter_g(LmState *st, const int *__restrict__ flags, cudaGraphConditionalHandle inner, int sharded) {
+__global__ void k_lm_begin_iter_g(LmState *st, const int *__restrict__ flags, cudaGraphConditionalHandle inner) {
     if (threadIdx.x || blockIdx.x) return;
     st->tries = 0; st->accepted = 0; st->gain = 0;
-    const bool hand_back = !sharded && flags[1] != 0;        // sharded: the ranks must agree — the flag travels with the scalars of the first try (k_lm_decide_g)
+    const bool hand_back = flags[1] != 0;
     if (hand_back) st->must_exit = -2;
     cudaGraphSetConditional(inner, hand_back ? 0u : 1u);
 }
 // after a try: gain / accept / reject as k_lm_decide, then the do-while condition of sparselevmarq.h:384-419
-__global__ void k_lm_decide_g(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, cudaGraphConditionalHandle inner,
-                              const int *__restrict__ flags, PeerDev pd) {
+__global__ void k_lm_decide_g(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, cudaGraphConditionalHandle inner) {
     if (threadIdx.x || blockIdx.x) return;
-    double err0 = red[0], dd = red[1], dB = red[2]; int inexact = 0;
-    if (pd.world > 1) { peer_sum_scalars(pd, red, flags[1], err0, dd, dB, inexact); Br = pd.Br_sum; }
-    if (inexact) { st->must_exit = -2; st->accepted = 0; cudaGraphSetConditional(inner, 0u); return; }
-    for (int i = 0; i < n_r; i++) { dd = fma(dr[i], dr[i], dd); dB = fma(dr[i], Br[i], dB); }
-    const double err = err0, mu = st->mu;
-    const double L = 0.5 * (mu * dd - dB);
-    const double gain = (err - st->prev_cost) / L;
-    st->L = L; st->gain = gain; st->trial_cost = err;
-    if (gain > 0 && ((err - st->prev_cost) < 0)) {
-        double t = 2 * gain - 1;
-        st->mu = mu * fmax(0.33, 1. - t * t * t);
-        st->v = 2.;
-        st->cost = err;
-        st->accepted = 1;
-        st->huber_eval = st->huber_delta;
-    } else { st->mu = mu * st->v; st->v = st->v * 5; }
-    st->tries += 1; st->total_tries += 1;
-    cudaGraphSetConditional(inner, (gain <= 0 && st->tries <= 5 && !st->accepted) ? 1u : 0u);
+    if (lm_decide_try(st, red, n_r, dr, Br)) st->huber_eval = st->huber_delta;
+    st->total_tries += 1;
+    cudaGraphSetConditional(inner, (st->gain <= 0 && st->tries <= 5 && !st->accepted) ? 1u : 0u);
 }
 // accepted trial point becomes the iterate (the host path swaps two pointers instead)
 __global__ void k_lm_commit(const LmState *__restrict__ st, long long n, const double *__restrict__ zt, double *__restrict__ z) {

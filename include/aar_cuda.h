@@ -33,7 +33,7 @@ enum {
     AAR_ERR_INVALID = 1,      /* bad argument / inconsistent description */
     AAR_ERR_CUDA = 2,         /* CUDA runtime error (no device, launch failure, out of memory) */
     AAR_ERR_UNSUPPORTED = 3,  /* e.g. a non-pinhole camera matrix, more than 4095 cameras */
-    AAR_ERR_COMM = 4,         /* NCCL error, or a peer rank that stopped answering the peer-memory reduction */
+    AAR_ERR_COMM = 4,         /* NCCL error */
     AAR_ERR_NUMERIC = 5       /* non-finite cost or non-positive Cholesky pivot */
 };
 
@@ -193,9 +193,7 @@ int aar_row_map(const aar_problem_desc *desc, int64_t capacity, int32_t *obs_fra
                 int32_t *obs_has_jacobian, int64_t *num_observations);
 
 /* multi-GPU (one process per GPU of one box): one handle per rank; id is the 128-byte ncclUniqueId created on rank 0.  Per LM try the
- * reduced system and three scalars are all-reduced with NCCL.  With AAR_PEER=1 in the environment aar_comm_init also maps every rank's
- * reduced system through cudaIpc and the all-reduce is fused into its consumers instead (the reduced Cholesky sums all ranks' pieces over
- * NVLink peer memory while loading them; no collective-library call inside the try, graph-resident loop on sharded handles). */
+ * reduced system and three scalars are all-reduced with NCCL. */
 int aar_comm_unique_id(void *id128);
 int aar_comm_init(aar_problem *p, const void *id128);
 
@@ -208,7 +206,7 @@ int aar_comm_init(aar_problem *p, const void *id128);
 #define AAR_NUM_PHASES 12
 int64_t aar_kernel_launches(const aar_problem *p);
 /* sizes of this rank's shard: [0] W slots  [1] (frame, camera) pairs  [2] (frame, marker) runs  [3] fused multiply-adds of the upper
- * triangle of the Schur update S -= E E^T per try  [4] bit 0: peer-memory reduction active (sharded handles), bit 1: graph-resident loop built, bits 8..: LM iterations run inside the graph  [5] most blocks seen by one frame  [6] [7] frame index range */
+ * triangle of the Schur update S -= E E^T per try  [4] bit 0: always 0, bit 1: graph-resident loop built, bits 8..: LM iterations run inside the graph  [5] most blocks seen by one frame  [6] [7] frame index range */
 int aar_problem_stats(const aar_problem *p, int64_t *out /* [8] */);
 int aar_set_profiling(aar_problem *p, int32_t on);
 int aar_get_phase_ms(const aar_problem *p, double *ms /* [AAR_NUM_PHASES] */);

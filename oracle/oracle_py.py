@@ -85,6 +85,7 @@ class Oracle:
         self.L.aar_oracle_set_sincos_mode(C.c_int(mode))
 
     def set_config(self, cams=True, markers=True, objects=True, intrinsics=False, with_huber=False, huber_delta=2.5):
+        self.cams, self.markers = bool(cams), bool(markers)
         self.L.aar_oracle_set_config(self.h, C.c_int(cams), C.c_int(markers), C.c_int(objects), C.c_int(intrinsics),
                                      C.c_int(with_huber), C.c_float(huber_delta))
 
@@ -135,7 +136,7 @@ class Oracle:
 
     def reduced_system(self, z, mu, f_lo=0, f_hi=None):
         z = np.ascontiguousarray(z, dtype=np.float64)
-        n_r = 6 * (self.nC - 1) + 6 * (self.nM - 1)
+        n_r = 6 * (self.nC - 1 if self.cams else 0) + 6 * (self.nM - 1 if self.markers else 0)      # the hook sizes S from the Config
         S = np.zeros((n_r, n_r)); b = np.zeros(n_r); cost = C.c_double(0)
         rc = self.L.aar_oracle_reduced_system(self.h, _ptr(z, _dp), C.c_double(mu), C.c_int(f_lo), C.c_int(self.nF if f_hi is None else f_hi),
                                               _ptr(S, _dp), _ptr(b, _dp), C.byref(cost))

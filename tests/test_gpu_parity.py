@@ -374,11 +374,21 @@ def test_exact_staging_fallback_matches(binding, oracle_mod, monkeypatch):
     assert np.abs(S32[iu] - S64[iu]).max() <= 1e-13 * np.abs(S64).max() and np.abs(b32 - b64).max() <= 1e-13 * np.abs(b64).max()
 
 
-def test_tensor_core_assembly_matches_oracle_and_legacy_kernel(binding, oracle_mod, monkeypatch):
+def _normal_equations(o, z):
+    """S = J^T J and b = -J^T r with nothing eliminated (objects=False: every column is a camera or marker column), from the
+    oracle's bit-exact Jacobian and residuals; the cost is r^T r."""
+    import scipy.sparse
+    colptr, rowidx, vals = o.jacobian(z)
+    r = o.error(z)
+    J = scipy.sparse.csc_matrix((vals, rowidx, colptr), shape=(len(r), o.num_vars))
+    return (J.T @ J).toarray(), -(J.T @ r), float(r @ r)
+
+
+def test_tensor_core_assembly_matches_oracle(binding, oracle_mod):
     """k_asm_pairs + k_asm_mruns (FP64 tensor cores, one warp per (frame, camera) pair / (frame, marker) run, aar_assemble.cuh)
-    against the oracle's normal equations and against the round-1 lane-per-observation kernel (AAR_ASM=legacy), which sums the
-    same products in another order: on a rig with duplicated detections, an emptied frame, root camera / marker observations,
-    with and without Huber weights, and for every Config flag combination."""
+    against the oracle's normal equations, which sum the same products in another order: on a rig with duplicated detections,
+    an emptied frame, root camera / marker observations, with and without Huber weights, and for every Config flag combination.
+    With the frames optimised the oracle eliminates them itself; without, S and b are J^T J and -J^T r of its Jacobian."""
     rig = small_rig(seed=31, F=120)
     # duplicated (frame, cam, marker) detections (only the last one has Jacobian rows) and a frame that loses all its rows
     dup = np.array([5, 40, 41], np.int64)
@@ -390,20 +400,16 @@ def test_tensor_core_assembly_matches_oracle_and_legacy_kernel(binding, oracle_m
         for cams, markers, objects in [(True, True, True), (False, True, True), (True, False, True), (True, True, False)]:
             o = oracle_mod.Oracle(rig); o.set_config(cams=cams, markers=markers, objects=objects, with_huber=huber, huber_delta=2.5)
             z0 = o.mats2evec()
-            kw = dict(cams=cams, markers=markers, objects=objects, with_huber=huber)
-            monkeypatch.delenv("AAR_ASM", raising=False)
-            S1, b1, c1 = binding.Problem(rig, **kw).reduced_system(z0, 5.0)
-            monkeypatch.setenv("AAR_ASM", "legacy")
-            S0, b0, c0 = binding.Problem(rig, **kw).reduced_system(z0, 5.0)
-            monkeypatch.delenv("AAR_ASM", raising=False)
-            iu = np.triu_indices(len(b0))
-            if len(b0):
-                assert np.abs(S1[iu] - S0[iu]).max() <= 1e-12 * np.abs(S0).max() and np.abs(b1 - b0).max() <= 1e-12 * np.abs(b0).max(), (huber, cams, markers, objects)
-            assert abs(c1 - c0) <= 1e-13 * c0
-            if cams and markers and objects:          # the oracle's reduced_system hook is written for the full Config
-                S_o, b_o, _ = o.reduced_system(z0, 5.0)
-                if len(b0):
-                    assert np.abs(S1[iu] - S_o[iu]).max() <= 1e-10 * np.abs(S_o).max() and np.abs(b1 - b_o).max() <= 1e-10 * np.abs(b_o).max(), (huber, cams, markers, objects)
+            S_g, b_g, c_g = binding.Problem(rig, cams=cams, markers=markers, objects=objects, with_huber=huber).reduced_system(z0, 5.0)
+            S_o, b_o, c_o = o.reduced_system(z0, 5.0) if objects else _normal_equations(o, z0)
+            assert S_g.shape == S_o.shape and len(b_g) > 0
+            iu = np.triu_indices(len(b_g))
+            dS = np.abs(S_g[iu] - S_o[iu]).max() / np.abs(S_o).max()
+            db = np.abs(b_g - b_o).max() / np.abs(b_o).max()
+            dc = abs(c_g - c_o) / c_o
+            parity_record("tensor_core_assembly_vs_oracle", huber=huber, cams=cams, markers=markers, objects=objects, n_r=len(b_g),
+                          rel_dev_S=dS, rel_dev_b=db, rel_dev_cost=dc, bar_S_b=1e-12, bar_cost=1e-13)
+            assert dS <= 1e-12 and db <= 1e-12 and dc <= 1e-13, (huber, cams, markers, objects, dS, db, dc)
 
 
 # ------------------------------------------------------------------ camera-intrinsics block (SURVEY 8(f) row 4)

@@ -1,5 +1,5 @@
 #!/bin/bash
-# cfg 3 (8 cameras, 24 markers, 10 k frames) sharded over the GPUs of this box; on 2 GPUs also the multi-GPU parity test (NCCL and peer-memory paths)
+# cfg 3 (8 cameras, 24 markers, 10 k frames) sharded over the GPUs of this box; on 2 GPUs also the multi-GPU parity test
 cd "${GRAFT_REPO_ROOT:-.}"; mkdir -p gpurun_out
 export AAR_RIG_CACHE=/tmp/rigs
 N=$(nvidia-smi -L | wc -l)
