@@ -112,26 +112,24 @@ struct aar_problem {
     DevBuf<double> d_z, d_zt, d_z0, d_Hf, d_W, d_Hrr, d_gr, d_red, d_dr, d_red3, d_tmp, d_r, d_J;
     DevBuf<LmState> d_st;
     DevBuf<int> d_flag;
-    LmState *h_st = nullptr; double *h_red3 = nullptr; int *h_flags = nullptr; // pinned
+    LmState *h_st = nullptr; double *h_red3 = nullptr; int *h_flags = nullptr; // pinned; h_st: LM state as last read back or pushed
     // ---- staged rows of central-difference numerators ([N][JROW] float32, or float64 in the exact fallback) and Huber weights ([N][4])
     DevBuf<float> d_Jn32; DevBuf<double> d_Jn64, d_Rv;
     int max_ms = 0, num_sms = 148; size_t smem_optin = 227 * 1024;
     bool use_cluster_solve = true;
     int force_exact_staging = 0; long long exact_reruns = 0;
     DevProblem dp{};
-    // ---- LM host mirror
+    // ---- LM
     aar_lm_params params{};
     bool lm_active = false, have_z0 = false;
-    float huber_cur = 2.5f, huber_eval = 2.5f;
-    double prev_cost = 0, cost = 0, initial_cost = 0;
-    int iter = 0; int exit_code = 0; long long total_tries = 0;
+    double initial_cost = 0;
     // ---- comm
     ncclComm_t comm = nullptr;
     // ---- instrumentation
     long long launches = 0; bool profiling = false; bool exact_next = false;   // exact_next: redo this Jacobian with FP64 staging
-    // graph-resident LM loop (aar_lm_iterate): two nested WHILE nodes, conditions set by k_lm_decide_g / k_lm_iter_end_g
+    // graph-resident LM loop (aar_lm_iterate): two nested WHILE nodes, conditions set by k_lm_begin_iter / k_lm_decide / k_lm_next_iter_g
     cudaGraph_t lm_graph = nullptr; cudaGraphExec_t lm_exec = nullptr; cudaGraphConditionalHandle lm_outer = 0, lm_inner = 0; cudaStream_t lm_side = nullptr;
-    bool lm_graph_tried = false, lm_graph_ok = false, capturing = false; long long lm_graph_launches = 0, lm_graph_iters = 0; int lm_body_launches = 0, lm_try_launches = 0;
+    bool lm_graph_tried = false, lm_graph_ok = false; long long lm_graph_launches = 0, lm_graph_iters = 0; int lm_body_launches = 0, lm_try_launches = 0;
     DevBuf<LmTraceDev> d_trace;
     // aar_error_report (aar_report.cuh): observation errors, entity statistics [C + M + F], select state [2 nq], digit histograms [nq][SEL_BINS]
     DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
@@ -314,9 +312,8 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, double *Jdump, bool de
         else { if (p->d_Jn32.n < JROW * Np) CU(p->d_Jn32.alloc(JROW * Np)); rc = launch_jacobian<float>(p, huber_eval, p->d_Jn32.p); }
         if (rc) return rc;
         if (exact) { p->exact_next = false; break; }
-        // graph-resident loop: k_lm_begin_iter_g looks at the flag on the device and hands the iteration back; host-driven LM loop: k_lm_decide
-        // refuses the step of an inexact staging and the flag arrives with the state of the try (no synchronisation of its own)
-        if (p->capturing || defer_check) break;
+        // LM loops: k_lm_begin_iter looks at the flag on the device and leaves the iteration undecided (no synchronisation of its own)
+        if (defer_check) break;
         // the float32 staging of the numerators is exact unless the kernel says otherwise (never seen on real data)
         CU(cudaMemcpyAsync(p->h_flags, p->d_flag.p, 4 * sizeof(int), cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
@@ -395,6 +392,58 @@ int fetch_state(aar_problem *p) {
 }
 int push_state(aar_problem *p) {
     CU(cudaMemcpyAsync(p->d_st.p, p->h_st, sizeof(LmState), cudaMemcpyHostToDevice, p->stream));
+    return AAR_OK;
+}
+
+// ---- the two halves of an LM iteration, launched by the host-driven loop and captured into the graph-resident one (`graph`).
+// The residual and Jacobian kernels take hubberDelta from the device state (dp.st_dev); the Huber arguments below only reach
+// the analytic variant, which runs on the host-driven loop, where h_st is current.
+
+// J^T J blocks and J^T r at z (sparselevmarq.h:353-367), then k_lm_begin_iter.  The first iteration of a solve (never inside
+// the graph) computes mu0 = tau * max diag(JtJ) (sparselevmarq.h:369-377).
+int lm_jacobian_phase(aar_problem *p, bool graph) {
+    const int n_r = p->n_r;
+    int rc;
+    prof_mark(p, 0);
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, nullptr, true))) return rc;
+    prof_mark(p, 1);
+    const double *diag = p->d_Hrr.p; int ld = n_r; double frames_maxdiag = 0.0;
+    if (p->h_st->mu < 0) {
+        p->h_st->maxdiag = -1e300; push_state(p);
+        if (p->opt_f && p->dp.F > 0) LAUNCH(p, k_maxdiag_frames, cdiv(p->dp.F, 128), 128, 0, p->dp, p->d_Hf.p, p->d_st.p);
+        if (p->comm) {
+            // global diagonal of Hrr (sum) into d_tmp and global frame maximum
+            double *tmp = p->d_tmp.p;
+            if (n_r) CU(cudaMemcpy2DAsync(tmp, sizeof(double), p->d_Hrr.p, (size_t)(n_r + 1) * sizeof(double), sizeof(double), (size_t)n_r, cudaMemcpyDeviceToDevice, p->stream));
+            if ((rc = allreduce(p, tmp, (size_t)n_r, ncclSum))) return rc;
+            if ((rc = allreduce(p, &p->d_st.p->maxdiag, 1, ncclMax))) return rc;
+            diag = tmp; ld = 0;
+        }
+        if ((rc = fetch_state(p))) return rc;
+        frames_maxdiag = p->h_st->maxdiag;
+    }
+    LAUNCH(p, k_lm_begin_iter, 1, 1, 0, p->d_st.p, n_r, diag, ld, p->params.tau, frames_maxdiag, p->d_flag.p, (int)graph, p->lm_inner);
+    return AAR_OK;
+}
+
+// one try of the do-while of SparseLevMarq::step (sparselevmarq.h:384-419): damped solve, back substitution, cost at the trial
+// point, the decision and the commit of an accepted trial point
+int lm_try(aar_problem *p, bool graph) {
+    const int n_r = p->n_r;
+    const double *Br = p->d_red.p + (size_t)n_r * n_r + n_r;
+    int rc;
+    CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
+    prof_mark(p, 2);
+    if ((rc = build_and_solve_reduced(p))) return rc;
+    prof_mark(p, 3);
+    if (p->opt_f && p->dp.F > 0)
+        LAUNCH(p, k_backsub, std::max(1, std::min(4 * p->num_sms, (int)cdiv(p->dp.F, BS_WARPS))), BS_WARPS * 32, 0, p->dp, p->d_fc.p, p->d_Hf.p, p->d_W.p, p->d_dr.p, p->d_z.p, p->d_zt.p, p->d_red3.p);
+    prof_mark(p, 4);
+    residual(p, p->d_zt.p, p->h_st->huber_delta, nullptr);
+    prof_mark(p, 5);
+    if ((rc = allreduce(p, p->d_red3.p, 3, ncclSum))) return rc;
+    LAUNCH(p, k_lm_decide, 1, 1, 0, p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->d_flag.p, (int)graph, p->lm_inner);
+    LAUNCH(p, k_lm_commit, std::max(1, std::min(2 * p->num_sms, (int)cdiv(p->n_vars, 256))), 256, 0, p->d_st.p, p->n_vars, p->d_zt.p, p->d_z.p);
     return AAR_OK;
 }
 
@@ -593,6 +642,8 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
     if (d->stream) p->stream = (cudaStream_t)d->stream; else { CU(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking)); p->own_stream = true; }
     for (auto &e : p->ev) CU(cudaEventCreate(&e));
     CU(cudaMallocHost((void **)&p->h_st, sizeof(LmState)));
+    std::memset(p->h_st, 0, sizeof(LmState));
+    p->h_st->huber_eval = 2.5f;      // the parity hooks evaluate with the Huber delta of the last accepted evaluation: 2.5 before any solve
     CU(cudaMallocHost((void **)&p->h_red3, 8 * sizeof(double)));
     CU(cudaMallocHost((void **)&p->h_flags, 4 * sizeof(int)));
     {
@@ -1024,7 +1075,7 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
     const size_t nj = 144 * (size_t)std::max<long long>(p->N, 1);
     if (p->d_J.n < nj) CU(p->d_J.alloc(nj));
-    if ((rc = jacobian_accumulate(p, p->huber_eval, p->d_J.p))) return rc;
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, p->d_J.p))) return rc;
     std::vector<double> J(nj), Ji(p->opt_i ? 32 * (size_t)std::max<long long>(p->N, 1) : 0);
     CU(cudaMemcpyAsync(J.data(), p->d_J.p, nj * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     if (p->opt_i && p->N > 0) CU(cudaMemcpyAsync(Ji.data(), p->d_Ji.p, 32 * (size_t)p->N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
@@ -1064,8 +1115,8 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
     CU(cudaSetDevice(p->device));
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-    residual(p, p->d_z.p, p->huber_eval, nullptr);
-    if ((rc = jacobian_accumulate(p, p->huber_eval, nullptr))) return rc;
+    residual(p, p->d_z.p, p->h_st->huber_eval, nullptr);
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, nullptr))) return rc;
     p->h_st->mu = mu; push_state(p);
     const int n_r = p->n_r;
     double *dS = p->d_red.p;
@@ -1094,34 +1145,41 @@ int aar_lm_begin(aar_problem *p, const double *z0, const aar_lm_params *params) 
     } else if (p->n_vars > 0) // restart from the starting point that is already resident on the device
         CU(cudaMemcpyAsync(p->d_z.p, p->d_z0.p, (size_t)p->n_vars * sizeof(double), cudaMemcpyDeviceToDevice, p->stream));
     // MultiCamMapper::solve: hubberDelta = 10 before the solver starts (multicam_mapper.cpp:425)
-    p->huber_cur = 10.f; p->huber_eval = 10.f;
+    const float huber0 = 10.f;
     CU(cudaMemsetAsync(p->d_flag.p, 0, 4 * sizeof(int), p->stream));
     // SparseLevMarq::init (sparselevmarq.h:237-249)
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-    residual(p, p->d_z.p, p->huber_cur, nullptr);
+    residual(p, p->d_z.p, huber0, nullptr);
     if ((rc = allreduce(p, p->d_red3.p, 1, ncclSum))) return rc;
     CU(cudaMemcpyAsync(p->h_red3, p->d_red3.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     CU(cudaStreamSynchronize(p->stream));
     CU(cudaGetLastError());
-    std::memset(p->h_st, 0, sizeof(LmState));
-    p->cost = p->prev_cost = p->initial_cost = p->h_red3[0];
-    p->h_st->cost = p->cost; p->h_st->prev_cost = p->prev_cost; p->h_st->mu = -1; p->h_st->v = 2; // v: uninitialised in the reference (sparselevmarq.h:133)
+    const aar_lm_params &P = p->params;
+    LmState &h = *p->h_st;
+    std::memset(&h, 0, sizeof(LmState));
+    h.cost = h.prev_cost = p->initial_cost = p->h_red3[0];
+    h.mu = -1; h.v = 2;       // v: uninitialised in the reference (sparselevmarq.h:133)
+    h.huber_delta = h.huber_eval = huber0;
+    h.ignore_stop = P.ignore_stop_rules; h.min_error = P.min_error; h.min_step = P.min_step_error_diff; h.min_avg = P.min_average_step_error_diff;
+    h.rows = (double)(8 * p->N);
     if ((rc = push_state(p))) return rc;
-    p->iter = 0; p->exit_code = 0; p->total_tries = 0; p->lm_active = true;
-    if (!std::isfinite(p->cost)) { set_err("initial cost is not finite"); return AAR_ERR_NUMERIC; }
+    p->lm_active = true;
+    if (!std::isfinite(h.cost)) { set_err("initial cost is not finite"); return AAR_ERR_NUMERIC; }
     return AAR_OK;
 }
 
 
-// ------------------------------------------------------------------------------- graph-resident LM loop ----
-// SparseLevMarq::solve (sparselevmarq.h:439-472) with the do-while of step() (:384-419) as two nested CUDA-graph WHILE nodes:
-//   WHILE outer { J^T J assembly; k_lm_begin_iter_g; WHILE inner { Schur + reduced solve + back substitution + trial residual;
-//                 k_lm_decide_g; k_lm_commit }; k_lm_iter_end_g }
-// Nothing returns to the host between the launch of the graph and its end: the accept / reject decision, the damping update,
-// the stop rules, the hubberDelta annealing and the per-iteration trace all live in LmState on the device.  The first LM iteration
-// of a solve always runs on the host-driven path (it sizes the scratch buffers and computes mu0, which needs a MAX all-reduce
-// when sharded); sharded handles (NCCL inside a conditional body), profiling and verbose mode stay on the host-driven path.
-constexpr int LM_TRACE_DEV_CAP = 4096;
+// ------------------------------------------------------------------------------- LM loops ----
+// aar_lm_iterate runs SparseLevMarq::solve (sparselevmarq.h:439-472) in one of two ways.  Both launch the same kernels in the same
+// order: lm_jacobian_phase, then lm_try until k_lm_decide says that no try follows (the do-while of step(), :384-419).  Every
+// decision (accept / reject, damping, stop rules, hubberDelta annealing, the record of an iteration) is made on the device, in LmState.
+//  - Graph-resident: two nested CUDA-graph WHILE nodes whose conditions the control kernels set,
+//      WHILE outer { lm_jacobian_phase; WHILE inner { lm_try }; k_lm_next_iter_g }
+//    Nothing returns to the host between the launch of the graph and its end.
+//  - Host-driven: the same two functions launched from the host, with one read-back of LmState per try.  It runs the first
+//    iteration of a solve (it sizes the scratch buffers and computes mu0, which needs a MAX all-reduce when sharded), the FP64 redo
+//    of an iteration whose float32 staging was inexact, sharded handles (NCCL inside a conditional body), the analytic variant,
+//    profiling, verbose mode, AAR_FORCE_EXACT_STAGING=1 and AAR_NO_GRAPH=1.
 #define GR(call)                                                                                          \
     do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { set_err("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); ok = false; goto done; } } while (0)
 
@@ -1130,8 +1188,6 @@ static bool lm_graph_build(aar_problem *p) {
     bool ok = true;
     cudaStream_t main_stream = p->stream;
     const long long launches_before = p->launches;
-    const int n_r = p->n_r;
-    double *S = p->d_red.p, *Br = S + (size_t)n_r * n_r + n_r;
     cudaGraph_t body_outer = nullptr, body_inner = nullptr, tmp = nullptr;
     cudaGraphNode_t node_outer, node_inner;
     bool cap_outer = false, cap_inner = false;
@@ -1147,10 +1203,8 @@ static bool lm_graph_build(aar_problem *p) {
     np.type = cudaGraphNodeTypeConditional; np.conditional.handle = p->lm_outer; np.conditional.type = cudaGraphCondTypeWhile; np.conditional.size = 1;
     GR(cudaGraphAddNode(&node_outer, p->lm_graph, nullptr, 0, &np));
     body_outer = np.conditional.phGraph_out[0];
-    p->capturing = true; p->dp.st_dev = p->d_st.p;
     GR(cudaStreamBeginCaptureToGraph(main_stream, body_outer, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed)); cap_outer = true;
-    if (jacobian_accumulate(p, 0.f, nullptr)) { ok = false; goto done; }
-    k_lm_begin_iter_g<<<1, 1, 0, main_stream>>>(p->d_st.p, p->d_flag.p, p->lm_inner); p->launches++;
+    if (lm_jacobian_phase(p, true)) { ok = false; goto done; }
     // the inner WHILE node goes in by hand, behind everything captured so far; the capture continues behind it
     GR(cudaStreamGetCaptureInfo_v2(main_stream, &cs, nullptr, &cg, &deps, &ndeps));
     std::memset(&ni, 0, sizeof ni);
@@ -1163,19 +1217,11 @@ static bool lm_graph_build(aar_problem *p) {
     l0 = p->launches;
     p->stream = p->lm_side;
     GR(cudaStreamBeginCaptureToGraph(p->lm_side, body_inner, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed)); cap_inner = true;
-    GR(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-    if (build_and_solve_reduced(p)) { ok = false; goto done; }
-    if (p->opt_f && p->dp.F > 0) {
-        k_backsub<<<std::max(1, std::min(4 * p->num_sms, (int)cdiv(p->dp.F, BS_WARPS))), BS_WARPS * 32, 0, p->stream>>>(p->dp, p->d_fc.p, p->d_Hf.p, p->d_W.p, p->d_dr.p, p->d_z.p, p->d_zt.p, p->d_red3.p);
-        p->launches++;
-    }
-    residual(p, p->d_zt.p, 0.f, nullptr);
-    k_lm_decide_g<<<1, 1, 0, p->stream>>>(p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->lm_inner); p->launches++;
-    k_lm_commit<<<std::max(1, std::min(2 * p->num_sms, (int)cdiv(p->n_vars, 256))), 256, 0, p->stream>>>(p->d_st.p, p->n_vars, p->d_zt.p, p->d_z.p); p->launches++;
+    if (lm_try(p, true)) { ok = false; goto done; }
     GR(cudaStreamEndCapture(p->lm_side, &tmp)); cap_inner = false;
     p->stream = main_stream;
     p->lm_try_launches = (int)(p->launches - l0);
-    k_lm_iter_end_g<<<1, 1, 0, main_stream>>>(p->d_st.p, p->d_flag.p, p->d_trace.p, p->lm_outer); p->launches++;
+    LAUNCH(p, k_lm_next_iter_g, 1, 1, 0, p->d_st.p, p->d_trace.p, p->lm_outer);
     p->lm_body_launches += 1;
     GR(cudaStreamEndCapture(main_stream, &tmp)); cap_outer = false;
     GR(cudaGraphInstantiate(&p->lm_exec, p->lm_graph, 0));
@@ -1183,7 +1229,6 @@ done:
     p->stream = main_stream;
     if (cap_inner) { cudaStreamEndCapture(p->lm_side, &tmp); }
     if (cap_outer) { cudaStreamEndCapture(main_stream, &tmp); }
-    p->capturing = false; p->dp.st_dev = nullptr;
     p->launches = launches_before;                       // capture is not execution
     if (!ok) { cudaGetLastError(); if (p->lm_exec) { cudaGraphExecDestroy(p->lm_exec); p->lm_exec = nullptr; } }
     p->lm_graph_ok = ok;
@@ -1191,179 +1236,113 @@ done:
 }
 #undef GR
 
-// runs up to `iters` LM iterations inside the graph; one host synchronisation at the end
-static int lm_graph_run(aar_problem *p, int iters, aar_lm_report *rep, int *iters_done, int *must_exit) {
-    const aar_lm_params &P = p->params;
+// up to `iters` LM iterations inside the graph; one host synchronisation at the end
+static int lm_graph_run(aar_problem *p, int iters, aar_lm_report *rep) {
     LmState &h = *p->h_st;
-    h.huber_delta = p->huber_cur; h.huber_eval = p->huber_eval;
-    h.iters_done = 0; h.max_iters = iters; h.must_exit = 0; h.ignore_stop = P.ignore_stop_rules;
-    h.min_error = P.min_error; h.min_step = P.min_step_error_diff; h.min_avg = P.min_average_step_error_diff; h.rows = (double)(8 * p->N);
-    h.total_tries = 0; h.trace_cap = LM_TRACE_DEV_CAP; h.trace_len = 0;
-    h.cost = p->cost; h.prev_cost = p->prev_cost;
+    const int iter0 = h.iter; const long long tries0 = h.total_tries;
+    h.max_iters = h.iter + iters; h.trace_len = 0;
     int rc;
     if ((rc = push_state(p))) return rc;
     CU(cudaGraphLaunch(p->lm_exec, p->stream));
     if ((rc = fetch_state(p))) return rc;                    // the one synchronisation of the call
     CU(cudaGetLastError());
-    p->lm_graph_launches++; p->lm_graph_iters += h.iters_done;
-    p->launches += (long long)h.iters_done * p->lm_body_launches + h.total_tries * p->lm_try_launches + (h.must_exit == -2 ? p->lm_body_launches : 0);
-    p->total_tries += h.total_tries; p->iter += h.iters_done;
-    p->cost = h.cost; p->prev_cost = h.prev_cost; p->huber_cur = h.huber_delta; p->huber_eval = h.huber_eval;
+    p->lm_graph_launches++; p->lm_graph_iters += h.iter - iter0;
+    p->launches += (long long)(h.iter - iter0) * p->lm_body_launches + (h.total_tries - tries0) * p->lm_try_launches + (h.must_exit == -2 ? p->lm_body_launches : 0);
     if (rep && rep->trace && h.trace_len > 0 && rep->trace_len < rep->trace_capacity) {
         const int n = std::min(h.trace_len, rep->trace_capacity - rep->trace_len);
-        static_assert(sizeof(LmTraceDev) == sizeof(aar_lm_trace), "trace layouts differ");
         CU(cudaMemcpyAsync(rep->trace + rep->trace_len, p->d_trace.p, (size_t)n * sizeof(aar_lm_trace), cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
         rep->trace_len += n;
     }
-    *iters_done = h.iters_done; *must_exit = h.must_exit;
+    return AAR_OK;
+}
+
+// one LM iteration with the host in the loop: one read-back of the state per try
+static int lm_host_iteration(aar_problem *p, aar_lm_report *rep) {
+    static_assert(sizeof(LmTraceDev) == sizeof(aar_lm_trace), "trace layouts differ");
+    LmState &h = *p->h_st;
+    const double prev_cost = h.prev_cost;
+    int rc;
+    if ((rc = lm_jacobian_phase(p, false))) return rc;
+    for (int ntries = 0;; ntries++) {
+        if ((rc = lm_try(p, false))) return rc;
+        if ((rc = fetch_state(p))) return rc;
+        prof_mark(p, 6);
+        CU(cudaGetLastError());
+        if (p->profiling) {
+            cudaEventSynchronize(p->ev[6]);
+            float ms;
+            if (ntries == 0) {
+                cudaEventElapsedTime(&ms, p->ev[0], p->ev[1]); p->phase_ms[0] += ms;
+                cudaEventElapsedTime(&ms, p->ev[7], p->ev[9]); p->phase_ms[5] += ms; p->phase_ms[6] += 1;
+                cudaEventElapsedTime(&ms, p->ev[9], p->ev[8]); p->phase_ms[7] += ms;
+                if (p->npairs > 0) { cudaEventElapsedTime(&ms, p->ev[9], p->ev[12]); p->phase_ms[10] += ms; cudaEventElapsedTime(&ms, p->ev[12], p->ev[8]); p->phase_ms[11] += ms; }
+            }
+            if (p->opt_f && p->dp.F > 0 && p->n_r > 0 && p->nslots > 0) { cudaEventElapsedTime(&ms, p->ev[10], p->ev[11]); p->phase_ms[8] += ms; p->phase_ms[9] += 1; }
+            cudaEventElapsedTime(&ms, p->ev[2], p->ev[3]); p->phase_ms[1] += ms;
+            cudaEventElapsedTime(&ms, p->ev[3], p->ev[4]); p->phase_ms[2] += ms;
+            cudaEventElapsedTime(&ms, p->ev[4], p->ev[5]); p->phase_ms[3] += ms;
+            cudaEventElapsedTime(&ms, p->ev[5], p->ev[6]); p->phase_ms[4] += ms;
+        }
+        if (!h.more_tries) break;
+    }
+    if (h.must_exit >= 0) {                              // the iteration completed: h.last is its record
+        const LmTraceDev &t = h.last;
+        if (p->params.verbose)
+            printf("Curr Error=%.5g AErr(prev-curr)=%.5g gain=%.5g dumping factor=%.5g\n", t.cost, (prev_cost - t.cost) / h.rows, t.gain, t.mu);
+        if (rep && rep->trace && rep->trace_len < rep->trace_capacity) std::memcpy(&rep->trace[rep->trace_len++], &t, sizeof(aar_lm_trace));
+    }
+    return AAR_OK;
+}
+
+// the error of a numeric stop (must_exit = -1), from the flags read back with the state
+static int lm_numeric_error(aar_problem *p) {
+    // flags[0]: a non-positive pivot in a frame block or in the reduced system (the kernels substituted 1 to keep going):
+    //   the step that was just taken is not the solution of the damped normal equations.  The reference does not check
+    //   its LDLT (sparselevmarq.h:394-400) and would continue on garbage; this path stops and says so.
+    // flags[2]: the rotation of a translation-perturbed inverse camera pose differed from the unperturbed one, so the
+    //   translation-only camera variants of k_expand_jac do not reproduce cv::Mat::inv() bit for bit.
+    const int *flags = p->h_flags;
+    set_err(flags[0] ? "non-positive Cholesky pivot at iteration %d (damped normal equations not positive definite)"
+                     : flags[2] ? "camera inverse of a translation-perturbed pose changed its rotation at iteration %d (bit-exact table assumption violated)"
+                                : "non-finite cost at iteration %d", p->h_st->iter);
+    CU(cudaMemsetAsync(p->d_flag.p, 0, 4 * sizeof(int), p->stream));
+    return AAR_ERR_NUMERIC;
+}
+
+static int lm_iterate(aar_problem *p, int max_iters, aar_lm_report *rep) {
+    LmState &h = *p->h_st;
+    const int iter0 = h.iter;
+    const char *no_graph = getenv("AAR_NO_GRAPH");           // development aid: host-driven loop only
+    const bool graph_eligible = !p->comm && !p->profiling && !p->params.verbose && !p->force_exact_staging && !p->analytic && !(no_graph && *no_graph == '1') && p->dp.N > 0;
+    h.must_exit = 0;
+    while (h.must_exit == 0 && h.iter - iter0 < max_iters) {
+        int rc;
+        if (graph_eligible && h.mu >= 0 && !p->exact_next && (p->lm_graph_ok || (!p->lm_graph_tried && lm_graph_build(p))))
+            rc = lm_graph_run(p, std::min(max_iters - (h.iter - iter0), LM_TRACE_DEV_CAP), rep);
+        else
+            rc = lm_host_iteration(p, rep);
+        if (rc) return rc;
+        if (h.must_exit == -1) return lm_numeric_error(p);
+        if (h.must_exit == -2) {     // inexact float32 staging: nothing was decided; redo the iteration with FP64 staging (never seen on real data)
+            p->exact_reruns++; p->exact_next = true; h.must_exit = 0;
+            CU(cudaMemsetAsync(p->d_flag.p + 1, 0, sizeof(int), p->stream));
+        }
+    }
+    if (rep) { rep->final_cost = h.cost; rep->iterations = h.iter - iter0; rep->exit_code = h.must_exit; rep->total_tries = h.total_tries; }
     return AAR_OK;
 }
 
 int aar_lm_iterate(aar_problem *p, int32_t max_iters, aar_lm_report *rep) {
     if (!p || !p->lm_active) { set_err("aar_lm_iterate without aar_lm_begin"); return AAR_ERR_INVALID; }
     CU(cudaSetDevice(p->device));
-    const aar_lm_params &P = p->params;
-    const int n_r = p->n_r;
-    const long long rows = 8 * p->N;
-    int rc;
-    int done_iters = 0; int mustExit = 0;
     if (rep) { rep->trace_len = 0; rep->initial_cost = p->initial_cost; }
-    double *S = p->d_red.p, *b = S + (size_t)n_r * n_r, *Br = b + n_r;
-    const char *no_graph = getenv("AAR_NO_GRAPH");           // development aid: host-driven loop only
-    const bool graph_eligible = !p->comm && !p->profiling && !P.verbose && !p->force_exact_staging && !p->analytic && !(no_graph && *no_graph == '1') && p->dp.N > 0;
-    for (int it = 0; it < max_iters && !mustExit; it++) {
-        if (graph_eligible && p->h_st->mu >= 0 && (p->lm_graph_ok || !p->lm_graph_tried)) {
-            // every iteration but the first of a solve: inside the graph, without the host (see lm_graph_build)
-            if (!p->lm_graph_tried) lm_graph_build(p);
-            if (p->lm_graph_ok) {
-                int gd = 0, gx = 0;
-                const int want = std::min(max_iters - it, LM_TRACE_DEV_CAP);
-                if ((rc = lm_graph_run(p, want, rep, &gd, &gx))) { p->lm_active = false; return rc; }
-                done_iters += gd;
-                if (gx == -1) {
-                    int flags[4];
-                    CU(cudaMemcpy(flags, p->d_flag.p, sizeof flags, cudaMemcpyDeviceToHost));
-                    set_err(flags[0] ? "non-positive Cholesky pivot at iteration %d (damped normal equations not positive definite)"
-                                     : flags[2] ? "camera inverse of a translation-perturbed pose changed its rotation at iteration %d (bit-exact table assumption violated)"
-                                                : "non-finite cost at iteration %d", p->iter);
-                    CU(cudaMemsetAsync(p->d_flag.p, 0, 4 * sizeof(int), p->stream));
-                    p->lm_active = false;
-                    return AAR_ERR_NUMERIC;
-                }
-                if (gx > 0) { mustExit = gx; break; }
-                it += gd;
-                if (it >= max_iters) break;
-                if (gx == 0) { it--; continue; }              // the graph ran its share of the trace buffer: go again
-                // gx == -2: the float32 staging was inexact in this iteration; it is redone below on the host path (FP64 staging)
-            }
-        }
-        // ---- J, JtJ blocks, B (sparselevmarq.h:353-367)
-        prof_mark(p, 0);
-            if ((rc = jacobian_accumulate(p, p->huber_eval, nullptr, true))) { p->lm_active = false; return rc; }
-        prof_mark(p, 1);
-        if (p->h_st->mu < 0) { // first iteration: mu = tau * max diag(JtJ) (sparselevmarq.h:369-377)
-            p->h_st->maxdiag = -1e300; push_state(p);
-            if (p->opt_f && p->dp.F > 0) LAUNCH(p, k_maxdiag_frames, cdiv(p->dp.F, 128), 128, 0, p->dp, p->d_Hf.p, p->d_st.p);
-            double *tmp = p->d_tmp.p; // [n_r diag | maxdiag]
-            if (p->comm) {
-                // global diagonal of Hrr (sum) and global frame maximum
-                if (n_r) CU(cudaMemcpy2DAsync(tmp, sizeof(double), p->d_Hrr.p, (size_t)(n_r + 1) * sizeof(double), sizeof(double), (size_t)n_r, cudaMemcpyDeviceToDevice, p->stream));
-                if ((rc = allreduce(p, tmp, (size_t)n_r, ncclSum))) return rc;
-                if ((rc = allreduce(p, &p->d_st.p->maxdiag, 1, ncclMax))) return rc;
-                if ((rc = fetch_state(p))) return rc;
-                LAUNCH(p, k_lm_begin_iter, 1, 1, 0, p->d_st.p, n_r, tmp, 0, P.tau, p->h_st->maxdiag);
-            } else {
-                if ((rc = fetch_state(p))) return rc;
-                LAUNCH(p, k_lm_begin_iter, 1, 1, 0, p->d_st.p, n_r, p->d_Hrr.p, n_r, P.tau, p->h_st->maxdiag);
-            }
-        } else LAUNCH(p, k_lm_begin_iter, 1, 1, 0, p->d_st.p, n_r, p->d_Hrr.p, n_r, P.tau, 0.0);
-        // ---- damping / solve / evaluate / accept-or-reject (sparselevmarq.h:384-419)
-        int ntries = 0; bool accepted = false; double gain = 0;
-        do {
-            CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-            prof_mark(p, 2);
-            if ((rc = build_and_solve_reduced(p))) return rc;
-            prof_mark(p, 3);
-            if (p->opt_f && p->dp.F > 0)
-                LAUNCH(p, k_backsub, std::max(1, std::min(4 * p->num_sms, (int)cdiv(p->dp.F, BS_WARPS))), BS_WARPS * 32, 0, p->dp, p->d_fc.p, p->d_Hf.p, p->d_W.p, p->d_dr.p, p->d_z.p, p->d_zt.p, p->d_red3.p);
-            prof_mark(p, 4);
-            residual(p, p->d_zt.p, p->huber_cur, nullptr);
-            prof_mark(p, 5);
-            if ((rc = allreduce(p, p->d_red3.p, 3, ncclSum))) return rc;
-            LAUNCH(p, k_lm_decide, 1, 1, 0, p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->d_flag.p);
-            // an accepted trial point becomes the iterate by a device copy (a pointer swap would invalidate the captured graph of the resident loop)
-            LAUNCH(p, k_lm_commit, std::max(1, std::min(2 * p->num_sms, (int)cdiv(p->n_vars, 256))), 256, 0, p->d_st.p, p->n_vars, p->d_zt.p, p->d_z.p);
-            if ((rc = fetch_state(p))) return rc;
-            prof_mark(p, 6);
-            CU(cudaGetLastError());
-            if (p->h_st->must_exit == -2) break;          // inexact float32 staging: nothing was decided, the iteration is redone below
-            p->total_tries++;
-            gain = p->h_st->gain;
-            accepted = p->h_st->accepted != 0;
-            if (accepted) { p->cost = p->h_st->cost; p->huber_eval = p->huber_cur; }
-            if (p->profiling) {
-                cudaEventSynchronize(p->ev[6]);
-                float ms;
-                if (ntries == 0) {
-                    cudaEventElapsedTime(&ms, p->ev[0], p->ev[1]); p->phase_ms[0] += ms;
-                    cudaEventElapsedTime(&ms, p->ev[7], p->ev[9]); p->phase_ms[5] += ms; p->phase_ms[6] += 1;
-                    cudaEventElapsedTime(&ms, p->ev[9], p->ev[8]); p->phase_ms[7] += ms;
-                    if (p->npairs > 0) { cudaEventElapsedTime(&ms, p->ev[9], p->ev[12]); p->phase_ms[10] += ms; cudaEventElapsedTime(&ms, p->ev[12], p->ev[8]); p->phase_ms[11] += ms; }
-                }
-                if (p->opt_f && p->dp.F > 0 && p->n_r > 0 && p->nslots > 0) { cudaEventElapsedTime(&ms, p->ev[10], p->ev[11]); p->phase_ms[8] += ms; p->phase_ms[9] += 1; }
-                cudaEventElapsedTime(&ms, p->ev[2], p->ev[3]); p->phase_ms[1] += ms;
-                cudaEventElapsedTime(&ms, p->ev[3], p->ev[4]); p->phase_ms[2] += ms;
-                cudaEventElapsedTime(&ms, p->ev[4], p->ev[5]); p->phase_ms[3] += ms;
-                cudaEventElapsedTime(&ms, p->ev[5], p->ev[6]); p->phase_ms[4] += ms;
-            }
-        } while (gain <= 0 && ntries++ < 5 && !accepted);
-        if (p->h_st->must_exit == -2) {                   // redo this iteration with FP64 staging of the numerators (never seen on real data)
-            p->exact_reruns++; p->exact_next = true;
-            p->h_st->must_exit = 0;
-            CU(cudaMemsetAsync(p->d_flag.p + 1, 0, sizeof(int), p->stream));
-            if ((rc = push_state(p))) return rc;
-            it--; continue;
-        }
-        const int *flags = p->h_flags;                    // fetched with the state of the last try
-        if (!std::isfinite(p->h_st->trial_cost)) { set_err("non-finite cost at iteration %d", p->iter); p->lm_active = false; return AAR_ERR_NUMERIC; }
-        if (flags[0] || flags[2]) {
-            // flags[0]: a non-positive pivot in a frame block or in the reduced system (the kernels substituted 1 to keep going):
-            //   the step that was just taken is not the solution of the damped normal equations.  The reference does not check
-            //   its LDLT (sparselevmarq.h:394-400) and would continue on garbage; this path stops and says so.
-            // flags[2]: the rotation of a translation-perturbed inverse camera pose differed from the unperturbed one, so the
-            //   translation-only camera variants of k_expand_jac do not reproduce cv::Mat::inv() bit for bit.
-            set_err(flags[0] ? "non-positive Cholesky pivot at iteration %d (damped normal equations not positive definite)"
-                             : "camera inverse of a translation-perturbed pose changed its rotation at iteration %d (bit-exact table assumption violated)", p->iter);
-            CU(cudaMemsetAsync(p->d_flag.p, 0, 4 * sizeof(int), p->stream));
-            p->lm_active = false;
-            return AAR_ERR_NUMERIC;
-        }
-        // ---- exit tests of SparseLevMarq::solve (sparselevmarq.h:458-464)
-        const double currErr = p->cost, prevErr = p->prev_cost;
-        if (!P.ignore_stop_rules) {
-            if (currErr < P.min_error) mustExit = 1;
-            if (std::fabs(prevErr - currErr) <= P.min_step_error_diff || std::fabs((prevErr - currErr) / (double)rows) <= P.min_average_step_error_diff || !accepted) mustExit = 2;
-            if (currErr > prevErr) mustExit = 3;
-        }
-        if (P.verbose)
-            printf("Curr Error=%.5g AErr(prev-curr)=%.5g gain=%.5g dumping factor=%.5g\n", currErr, (prevErr - currErr) / (double)rows, gain, p->h_st->mu);
-        if (rep && rep->trace && rep->trace_len < rep->trace_capacity) {
-            aar_lm_trace &t = rep->trace[rep->trace_len++];
-            t.cost = currErr; t.mu = p->h_st->mu; t.gain = gain; t.tries = p->h_st->tries; t.accepted = accepted; t.huber_delta = p->huber_cur;
-        }
-        // step callback: MultiCamMapper::optCallBack (multicam_mapper.cpp:412-417)
-        if (p->huber_cur > 2.5f) p->huber_cur = (float)((double)p->huber_cur - 7.5 / 500);
-        p->prev_cost = currErr;
-        p->h_st->prev_cost = currErr; p->h_st->cost = currErr;
-        if ((rc = push_state(p))) return rc;
-        p->iter++; done_iters++;
-    }
-    p->exit_code = mustExit;
-    if (rep) { rep->final_cost = p->cost; rep->iterations = done_iters; rep->exit_code = mustExit; rep->total_tries = p->total_tries; }
-    return AAR_OK;
+    p->dp.st_dev = p->d_st.p;
+    const int rc = lm_iterate(p, max_iters, rep);
+    p->dp.st_dev = nullptr;                              // the evaluation hooks obey their Huber argument
+    if (rc) p->lm_active = false;
+    return rc;
 }
-
 int aar_lm_end(aar_problem *p, double *z_out) {
     if (!p || !p->lm_active) return AAR_ERR_INVALID;
     CU(cudaSetDevice(p->device));

@@ -14,19 +14,23 @@ constexpr int FC_STRIDE_K = 28;  // per frame: packed lower Cholesky factor of H
 
 // Everything the kernels need, by value.
 // ---------------------------------------------------------------------------------------------
-// LM state, device resident (sparselevmarq.h:130-135, 237-249).
+struct LmTraceDev { double cost, mu, gain; int tries, accepted; float huber_delta; int pad; };   // == aar_lm_trace (include/aar_cuda.h)
+constexpr int LM_TRACE_DEV_CAP = 4096;   // records of one launch of the graph-resident loop
+// LM state, device resident (sparselevmarq.h:130-135, 237-249): the only copy of the solver's state (the host's h_st is its last
+// read-back).  The solve, residual and Jacobian kernels read mu, maxdiag, huber_delta, huber_eval and accepted at these offsets.
 struct LmState {
     double cost, prev_cost, trial_cost, mu, v, gain, L;
     double maxdiag;          // local max diagonal of JtJ (first iteration)
     float huber_delta, huber_eval;   // hubberDelta of the next evaluation / the one the accepted iterate was evaluated with (multicam_mapper.cpp:412-417)
-    int accepted, tries, iter, exit_code, chol_fail, pad;
-    // ---- control block of the graph-resident loop (aar_lm_iterate: SparseLevMarq::solve, sparselevmarq.h:439-472, without a host in it)
-    int iters_done, max_iters, must_exit /* 0 run | 1..3 stop rules | -1 numeric | -2 hand back to the host loop */, ignore_stop;
+    int accepted, tries;
+    int iter;                // iterations completed since aar_lm_begin
+    int more_tries;          // the do-while of step() (sparselevmarq.h:384-419) runs another try
+    int must_exit;           // 0 run | 1..3 stop rules | -1 numeric | -2 inexact float32 staging: redo the iteration with FP64 staging
+    int ignore_stop, max_iters /* the graph-resident loop stops at this iteration count */, trace_len /* records in its trace */;
     double min_error, min_step, min_avg, rows;
-    long long total_tries;
-    int trace_cap, trace_len;
+    long long total_tries;   // tries since aar_lm_begin
+    LmTraceDev last;         // record of the last completed iteration
 };
-struct LmTraceDev { double cost, mu, gain; int tries, accepted; float huber_delta; int pad; };   // == aar_lm_trace (include/aar_cuda.h)
 
 struct DevProblem {
     int C, M, F;                 // cameras, markers, LOCAL frames (this rank's shard)
@@ -48,7 +52,7 @@ struct DevProblem {
     const float4 *und_a, *und_b, *raw_a, *raw_b; // x0 y0 x1 y1 | x2 y2 x3 y3
     double *intr;                // [C][4] fx cx fy cy at z (constant unless the intrinsics are optimised: then written by k_expand_intr)
     double *intr_tr;             // the same at the trial point (k_residual); == intr when the intrinsics are fixed
-    const LmState *st_dev;       // graph-resident loop: the Huber delta comes from the device state instead of the launch parameter (null otherwise)
+    const LmState *st_dev;       // inside aar_lm_iterate: the Huber delta comes from the device state instead of the launch parameter (null otherwise)
     int opt_i, nri, col_intr0;   // intrinsics optimised; 2 C pseudo-blocks behind the pose blocks; their first column in the internal z (aar_intrinsics.cuh)
     // frame CSR of W slots: per frame the camera blocks seen (in order of first appearance), then the marker blocks
     const int *frame_slot_ptr;   // [F+1]
@@ -355,16 +359,21 @@ __global__ void k_maxdiag_frames(DevProblem p, const double *__restrict__ Hf, Lm
     }
 }
 
-// One-thread control kernels -----------------------------------------------------------------
-// after the (all-reduced) normal equations of a new iteration are available
-__global__ void k_lm_begin_iter(LmState *st, int n_r, const double *__restrict__ Hrr_diag_src, int ld, double tau, double frames_maxdiag_global) {
+// One-thread control kernels of SparseLevMarq::solve (sparselevmarq.h:439-472), launched by both LM loops of aar_lm_iterate;
+// inside the CUDA graph (`graph` != 0) they also set the conditions of its WHILE nodes.
+// Start of an iteration, after the (all-reduced) normal equations: mu0 (first iteration only, sparselevmarq.h:369-377), reset.
+// An inexact float32 staging of this Jacobian (flags[1]) leaves the iteration undecided (must_exit = -2): no try is decided.
+__global__ void k_lm_begin_iter(LmState *st, int n_r, const double *__restrict__ Hrr_diag_src, int ld, double tau, double frames_maxdiag_global,
+                                const int *__restrict__ flags, int graph, cudaGraphConditionalHandle inner) {
     if (threadIdx.x || blockIdx.x) return;
-    if (st->mu < 0) { // first time only (sparselevmarq.h:369-377)
+    if (st->mu < 0) {
         double m = frames_maxdiag_global;
         for (int i = 0; i < n_r; i++) m = fmax(m, Hrr_diag_src[(size_t)i * ld + i]);
         st->mu = m * tau;
     }
     st->tries = 0; st->accepted = 0; st->gain = 0;
+    st->must_exit = flags[1] ? -2 : 0;
+    if (graph) cudaGraphSetConditional(inner, st->must_exit == 0 ? 1u : 0u);
 }
 // gain / accept / reject of one try (sparselevmarq.h:402-419). red = [trial_cost, dd_f, dB_f] (all-reduced);
 // delta_r.delta_r and delta_r.Br are added here (identical on every rank).  Returns whether the trial point was accepted.
@@ -386,57 +395,49 @@ __device__ __forceinline__ bool lm_decide_try(LmState *st, const double *__restr
     st->tries += 1;
     return accept;
 }
-__global__ void k_lm_decide(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, const int *__restrict__ flags) {
-    if (threadIdx.x || blockIdx.x) return;
-    if (flags[1]) { st->must_exit = -2; st->accepted = 0; return; }       // inexact float32 staging of this Jacobian: decide nothing, the host redoes the iteration
-    lm_decide_try(st, red, n_r, dr, Br);
-}
-
-// ---- the same decisions without a host in the loop: CUDA-graph WHILE nodes whose conditions these kernels set -------------
-// start of an iteration (after J^T J): mu0 never needs computing here (the first iteration runs on the host path); an inexact
-// float32 staging (flags[1]) hands the iteration back to the host loop before any step is tried
-__global__ void k_lm_begin_iter_g(LmState *st, const int *__restrict__ flags, cudaGraphConditionalHandle inner) {
-    if (threadIdx.x || blockIdx.x) return;
-    st->tries = 0; st->accepted = 0; st->gain = 0;
-    const bool hand_back = flags[1] != 0;
-    if (hand_back) st->must_exit = -2;
-    cudaGraphSetConditional(inner, hand_back ? 0u : 1u);
-}
-// after a try: gain / accept / reject as k_lm_decide, then the do-while condition of sparselevmarq.h:384-419
-__global__ void k_lm_decide_g(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, cudaGraphConditionalHandle inner) {
-    if (threadIdx.x || blockIdx.x) return;
-    if (lm_decide_try(st, red, n_r, dr, Br)) st->huber_eval = st->huber_delta;
-    st->total_tries += 1;
-    cudaGraphSetConditional(inner, (st->gain <= 0 && st->tries <= 5 && !st->accepted) ? 1u : 0u);
-}
-// accepted trial point becomes the iterate (the host path swaps two pointers instead)
-__global__ void k_lm_commit(const LmState *__restrict__ st, long long n, const double *__restrict__ zt, double *__restrict__ z) {
-    if (!st->accepted) return;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) z[i] = zt[i];
-}
-// end of an iteration: stop rules of SparseLevMarq::solve (sparselevmarq.h:453-465), trace, step callback (hubberDelta annealing)
-__global__ void k_lm_iter_end_g(LmState *st, int *__restrict__ flags, LmTraceDev *__restrict__ trace, cudaGraphConditionalHandle outer) {
-    if (threadIdx.x || blockIdx.x) return;
-    if (st->must_exit == -2) { cudaGraphSetConditional(outer, 0u); return; }
+// end of an iteration (sparselevmarq.h:453-465): a non-finite cost, a non-positive pivot (flags[0]) or a broken camera table
+// assumption (flags[2]) stop with must_exit = -1 and no record; otherwise stop rules, record, step callback (multicam_mapper.cpp:412-417)
+__device__ __forceinline__ void lm_end_iter(LmState *st, const int *__restrict__ flags) {
+    if (!(st->trial_cost - st->trial_cost == 0.0) || flags[0] || flags[2]) { st->must_exit = -1; return; }
     const double currErr = st->cost, prevErr = st->prev_cost;
     int mustExit = 0;
-    if (!(st->trial_cost - st->trial_cost == 0.0) || flags[0] || flags[2]) mustExit = -1;      // non-finite cost, non-positive pivot, camera table assumption
-    else if (!st->ignore_stop) {
+    if (!st->ignore_stop) {
         if (currErr < st->min_error) mustExit = 1;
         if (fabs(prevErr - currErr) <= st->min_step || fabs((prevErr - currErr) / st->rows) <= st->min_avg || !st->accepted) mustExit = 2;
         if (currErr > prevErr) mustExit = 3;
     }
-    if (mustExit >= 0 && st->trace_len < st->trace_cap) {
-        LmTraceDev &t = trace[st->trace_len++];
-        t.cost = currErr; t.mu = st->mu; t.gain = st->gain; t.tries = st->tries; t.accepted = st->accepted; t.huber_delta = st->huber_delta; t.pad = 0;
-    }
-    if (mustExit >= 0) {
-        if (st->huber_delta > 2.5f) st->huber_delta = (float)((double)st->huber_delta - 7.5 / 500);
-        st->prev_cost = currErr; st->cost = currErr;
-        st->iters_done += 1;
-    }
+    LmTraceDev &t = st->last;
+    t.cost = currErr; t.mu = st->mu; t.gain = st->gain; t.tries = st->tries; t.accepted = st->accepted; t.huber_delta = st->huber_delta; t.pad = 0;
+    if (st->huber_delta > 2.5f) st->huber_delta = (float)((double)st->huber_delta - 7.5 / 500);
+    st->prev_cost = currErr; st->cost = currErr;
+    st->iter += 1;
     st->must_exit = mustExit;
-    cudaGraphSetConditional(outer, (mustExit == 0 && st->iters_done < st->max_iters) ? 1u : 0u);
+}
+
+// after a try: its decision, the do-while condition of step() (sparselevmarq.h:384-419) and, when no try follows, the end of the
+// iteration.  A try after an inexact staging (must_exit = -2, host-driven loop only) is not decided.
+__global__ void k_lm_decide(LmState *st, const double *__restrict__ red, int n_r, const double *__restrict__ dr, const double *__restrict__ Br, const int *__restrict__ flags,
+                            int graph, cudaGraphConditionalHandle inner) {
+    if (threadIdx.x || blockIdx.x) return;
+    st->more_tries = 0;
+    if (st->must_exit != -2) {
+        if (lm_decide_try(st, red, n_r, dr, Br)) st->huber_eval = st->huber_delta;
+        st->total_tries += 1;
+        st->more_tries = st->gain <= 0 && st->tries <= 5 && !st->accepted;
+        if (!st->more_tries) lm_end_iter(st, flags);
+    }
+    if (graph) cudaGraphSetConditional(inner, st->more_tries ? 1u : 0u);
+}
+// accepted trial point becomes the iterate (a pointer swap would invalidate the captured graph of the resident loop)
+__global__ void k_lm_commit(const LmState *__restrict__ st, long long n, const double *__restrict__ zt, double *__restrict__ z) {
+    if (!st->accepted) return;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) z[i] = zt[i];
+}
+// graph-resident loop only, after the inner WHILE node: the record of a completed iteration into the trace, the outer condition
+__global__ void k_lm_next_iter_g(LmState *st, LmTraceDev *__restrict__ trace, cudaGraphConditionalHandle outer) {
+    if (threadIdx.x || blockIdx.x) return;
+    if (st->must_exit >= 0 && st->trace_len < LM_TRACE_DEV_CAP) trace[st->trace_len++] = st->last;
+    cudaGraphSetConditional(outer, (st->must_exit == 0 && st->iter < st->max_iters) ? 1u : 0u);
 }
 
 // one-off device undistortion pass — cv::undistortPoints(..., K, dist, noArray, K) as called by

@@ -475,35 +475,40 @@ def test_intrinsics_block_lm_steps_and_solve(binding, oracle_mod):
     _end_point_bar(d_cost, env_c, 2e-5)
 
 
+# bars of a comparison of two LM runs that take the same decisions (also used by test_gpu_lm_loop.py)
+def _same(a, b, tol=1e-9):
+    a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
+    return a.shape == b.shape and np.abs(a - b).max() <= tol * max(np.abs(b).max(), 1e-300)
+
+
+def _same_cost(plain, z_g, c_g, z_h, c_h):
+    """The cost sums squares of residuals of float32-rounded projections (multicam_mapper.cpp:644-648): where the two iterates
+    differ in the last bits, a projection may round to the neighbouring float and move its row's square by a float32 step.  The
+    costs agree to 1e-12 beyond what the rows that round differently at the two iterates account for (Huber weights are <= 1)."""
+    r_g, _ = plain.residual(z_g); r_h, _ = plain.residual(z_h)
+    flips = r_g != r_h
+    return abs(c_g - c_h) <= 1e-12 * c_h + np.abs(r_g[flips] ** 2 - r_h[flips] ** 2).sum(), int(flips.sum())
+
+
+def _end_point_dev(p, z0, z_g, z_h):
+    """Relative distance of the two end points of a full solve, and the bar it passed.  1e-9 unless a quantised Jacobian entry
+    rounded differently on the way: two runs of the SAME loop then also land on end points 7e-9 apart at cfg2 (measured on the
+    B200: identical iterations, tries, damping and Huber schedule; the order of the FP64 atomic sums decides which end point), so a
+    larger distance must lie within 4 x how far the end point moves under a 1e-13 relative change of z0 (_oracle_envelope), and 1e-6."""
+    dz = np.abs(z_g - z_h).max() / np.abs(z_h).max()
+    if dz <= 1e-9:
+        return dz, "1e-9"
+    rng = np.random.default_rng(123)
+    env = max(np.abs(p.solve(z0 * (1 + 1e-13 * rng.standard_normal(z0.shape)))[0] - z_h).max() / np.abs(z_h).max() for _ in range(3))
+    assert 0 < env and dz <= min(4 * env, 1e-6), (dz, env)
+    return dz, "envelope %.2e" % env
+
+
 def test_graph_resident_loop_equals_host_driven_loop(binding, oracle_mod, monkeypatch):
     """aar_lm_iterate runs SparseLevMarq::solve as nested CUDA-graph WHILE nodes (decisions on the device); AAR_NO_GRAPH=1 keeps the
     host-driven loop (one read-back per try).  Same kernels in the same order: iteration and try counts must be identical and
     iterates, costs and damping equal up to the order of the atomic sums of the assembly (two runs of the SAME loop differ in the last
     bits too), with and without Huber (the hubberDelta annealing lives in the device state)."""
-    def same(a, b, tol=1e-9):
-        a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
-        return a.shape == b.shape and np.abs(a - b).max() <= tol * max(np.abs(b).max(), 1e-300)
-
-    def same_cost(plain, z_g, c_g, z_h, c_h):
-        """The cost sums squares of residuals of float32-rounded projections (multicam_mapper.cpp:644-648): where the two iterates
-        differ in the last bits, a projection may round to the neighbouring float and move its row's square by a float32 step.  The
-        costs agree to 1e-12 beyond what the rows that round differently at the two iterates account for (Huber weights are <= 1)."""
-        r_g, _ = plain.residual(z_g); r_h, _ = plain.residual(z_h)
-        flips = r_g != r_h
-        return abs(c_g - c_h) <= 1e-12 * c_h + np.abs(r_g[flips] ** 2 - r_h[flips] ** 2).sum(), int(flips.sum())
-
-    def end_point_dev(p, z0, z_g, z_h):
-        """Relative distance of the two end points of a full solve, and the bar it passed.  1e-9 unless a quantised Jacobian entry
-        rounded differently on the way: two runs of the SAME loop then also land on end points 7e-9 apart at cfg2 (measured on the
-        B200: identical iterations, tries, damping and Huber schedule; the order of the FP64 atomic sums decides which end point), so a
-        larger distance must lie within 4 x how far the end point moves under a 1e-13 relative change of z0 (_oracle_envelope), and 1e-6."""
-        dz = np.abs(z_g - z_h).max() / np.abs(z_h).max()
-        if dz <= 1e-9:
-            return dz, "1e-9"
-        rng = np.random.default_rng(123)
-        env = max(np.abs(p.solve(z0 * (1 + 1e-13 * rng.standard_normal(z0.shape)))[0] - z_h).max() / np.abs(z_h).max() for _ in range(3))
-        assert 0 < env and dz <= min(4 * env, 1e-6), (dz, env)
-        return dz, "envelope %.2e" % env
     flips_seen = 0; end_points = {}
     for name, huber in (("cfg1", False), ("cfg2", False), ("cfg1", True)):
         rig = synth.make_config(name)
@@ -515,10 +520,10 @@ def test_graph_resident_loop_equals_host_driven_loop(binding, oracle_mod, monkey
         monkeypatch.delenv("AAR_NO_GRAPH")
         l0 = p.kernel_launches
         z_g, c_g, it_g, tr_g = p.solve(z0)
-        cost_ok, flips = same_cost(plain, z_g, c_g, z_h, c_h); flips_seen += flips
+        cost_ok, flips = _same_cost(plain, z_g, c_g, z_h, c_h); flips_seen += flips
         assert it_g == it_h and cost_ok, (name, huber, it_g, it_h, c_g, c_h, flips)
-        end_points[name + ("_huber" if huber else "")] = end_point_dev(p, z0, z_g, z_h)
-        assert np.array_equal(tr_g[:, 3:5], tr_h[:, 3:5]) and same(tr_g[:, 0], tr_h[:, 0]) and same(tr_g[:, 1], tr_h[:, 1], 1e-7) and np.array_equal(tr_g[:, 5], tr_h[:, 5])
+        end_points[name + ("_huber" if huber else "")] = _end_point_dev(p, z0, z_g, z_h)
+        assert np.array_equal(tr_g[:, 3:5], tr_h[:, 3:5]) and _same(tr_g[:, 0], tr_h[:, 0]) and _same(tr_g[:, 1], tr_h[:, 1], 1e-7) and np.array_equal(tr_g[:, 5], tr_h[:, 5])
         assert p.kernel_launches > l0
         # a capped number of iterations and the stop rules switched off (the bench's mode)
         prm = binding.Problem.default_params(max_iters=7, ignore_stop_rules=1)
@@ -526,8 +531,8 @@ def test_graph_resident_loop_equals_host_driven_loop(binding, oracle_mod, monkey
         z_h, c_h, it_h, tr_h = p.solve(z0, prm)
         monkeypatch.delenv("AAR_NO_GRAPH")
         z_g, c_g, it_g, tr_g = p.solve(z0, prm)
-        cost_ok, flips = same_cost(plain, z_g, c_g, z_h, c_h); flips_seen += flips
-        assert it_g == it_h == 7 and cost_ok and same(z_g, z_h) and np.array_equal(tr_g[:, 3:6], tr_h[:, 3:6]), (name, huber, c_g, c_h, flips)
+        cost_ok, flips = _same_cost(plain, z_g, c_g, z_h, c_h); flips_seen += flips
+        assert it_g == it_h == 7 and cost_ok and _same(z_g, z_h) and np.array_equal(tr_g[:, 3:6], tr_h[:, 3:6]), (name, huber, c_g, c_h, flips)
         plain.close()
     parity_record("graph_resident_loop_vs_host_driven_loop", same_iterations_tries_huber=True, rel_tol_z=1e-9, rel_tol_cost=1e-12,
                   rows_rounding_differently=flips_seen, full_solve_end_point_rel_dev=end_points, workloads=["cfg1", "cfg2", "cfg1 + Huber"])
