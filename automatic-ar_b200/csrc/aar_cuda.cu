@@ -13,6 +13,7 @@
 #include <unistd.h>
 #include <map>
 #include <memory>
+#include <mutex>
 #include <numeric>
 #include <string>
 #include <thread>
@@ -117,6 +118,7 @@ struct aar_problem {
     DevBuf<float> d_Jn32; DevBuf<double> d_Jn64, d_Rv;
     int max_ms = 0, num_sms = 148; size_t smem_optin = 227 * 1024;
     bool use_cluster_solve = true;
+    bool last_cluster_solve = false, last_smem_acc = false, last_cm_rep = false;   // paths of the last reduced solve and assembly (aar_problem_stats)
     int force_exact_staging = 0; long long exact_reruns = 0;
     DevProblem dp{};
     // ---- LM
@@ -221,6 +223,38 @@ int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_ou
 
 void prof_mark(aar_problem *p, int i) { if (p->profiling) cudaEventRecord(p->ev[i], p->stream); }
 
+// Dynamic shared-memory caps, set once per device for every kernel launched with more than 48 KB.  A function attribute holds for
+// the whole process on a device: a cap sized for one handle would make the larger launches of another, earlier handle fail.  So
+// every cap is the most the device allows next to the kernel's static shared memory.  The cap reserves nothing: occupancy follows
+// the size a launch asks for.  *cluster_ok: the cluster Cholesky may run on this device.
+template <typename K> cudaError_t cap_dynamic_smem(K *kernel, size_t smem_optin) {
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem_optin - a.sharedSizeBytes));
+}
+int set_smem_caps(aar_problem *p, bool *cluster_ok) {
+    static std::mutex mu;
+    static std::map<int, bool> done;          // device -> the cluster kernel's attributes were accepted
+    std::lock_guard<std::mutex> lock(mu);
+    auto it = done.find(p->device);
+    if (it == done.end()) {
+        const size_t o = p->smem_optin;
+        CU(cap_dynamic_smem(k_jac_project<float>, o)); CU(cap_dynamic_smem(k_jac_project<double>, o));
+        CU(cap_dynamic_smem(k_asm_pairs<float>, o)); CU(cap_dynamic_smem(k_asm_pairs<double>, o));
+        CU(cap_dynamic_smem(k_asm_mruns<float>, o)); CU(cap_dynamic_smem(k_asm_mruns<double>, o));
+        CU(cap_dynamic_smem(k_schur_prepare, o)); CU(cap_dynamic_smem(k_schur_syrk, o));
+        CU(cap_dynamic_smem(k_report_obs, o)); CU(cap_dynamic_smem(k_sel_hist, o)); CU(cap_dynamic_smem(k_track_cta, o));
+        // cluster Cholesky: up to 16 CTAs per cluster (non-portable size)
+        const bool ok = cap_dynamic_smem(k_reduced_solve_cluster2, o) == cudaSuccess &&
+                        cudaFuncSetAttribute(k_reduced_solve_cluster2, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
+        if (!ok) cudaGetLastError();
+        it = done.emplace(p->device, ok).first;
+    }
+    *cluster_ok = it->second;
+    return AAR_OK;
+}
+
 // Launches the Jacobian kernels: k_jac_project (numerators + residual at z, one row per observation) and the tensor-core assembly
 // k_asm_pairs + k_asm_mruns (aar_assemble.cuh).
 template <typename JT>
@@ -245,13 +279,11 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
     // camera x marker blocks: ASM_CM_REPLICAS copies of a [nrc][nrm][36] table (up to 256 MB; larger rigs add straight into the reduced matrix)
     const size_t cm_n = (size_t)p->nrc * p->nrm * 36;
     const bool use_rep = p->opt_c && p->opt_m && cm_n > 0 && cm_n * ASM_CM_REPLICAS * sizeof(double) <= (256u << 20);
+    p->last_smem_acc = pl.smem_acc; p->last_cm_rep = use_rep;
     if (use_rep) {
         if (p->d_cm_rep.n < cm_n * ASM_CM_REPLICAS) CU(p->d_cm_rep.alloc(cm_n * ASM_CM_REPLICAS));
         CU(cudaMemsetAsync(p->d_cm_rep.p, 0, cm_n * ASM_CM_REPLICAS * sizeof(double), p->stream));
     }
-    CU(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem1, 1024)));
-    CU(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-    CU(cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
     if (p->analytic) {
         if constexpr (std::is_same<JT, double>::value) LAUNCH(p, k_jac_analytic, cdiv(N, 128), 128, 0, p->dp, huber_eval, Jn, p->d_Rv.p);
         else { set_err("the analytic variant stages its rows in double"); return AAR_ERR_INVALID; }
@@ -379,6 +411,7 @@ int build_and_solve_reduced(aar_problem *p) {
             CU(cudaLaunchCooperativeKernel((const void *)k_reduced_solve, dim3(gridc), dim3(CH_THREADS), args, 0, p->stream));
             p->launches++;
         }
+        p->last_cluster_solve = done;
         LAUNCH(p, k_apply_reduced, cdiv(n_r, 128), 128, 0, n_r, p->d_z.p, p->d_dr.p, p->d_zt.p);
     }
     return AAR_OK;
@@ -778,16 +811,14 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
         LAUNCH(p, k_undistort, cdiv(2 * Nl, 256), 256, 0, 2 * Nl, 1, reinterpret_cast<const float2 *>(p->d_raw_b.p), p->d_obs_cm.p, p->d_K9.p, p->d_dist5.p, reinterpret_cast<float2 *>(p->d_und_b.p));
     }
     { const char *e = getenv("AAR_FORCE_EXACT_STAGING"); p->force_exact_staging = e && *e == '1'; }   // test hook: FP64 staging of the Jacobian block
-    CU(cudaFuncSetAttribute(k_schur_syrk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SY_SMEM));
-    {   // cluster Cholesky: up to 16 CTAs per cluster (non-portable size), block row + staging in shared memory
+    {   // cluster Cholesky: up to 16 CTAs per cluster, block row + staging in shared memory
+        bool cluster_ok = false;
+        if (int rc = set_smem_caps(p, &cluster_ok)) return rc;
         const int nblk = (p->n_r + CH_NB - 1) / CH_NB;
         const size_t smem = cluster2_smem_bytes(nblk);
         const char *e = getenv("AAR_NO_CLUSTER_SOLVE");                       // development aid: force the cooperative-grid kernel
-        if (nblk > 16 || smem > p->smem_optin - 1024 || (p->n_r & 1) || (e && *e == '1')) p->use_cluster_solve = false;
-        else if (cudaFuncSetAttribute(k_reduced_solve_cluster2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-                 cudaFuncSetAttribute(k_reduced_solve_cluster2, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) { cudaGetLastError(); p->use_cluster_solve = false; }
+        if (!cluster_ok || nblk > 16 || smem > p->smem_optin - 1024 || (p->n_r & 1) || (e && *e == '1')) p->use_cluster_solve = false;
     }
-    CU(cudaFuncSetAttribute(k_schur_prepare, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(8 * SP_TILE_BYTES + (size_t)p->n_r * sizeof(double))));
     CU(cudaStreamSynchronize(p->stream));
     cmark("undistortion, attributes, sync");
     aar_lm_default_params(&p->params);
@@ -1007,7 +1038,6 @@ int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out)
     if (N > 0) {
         const size_t msm = (size_t)p->M * 20;
         const int marker_smem = msm + 4096 <= p->smem_optin;
-        if (marker_smem) CU(cudaFuncSetAttribute(k_report_obs, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
         int per_sm = 1; CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_report_obs, REP_THREADS, marker_smem ? msm : 0));
         const int grid = (int)std::min<long long>((long long)std::max(per_sm, 1) * p->num_sms, cdiv(N, REP_THREADS));
         LAUNCH(p, k_report_obs, grid, REP_THREADS, marker_smem ? msm : 0, N, p->d_r.p, p->dp.obs_f, p->dp.obs_cm, p->C, p->M, p->f_begin, marker_smem,
@@ -1024,7 +1054,6 @@ int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out)
         if (p->d_sel.n < 2 * (size_t)nq) CU(p->d_sel.alloc(2 * (size_t)nq));
         if (p->d_sel_hist.n < (size_t)nq * SEL_BINS) CU(p->d_sel_hist.alloc((size_t)nq * SEL_BINS));
         CU(cudaMemcpyAsync(p->d_sel.p, sel.data(), sel.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, p->stream));
-        CU(cudaFuncSetAttribute(k_sel_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SEL_BINS * sizeof(unsigned))));
         const auto *keys = reinterpret_cast<const unsigned long long *>(p->d_rep_err.p);
         for (int pass = 0; pass < SEL_PASSES; pass++) {
             const int smem_hist = pass == 0;                       // one histogram, most contended digit (sign, exponent)
@@ -1405,7 +1434,6 @@ int aar_track_run(aar_problem *p, const aar_lm_params *params) {
     const char *e = getenv("AAR_TRACK");
     prof_mark(p, 13);
     if (smem <= p->smem_optin && !(e && !strcmp(e, "warp"))) {      // one CTA per frame, T1 = inv(Tc) * To once per camera and pose variant
-        if (smem > 48 * 1024) CU(cudaFuncSetAttribute(k_track_cta, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         LAUNCH(p, k_track_cta, F, TRKB_THREADS, smem, p->dp, tp, p->d_frame_obs_ptr.p, p->d_trk_cam_inv.p, p->d_trk_Y.p, p->d_trk_z.p, p->d_trk_cost.p, p->d_trk_iters.p);
     } else
         LAUNCH(p, k_track, cdiv(F, TRK_WARPS), TRK_WARPS * 32, 0, p->dp, tp, p->d_frame_obs_ptr.p, p->d_trk_cam_inv.p, p->d_trk_Y.p, p->d_trk_z.p, p->d_trk_cost.p, p->d_trk_iters.p);
@@ -1462,7 +1490,8 @@ int aar_comm_init(aar_problem *p, const void *id128) {
 int64_t aar_kernel_launches(const aar_problem *p) { return p ? p->launches : 0; }
 int aar_problem_stats(const aar_problem *p, int64_t *out) {
     if (!p || !out) return AAR_ERR_INVALID;
-    out[0] = p->nslots; out[1] = p->npairs; out[2] = p->nmruns; out[3] = p->schur_fma; out[4] = (p->lm_graph_ok ? 2 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
+    out[0] = p->nslots; out[1] = p->npairs; out[2] = p->nmruns; out[3] = p->schur_fma;
+    out[4] = (p->lm_graph_ok ? 2 : 0) | (p->last_cluster_solve ? 4 : 0) | (p->last_smem_acc ? 8 : 0) | (p->last_cm_rep ? 16 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
     return AAR_OK;
 }
 int aar_set_profiling(aar_problem *p, int32_t on) { if (!p) return AAR_ERR_INVALID; p->profiling = on != 0; for (double &m : p->phase_ms) m = 0; p->track_ms = 0; p->track_runs = 0; return AAR_OK; }

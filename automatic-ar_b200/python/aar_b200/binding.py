@@ -323,6 +323,8 @@ class Problem:
         _chk(lib().aar_problem_stats(self.h, v), "aar_problem_stats")
         d = dict(zip(["slots", "pairs", "mruns", "schur_fma", "mode_bits", "max_slots_per_frame", "frame_begin", "frame_end"], [int(x) for x in v]))
         d["peer_reduction"] = bool(d["mode_bits"] & 1); d["graph_loop"] = bool(d["mode_bits"] & 2); d["graph_iterations"] = d["mode_bits"] >> 8
+        # paths of the last reduced solve and the last assembly
+        d["cluster_solve"] = bool(d["mode_bits"] & 4); d["smem_accumulators"] = bool(d["mode_bits"] & 8); d["cm_replicas"] = bool(d["mode_bits"] & 16)
         return d
 
     def set_profiling(self, on=True):

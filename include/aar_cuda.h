@@ -206,7 +206,10 @@ int aar_comm_init(aar_problem *p, const void *id128);
 #define AAR_NUM_PHASES 12
 int64_t aar_kernel_launches(const aar_problem *p);
 /* sizes of this rank's shard: [0] W slots  [1] (frame, camera) pairs  [2] (frame, marker) runs  [3] fused multiply-adds of the upper
- * triangle of the Schur update S -= E E^T per try  [4] bit 0: always 0, bit 1: graph-resident loop built, bits 8..: LM iterations run inside the graph  [5] most blocks seen by one frame  [6] [7] frame index range */
+ * triangle of the Schur update S -= E E^T per try  [4] bit 0: always 0, bit 1: graph-resident loop built, bit 2: the last reduced solve
+ * ran the cluster Cholesky (else the cooperative-grid one), bit 3: the last assembly kept its camera / marker accumulators in shared
+ * memory (else it added them into global memory), bit 4: the last assembly used the camera x marker replicas, bits 8..: LM iterations
+ * run inside the graph  [5] most blocks seen by one frame  [6] [7] frame index range */
 int aar_problem_stats(const aar_problem *p, int64_t *out /* [8] */);
 int aar_set_profiling(aar_problem *p, int32_t on);
 int aar_get_phase_ms(const aar_problem *p, double *ms /* [AAR_NUM_PHASES] */);
