@@ -38,7 +38,7 @@ __global__ void k_expand_analytic(DevProblem p, const double *__restrict__ z) {
     for (int i = 0; i < 27; i++) dst[i] = dR[i];
 }
 
-// receives the derivative pairs of aar_an_observation into an [18][8] block (a staged row, or the parity hook's dense block)
+// receives the derivative pairs of aar_an_observation into the [18][8] block at the head of a staged row
 struct AnBlockSink {
     double *dst;
     AAR_HD void put(int col, int corner, double jx, double jy) { *reinterpret_cast<double2 *>(dst + col * 8 + 2 * corner) = make_double2(jx, jy); }
@@ -84,20 +84,6 @@ __global__ void __launch_bounds__(128) k_jac_analytic(DevProblem p, float huber_
         for (int i = 0; i < 4; i++) w[i] = huber_weight(e[2 * i] * e[2 * i] + e[2 * i + 1] * e[2 * i + 1], huber_delta);
         double2 *dst = reinterpret_cast<double2 *>(Rv + (size_t)o * 4); dst[0] = make_double2(w[0], w[1]); dst[1] = make_double2(w[2], w[3]);
     }
-}
-
-// parity hook: the dense 8 x 18 block of every observation, [col][row] like k_jacobian_dump
-__global__ void __launch_bounds__(128) k_jacobian_dump_an(DevProblem p, double *__restrict__ Jdump) {
-    const long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (o >= p.N) return;
-    const int cm = p.obs_cm[o];
-    double *dst = Jdump + (size_t)o * 144;
-    for (int i = 0; i < 144; i++) dst[i] = 0.0;
-    if (obs_nojac(cm)) return;
-    AnObsDev q; an_load_obs(p, o, cm, q);
-    double e[8];
-    AnBlockSink sink{dst};
-    an_eval(p, q, e, sink);
 }
 
 // eval_curr_solution (mcm.cpp:996-1028) of the full-FP64 variant: e = m - p in double, Huber weight, sum of squares.  Same interface as

@@ -110,7 +110,7 @@ struct aar_problem {
     DevBuf<double> d_fc, d_E, d_xinv;
     DevBuf<int> d_pair_slot_i; DevBuf<double> d_intr_tr, d_Ji;
     DevBuf<double> d_intr, d_K9, d_dist5, d_cam_tab, d_mk_tab, d_fr_tab, d_cam_tr, d_mk_tr, d_fr_tr, d_cam_fixed, d_mk_fixed, d_fr_fixed;
-    DevBuf<double> d_z, d_zt, d_z0, d_Hf, d_W, d_Hrr, d_gr, d_red, d_dr, d_red3, d_tmp, d_r, d_J;
+    DevBuf<double> d_z, d_zt, d_z0, d_Hf, d_W, d_Hrr, d_gr, d_red, d_dr, d_red3, d_tmp, d_r;
     DevBuf<LmState> d_st;
     DevBuf<int> d_flag;
     LmState *h_st = nullptr; double *h_red3 = nullptr; int *h_flags = nullptr; // pinned; h_st: LM state as last read back or pushed
@@ -313,26 +313,18 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
     return AAR_OK;
 }
 
-// J^T J blocks and J^T r at d_z (sparselevmarq.h:353-367) into Hf / W / Hrr / gr; or the dense per-observation
-// Jacobian blocks into Jdump (parity hook)
-int jacobian_accumulate(aar_problem *p, float huber_eval, double *Jdump, bool defer_check = false) {
+// J^T J blocks and J^T r at d_z (sparselevmarq.h:353-367) into Hf / W / Hrr / gr.  *rows64: the staged rows of this evaluation
+// are d_Jn64 (FP64 staging), not d_Jn32.
+int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = false, bool *rows64 = nullptr) {
     const long long jobs = (long long)p->C * NVAR_CAM + (long long)p->M * NVAR_RT + (long long)p->dp.F * NVAR_RT;
     LAUNCH(p, k_expand_jac, cdiv(jobs, 128), 128, 0, p->dp, p->d_z.p, p->d_flag.p);
     if (p->opt_i) LAUNCH(p, k_expand_intr, cdiv(p->C, 64), 64, 0, p->dp, p->d_z.p, p->d_intr.p);
     if (p->analytic) LAUNCH(p, k_expand_analytic, cdiv((long long)p->C + p->M + p->dp.F, 128), 128, 0, p->dp, p->d_z.p);
     else if (p->npairs > 0) LAUNCH(p, k_pair_tab, std::max(1, std::min(p->npairs, 10 * p->num_sms)), PAIR_TAB, 0, p->dp);      // 10 CTAs of 192 threads per SM: one full wave
-    if (Jdump && p->analytic) {
-        if (p->dp.N > 0) LAUNCH(p, k_jacobian_dump_an, cdiv(p->dp.N, 128), 128, 0, p->dp, Jdump);
-        return AAR_OK;
-    }
-    if (Jdump) {
-        if (p->dp.N > 0) LAUNCH(p, k_jacobian_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, huber_eval, Jdump);
-        if (p->opt_i && p->dp.N > 0) { if (p->d_Ji.n < 32 * (size_t)p->dp.N) CU(p->d_Ji.alloc(32 * (size_t)p->dp.N)); LAUNCH(p, k_intr_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, p->d_Ji.p); }
-        return AAR_OK;
-    }
     const size_t N = (size_t)p->dp.N;
     for (int attempt = 0; attempt < 2; attempt++) {
         const bool exact = p->force_exact_staging || attempt == 1 || p->exact_next || p->analytic;      // the analytic variant has no float32 staging
+        if (rows64) *rows64 = exact;
         if (p->d_Hrr.n) CU(cudaMemsetAsync(p->d_Hrr.p, 0, p->d_Hrr.n * sizeof(double), p->stream));
         if (p->d_gr.n) CU(cudaMemsetAsync(p->d_gr.p, 0, p->d_gr.n * sizeof(double), p->stream));
         if (p->d_Hf.n) CU(cudaMemsetAsync(p->d_Hf.p, 0, p->d_Hf.n * sizeof(double), p->stream));
@@ -438,7 +430,7 @@ int lm_jacobian_phase(aar_problem *p, bool graph) {
     const int n_r = p->n_r;
     int rc;
     prof_mark(p, 0);
-    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, nullptr, true))) return rc;
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, true))) return rc;
     prof_mark(p, 1);
     const double *diag = p->d_Hrr.p; int ld = n_r; double frames_maxdiag = 0.0;
     if (p->h_st->mu < 0) {
@@ -1102,14 +1094,31 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
     if (p->lm_active) { set_err("aar_eval_jacobian between aar_lm_begin and aar_lm_end would replace the resident iterate"); return AAR_ERR_INVALID; }
     CU(cudaSetDevice(p->device));
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
-    const size_t nj = 144 * (size_t)std::max<long long>(p->N, 1);
-    if (p->d_J.n < nj) CU(p->d_J.alloc(nj));
-    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, p->d_J.p))) return rc;
-    std::vector<double> J(nj), Ji(p->opt_i ? 32 * (size_t)std::max<long long>(p->N, 1) : 0);
-    CU(cudaMemcpyAsync(J.data(), p->d_J.p, nj * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-    if (p->opt_i && p->N > 0) CU(cudaMemcpyAsync(Ji.data(), p->d_Ji.p, 32 * (size_t)p->N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    // the staged rows the solver assembles from: float32 when every numerator fits one, else re-staged in FP64 before this returns
+    bool rows64 = false;
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, false, &rows64))) return rc;
+    const size_t N = (size_t)p->N;
+    std::vector<double> J64(rows64 ? JROW * N : 0), Ji(p->opt_i ? 32 * N : 0);
+    std::vector<float> J32(rows64 ? 0 : JROW * N);
+    if (N > 0) {
+        if (rows64) CU(cudaMemcpyAsync(J64.data(), p->d_Jn64.p, JROW * N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+        else CU(cudaMemcpyAsync(J32.data(), p->d_Jn32.p, JROW * N * sizeof(float), cudaMemcpyDeviceToHost, p->stream));
+        if (p->opt_i) {     // intrinsics columns: no staged rows, recomputed from the pose and pair tables just expanded
+            if (p->d_Ji.n < 32 * N) CU(p->d_Ji.alloc(32 * N));
+            LAUNCH(p, k_intr_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, p->d_Ji.p);
+            CU(cudaMemcpyAsync(Ji.data(), p->d_Ji.p, 32 * N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+        }
+    }
     CU(cudaStreamSynchronize(p->stream));
     CU(cudaGetLastError());
+    // entry (o, col, q) of the dense 8x18 block, col = 6 * block + dof: a derivative in the analytic variant, else the
+    // central-difference numerator divided by 2 delta as obtain_marker_derivs does (mcm.cpp:976-994; a product with the
+    // reciprocal would not round the same)
+    auto Jv = [&](long long o, int col, int q) {
+        const size_t i = (size_t)o * JROW + (size_t)col * 8 + q;
+        const double v = rows64 ? J64[i] : (double)J32[i];
+        return p->analytic ? v : v / (2 * p->J_delta);
+    };
     // compressed columns in the order setFromTriplets leaves them: columns ascending, rows ascending
     std::vector<std::vector<long long>> by_cam((size_t)p->C), by_marker((size_t)p->M), by_frame((size_t)p->F);
     for (long long o = 0; o < p->N; o++) {
@@ -1121,7 +1130,7 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
     auto emit = [&](const std::vector<long long> &obs, int local_col0) {
         for (int d = 0; d < 6; d++) {
             for (long long o : obs)
-                for (int q = 0; q < 8; q++) { rowidx[nnz] = (int32_t)(8 * o + q); vals[nnz] = J[(size_t)o * 144 + (size_t)(local_col0 + d) * 8 + q]; nnz++; }
+                for (int q = 0; q < 8; q++) { rowidx[nnz] = (int32_t)(8 * o + q); vals[nnz] = Jv(o, local_col0 + d, q); nnz++; }
             colptr[++col] = nnz;
         }
     };
@@ -1145,7 +1154,7 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
     residual(p, p->d_z.p, p->h_st->huber_eval, nullptr);
-    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, nullptr))) return rc;
+    if ((rc = jacobian_accumulate(p, p->h_st->huber_eval))) return rc;
     p->h_st->mu = mu; push_state(p);
     const int n_r = p->n_r;
     double *dS = p->d_red.p;

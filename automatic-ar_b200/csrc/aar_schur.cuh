@@ -115,15 +115,12 @@ __global__ void __launch_bounds__(256, AAR_SP_MINBLOCKS) k_schur_prepare(DevProb
 // reduced block blk in frame f, or -1.  gridDim.x = ntiles * nchunks (tile fastest).
 // Software pipeline over batches of SY_FB frames: slot indices are fetched two batches ahead (registers), the E
 // blocks one batch ahead (cp.async into the other shared-memory buffer, zero-filled for absent blocks), so the
-// FP64 FMAs of batch b overlap the global-memory latency of batches b+1 and b+2.
+// FP64 tensor-core products of batch b overlap the global-memory latency of batches b+1 and b+2.
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc, bool valid) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     const int sz = valid ? 16 : 0;
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(gsrc), "r"(sz) : "memory");
 }
-#ifndef AAR_SY_DMMA
-#define AAR_SY_DMMA 1          // 1: mma.sync.m8n8k4.f64 (FP64 tensor cores), 0: per-thread 6x6x6 FMA blocks (round-1 kernel)
-#endif
 #ifndef AAR_SY_MINBLOCKS
 #define AAR_SY_MINBLOCKS 2
 #endif
@@ -139,10 +136,8 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
     int ti = 0;
     while (tile >= tiles_side - ti) { tile -= tiles_side - ti; ti++; }
     const int tj = ti + tile;
-    const int tid = threadIdx.x, bi = tid / SY_TB, bj = tid % SY_TB;
+    const int tid = threadIdx.x;
     const int f0 = (int)((long long)p.F * chunk / nchunks), f1 = (int)((long long)p.F * (chunk + 1) / nchunks);
-    const int gi = ti * SY_TB + bi, gj = tj * SY_TB + bj;                    // global block indices of this thread's pair
-    const bool mine = gi < nb && gj < nb && (ti != tj || bi <= bj);          // upper block triangle only
     const int nbatch = (f1 - f0 + SY_FB - 1) / SY_FB;
     // slot-index prefetch: thread e < 2*SY_FB*SY_TB owns entry (side, ff, blk) of every batch
     const bool idx_thread = tid < 2 * SY_FB * SY_TB;
@@ -161,8 +156,7 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
-#if AAR_SY_DMMA
-    // FP64 tensor-core path: the CTA tile is a 96 x 96 x (6 * SY_FB) GEMM per batch, A[m][k] = E_I[i][r] with m = (block, i) of the
+    // FP64 tensor cores: the CTA tile is a 96 x 96 x (6 * SY_FB) GEMM per batch, A[m][k] = E_I[i][r] with m = (block, i) of the
     // row side and k = (frame in batch, r), B[k][n] the same of the column side; absent blocks were zero-filled by cp.async.
     // 2 x 4 warps, 48 x 24 outputs each = 6 x 3 mma.m8n8k4 tiles (36 accumulators per lane), 6 k-steps per batch:
     // 9 shared-memory loads per 18 DMMA instead of 36 vector loads per 216 FMAs.
@@ -179,11 +173,6 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
     for (int t = 0; t < 6; t++)
 #pragma unroll
         for (int u = 0; u < 3; u++) { cacc[t][u][0] = 0.0; cacc[t][u][1] = 0.0; }
-#else
-    double acc[36];
-#pragma unroll
-    for (int i = 0; i < 36; i++) acc[i] = 0.0;
-#endif
     // prologue: slots of batch 0 -> shared, copy of batch 0 in flight, slots of batch 1 in registers
     int slot_next = fetch_slot(0);
     if (idx_thread) (&sPresent[0][0][0][0])[tid] = slot_next;
@@ -198,7 +187,6 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
         if (b + 1 < nbatch) { issue_copy(nxt); asm volatile("cp.async.wait_group 1;" ::: "memory"); }
         else asm volatile("cp.async.wait_group 0;" ::: "memory");
         __syncthreads();
-#if AAR_SY_DMMA
         {
             const double *A0 = &sE[cur][0][0][0], *B0 = &sE[cur][1][0][0];
 #pragma unroll
@@ -216,34 +204,8 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
                                      : "+d"(cacc[t][u][0]), "+d"(cacc[t][u][1]) : "d"(a[t]), "d"(bb[u]));
             }
         }
-#else
-        if (mine) {
-            const int nf = min(SY_FB, f1 - (f0 + b * SY_FB));
-            for (int ff = 0; ff < nf; ff++) {
-                if (sPresent[cur][0][ff][bi] < 0 || sPresent[cur][1][ff][bj] < 0) continue;
-                const double2 *ei = reinterpret_cast<const double2 *>(&sE[cur][0][ff][bi * SY_LD]), *ej = reinterpret_cast<const double2 *>(&sE[cur][1][ff][bj * SY_LD]);
-                double a[36];
-#pragma unroll
-                for (int i = 0; i < 18; i++) { const double2 v = ei[i]; a[2 * i] = v.x; a[2 * i + 1] = v.y; }
-#pragma unroll
-                for (int c = 0; c < 6; c++) {
-                    double bcol[6];
-#pragma unroll
-                    for (int k = 0; k < 3; k++) { const double2 v = ej[c * 3 + k]; bcol[2 * k] = v.x; bcol[2 * k + 1] = v.y; }
-#pragma unroll
-                    for (int r = 0; r < 6; r++) {
-                        double s = acc[r * 6 + c];
-#pragma unroll
-                        for (int k = 0; k < 6; k++) s = fma(a[r * 6 + k], bcol[k], s);
-                        acc[r * 6 + c] = s;
-                    }
-                }
-            }
-        }
-#endif
         __syncthreads();
     }
-#if AAR_SY_DMMA
 #pragma unroll
     for (int t = 0; t < 6; t++)
 #pragma unroll
@@ -256,16 +218,6 @@ __global__ void __launch_bounds__(SY_THREADS, AAR_SY_MINBLOCKS) k_schur_syrk(Dev
                 if (gim < nb && gjn < nb && (ti != tj || bim <= bjn) && v != 0.0)
                     atomicAdd(S + (size_t)(6 * gim + m % 6) * p.n_r + 6 * gjn + n % 6, -v);
             }
-    (void)mine; (void)bi; (void)bj;
-#else
-    if (mine) {
-        double *dst = S + (size_t)(6 * gi) * p.n_r + 6 * gj;
-#pragma unroll
-        for (int r = 0; r < 6; r++)
-#pragma unroll
-            for (int c = 0; c < 6; c++) if (acc[r * 6 + c] != 0.0) atomicAdd(dst + (size_t)r * p.n_r + c, -acc[r * 6 + c]);
-    }
-#endif
 }
 
 } // namespace aar

@@ -64,10 +64,12 @@ def test_index_maps_bit_exact(binding, oracle_mod):
                   erased_or_duplicate_detections=4, bit_exact=True)
 
 
-@pytest.mark.parametrize("distorted", [False, True])
-def test_residual_and_jacobian_bit_exact(binding, oracle_mod, distorted):
+@pytest.mark.parametrize("distorted,staging", [(False, "float32"), (True, "float32"), (True, "fp64")], ids=["False", "True", "fp64_staging"])
+def test_residual_and_jacobian_bit_exact(binding, oracle_mod, monkeypatch, distorted, staging):
     rig = small_rig(seed=5, distorted=distorted, F=60)
     o = oracle_mod.Oracle(rig, sincos_mode=1)
+    if staging == "fp64":       # read when the handle is created: every evaluation stages its Jacobian rows in FP64
+        monkeypatch.setenv("AAR_FORCE_EXACT_STAGING", "1")
     p = binding.Problem(rig)
     und, raw = p.observations()
     obs = o.observations()
@@ -91,7 +93,7 @@ def test_residual_and_jacobian_bit_exact(binding, oracle_mod, distorted):
     flips = (o.error(z0) != p.residual(z0)[0]).sum()
     o.set_sincos_mode(1)
     assert flips <= 2
-    parity_record("undistortion_residual_jacobian_vs_oracle", distorted=bool(distorted), residual_rows=int(len(r_o)), jacobian_nnz=int(len(v_o)), bit_exact=True,
+    parity_record("undistortion_residual_jacobian_vs_oracle", distorted=bool(distorted), staging=staging, residual_rows=int(len(r_o)), jacobian_nnz=int(len(v_o)), bit_exact=True,
                   float32_flips_against_libm_sincos_oracle=int(flips))
 
 
@@ -109,6 +111,20 @@ def test_config_flags_and_huber(binding, oracle_mod):
     p = binding.Problem(rig, with_huber=True)
     z = o.mats2evec()
     assert np.array_equal(p.residual(z, huber_delta=1.5)[0], o.error(z))
+
+
+def test_jacobian_bit_exact_with_marker_tables_in_global_memory(binding, oracle_mod):
+    """130 markers: their pose tables (130 x 49 doubles) outgrow the 48 KB of shared memory k_jac_project stages them in
+    (launch_jacobian), so the kernel reads them from global memory.  Residuals and Jacobian bit-exact against the oracle."""
+    rig = small_rig(seed=29, M=130, F=100, obs_per_frame=12.0)
+    assert rig.M * 49 * 8 > 48 * 1024
+    o = oracle_mod.Oracle(rig); p = binding.Problem(rig)
+    z0 = o.mats2evec()
+    for z in (z0, z0 + np.random.default_rng(1).normal(0, 1e-3, z0.shape)):
+        assert np.array_equal(p.residual(z)[0], o.error(z))
+        cp_o, ri_o, v_o = o.jacobian(z); cp_g, ri_g, v_g = p.jacobian(z)
+        assert np.array_equal(cp_o, cp_g) and np.array_equal(ri_o, ri_g) and np.array_equal(v_o, v_g)
+    parity_record("jacobian_vs_oracle_marker_tables_in_global_memory", markers=int(rig.M), observations=int(p.num_obs), jacobian_nnz=int(len(v_g)), bit_exact=True)
 
 
 def test_reduced_system_matches_oracle(binding, oracle_mod):
