@@ -27,6 +27,7 @@
 #include "aar_host_math.h"
 #include "aar_kernels.cuh"
 #include "aar_report.cuh"
+#include "aar_fixed.cuh"
 
 using namespace aar;
 
@@ -135,6 +136,8 @@ struct aar_problem {
     DevBuf<LmTraceDev> d_trace;
     // aar_error_report (aar_report.cuh): observation errors, entity statistics [C + M + F], select state [2 nq], digit histograms [nq][SEL_BINS]
     DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
+    // aar_set_fixed (aar_fixed.cuh): one byte per reduced block and per local frame; without a mask nothing is launched
+    bool has_fixed = false; DevBuf<uint8_t> d_blk_fixed, d_frame_fixed;
     cudaEvent_t ev[16] = {}; double phase_ms[AAR_NUM_PHASES] = {};
 };
 
@@ -313,6 +316,16 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
     return AAR_OK;
 }
 
+// the columns of fixed entities become explicit zeros of J: their rows / columns of J^T J and entries of J^T r (aar_fixed.cuh)
+void hold_fixed(aar_problem *p) {
+    if (!p->has_fixed) return;
+    // a warp per 32 W slots, a thread per entry of Hrr / gr / Hf; at most 8 CTAs of 256 threads per SM, grid-stride beyond
+    const long long work = std::max<long long>(p->nslots, (long long)p->n_r * p->n_r + p->n_r + (long long)p->dp.F * HF_STRIDE);
+    const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(cdiv(work, 256), 8LL * p->num_sms));
+    LAUNCH(p, k_hold_fixed, grid, 256, 0, p->n_r, p->d_blk_fixed.p, p->dp.F, p->d_frame_fixed.p, p->nslots, p->d_slot_block.p, p->d_slot_frame.p,
+           p->d_Hrr.p, p->d_gr.p, p->d_Hf.p, p->d_W.p);
+}
+
 // J^T J blocks and J^T r at d_z (sparselevmarq.h:353-367) into Hf / W / Hrr / gr.  *rows64: the staged rows of this evaluation
 // are d_Jn64 (FP64 staging), not d_Jn32.
 int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = false, bool *rows64 = nullptr) {
@@ -345,6 +358,7 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = fal
         p->exact_reruns++;
         CU(cudaMemsetAsync(p->d_flag.p + 1, 0, sizeof(int), p->stream));
     }
+    hold_fixed(p);
     return AAR_OK;
 }
 
@@ -1503,6 +1517,51 @@ int aar_problem_stats(const aar_problem *p, int64_t *out) {
     out[4] = (p->lm_graph_ok ? 2 : 0) | (p->last_cluster_solve ? 4 : 0) | (p->last_smem_acc ? 8 : 0) | (p->last_cm_rep ? 16 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
     return AAR_OK;
 }
+int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed) {
+    if (!p) return AAR_ERR_INVALID;
+    if (p->lm_active) { set_err("aar_set_fixed between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
+    // only flags on optimised, non-root entities count; the masks of this rank hold its own frames
+    const int nb = p->nrc + p->nrm + p->nri, Fl = p->dp.F;
+    std::vector<uint8_t> blk((size_t)std::max(nb, 1), 0), fr((size_t)std::max(Fl, 1), 0);
+    bool any = false; long long free_blocks = p->nri;              // the intrinsics pseudo-blocks are never held fixed
+    if (p->opt_c)
+        for (int i = 0; i < p->C; i++) {
+            if (i == p->root_cam) continue;
+            const bool f = cam_fixed && cam_fixed[i];
+            blk[(size_t)(i - (i > p->root_cam ? 1 : 0))] = f; any |= f; free_blocks += !f;
+        }
+    if (p->opt_m)
+        for (int j = 0; j < p->M; j++) {
+            if (j == p->root_marker) continue;
+            const bool f = marker_fixed && marker_fixed[j];
+            blk[(size_t)(p->nrc + j - (j > p->root_marker ? 1 : 0))] = f; any |= f; free_blocks += !f;
+        }
+    if (p->opt_f)
+        for (int k = 0; k < p->F; k++) {
+            const bool f = frame_fixed && frame_fixed[k];
+            if (k >= p->f_begin && k < p->f_end) fr[(size_t)(k - p->f_begin)] = f;
+            any |= f; free_blocks += !f;
+        }
+    // with every column fixed the step is 0 and the gain 0 / 0
+    if (any && free_blocks == 0) { set_err("aar_set_fixed: the mask leaves no free column to solve for"); return AAR_ERR_INVALID; }
+    CU(cudaSetDevice(p->device));
+    if (any) {
+        if (!p->d_blk_fixed.p) { CU(p->d_blk_fixed.alloc(blk.size())); CU(p->d_frame_fixed.alloc(fr.size())); }   // allocated once: the captured graph keeps the pointers
+        CU(cudaMemcpyAsync(p->d_blk_fixed.p, blk.data(), blk.size(), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_frame_fixed.p, fr.data(), fr.size(), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaStreamSynchronize(p->stream));
+    }
+    if (any != p->has_fixed) {   // the body of the graph-resident loop gains or loses k_hold_fixed: capture it again on the next aar_lm_iterate
+        if (p->lm_exec) cudaGraphExecDestroy(p->lm_exec);
+        if (p->lm_graph) cudaGraphDestroy(p->lm_graph);
+        if (p->lm_side) cudaStreamDestroy(p->lm_side);
+        p->lm_exec = nullptr; p->lm_graph = nullptr; p->lm_side = nullptr;
+        p->lm_graph_tried = p->lm_graph_ok = false;
+    }
+    p->has_fixed = any;
+    return AAR_OK;
+}
+
 int aar_set_profiling(aar_problem *p, int32_t on) { if (!p) return AAR_ERR_INVALID; p->profiling = on != 0; for (double &m : p->phase_ms) m = 0; p->track_ms = 0; p->track_runs = 0; return AAR_OK; }
 int aar_get_phase_ms(const aar_problem *p, double *ms) {
     if (!p || !ms) return AAR_ERR_INVALID;

@@ -1,13 +1,15 @@
 // find_solution — the reference's app (/root/reference/apps/find_solution.cpp:28-181) on the CUDA path, OpenCV-free:
 //   find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>]
 //                 [-consensus-max <k>] [-init <initial.solution>] [-analytic] [-reject-outliers <px>]
+//                 [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]
 // Reads <folder>/<cam>/calib.yml and <folder>/aruco.detections, builds the starting point with the Initializer (device: IPPE per
 // detection + consensus; include/aar_init.h), writes initial<suffix>.solution(.yaml), solves on the GPU (include/aar_cuda.h) and
 // writes final<suffix>.solution(.yaml) — the file names of find_solution.cpp:76-100.  Two additions: -consensus-max (SURVEY 8(f) row 3,
 // the reference's exhaustive consensus is O(n^2) in the number of co-observations) and -init (start from an existing .solution
 // instead of the detections) and -analytic (analytic Jacobian, residuals in double: include/aar_analytic.h; not the reference's arithmetic),
 // -reject-outliers <px> (after the solve, remove the detections whose reprojection error is above px and solve again with the same settings;
-// the final file holds the second solve).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
+// the final file holds the second solve), -fix-cams / -fix-markers / -fix-frames (hold those poses as they are in both solves, e.g. the
+// calibrated cameras of a rig that gains one: MultiCamMapper::set_fixed_*).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -19,14 +21,14 @@
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>]" << std::endl;
+        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]" << std::endl;
         return -1;
     }
     const std::string folder = argv[1];
     const double marker_size = std::stod(argv[2]);
     bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
-    std::set<int> excluded_cams; std::string init_path;
-    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT } flag = NONE;
+    std::set<int> excluded_cams, fix_cams, fix_markers, fix_frames; std::string init_path;
+    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF } flag = NONE;
     for (int i = 3; i < argc; i++) {
         const std::string a = argv[i];
         if (a == "-subseqs") { use_subseqs = true; flag = NONE; }
@@ -37,7 +39,13 @@ int main(int argc, char **argv) {
         else if (a == "-consensus-max") flag = CMAX;
         else if (a == "-init") flag = INIT;
         else if (a == "-reject-outliers") flag = REJECT;
+        else if (a == "-fix-cams") flag = FIXC;
+        else if (a == "-fix-markers") flag = FIXM;
+        else if (a == "-fix-frames") flag = FIXF;
         else if (flag == EXCLUDE) excluded_cams.insert(std::stoi(a));
+        else if (flag == FIXC) fix_cams.insert(std::stoi(a));
+        else if (flag == FIXM) fix_markers.insert(std::stoi(a));
+        else if (flag == FIXF) fix_frames.insert(std::stoi(a));
         else if (flag == THRESH) { threshold = std::stod(a); flag = NONE; }
         else if (flag == CMAX) { consensus_max = std::stoi(a); flag = NONE; }
         else if (flag == INIT) { init_path = a; flag = NONE; }
@@ -80,6 +88,7 @@ int main(int argc, char **argv) {
         mcm.set_optmize_flag_cam_intrinsics(false);              // find_solution.cpp:140
         if (with_huber) mcm.set_with_huber(true);
         if (analytic) mcm.set_analytic_jacobian(true);
+        mcm.set_fixed_cams(fix_cams); mcm.set_fixed_markers(fix_markers); mcm.set_fixed_frames(fix_frames);
         auto start = std::chrono::system_clock::now();
         mcm.solve();
         d += std::chrono::system_clock::now() - start;

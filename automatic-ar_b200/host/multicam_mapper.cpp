@@ -221,8 +221,24 @@ void MultiCamMapper::eVec2Mats_full(const std::vector<double> &in) {
     }
 }
 
+static void check_ids(const std::set<int> &ids, const std::map<int, Mat44> &held, const char *what) {
+    for (int id : ids) if (!held.count(id)) throw std::invalid_argument(std::string("set_fixed_") + what + ": no " + what + " with id " + std::to_string(id));
+}
+void MultiCamMapper::set_fixed_cams(const std::set<int> &ids) { check_ids(ids, transforms_to_root_cam, "cams"); fixed_cams = ids; }
+void MultiCamMapper::set_fixed_markers(const std::set<int> &ids) { check_ids(ids, transforms_to_root_marker, "markers"); fixed_markers = ids; }
+void MultiCamMapper::set_fixed_frames(const std::set<int> &ids) { check_ids(ids, object_to_global, "frames"); fixed_frames = ids; }
+
 void MultiCamMapper::solve() {
     if (!handle) make_handle(corners_undistorted);
+    {   // aar_set_fixed: one byte per camera / marker / frame in id order; NULL for an empty set, all NULL clears
+        auto mask = [](const std::set<int> &ids, const std::map<int, Mat44> &held) {
+            std::vector<uint8_t> m; if (ids.empty()) return m;
+            for (auto &p : held) m.push_back(ids.count(p.first) ? 1 : 0);
+            return m;
+        };
+        const std::vector<uint8_t> c = mask(fixed_cams, transforms_to_root_cam), m = mask(fixed_markers, transforms_to_root_marker), f = mask(fixed_frames, object_to_global);
+        check(aar_set_fixed(handle, c.empty() ? nullptr : c.data(), m.empty() ? nullptr : m.data(), f.empty() ? nullptr : f.data()), "aar_set_fixed");
+    }
     io_vec.assign((size_t)aar_num_vars(handle), 0.0);
     check(aar_mats2evec(handle, io_vec.data()), "aar_mats2evec");
     aar_lm_params prm; aar_lm_default_params(&prm);
@@ -237,12 +253,13 @@ void MultiCamMapper::solve() {
     const size_t C = transforms_to_root_cam.size(), M = transforms_to_root_marker.size(), F = object_to_global.size();
     std::vector<double> Tc(16 * C), Tm(16 * M), To(16 * F);
     check(aar_evec2mats(handle, io_vec.data(), Tc.data(), Tm.data(), To.data()), "aar_evec2mats");
+    // fixed entities keep the caller's matrices: r -> R of the device expansion does not give back the R the vector was taken from
     size_t i = 0;
-    if (config.optimize_cam_poses) for (auto &p : transforms_to_root_cam) { std::memcpy(p.second.m, &Tc[16 * i], sizeof p.second.m); i++; }
+    if (config.optimize_cam_poses) for (auto &p : transforms_to_root_cam) { if (!fixed_cams.count(p.first)) std::memcpy(p.second.m, &Tc[16 * i], sizeof p.second.m); i++; }
     i = 0;
-    if (config.optimize_marker_poses) for (auto &p : transforms_to_root_marker) { std::memcpy(p.second.m, &Tm[16 * i], sizeof p.second.m); i++; }
+    if (config.optimize_marker_poses) for (auto &p : transforms_to_root_marker) { if (!fixed_markers.count(p.first)) std::memcpy(p.second.m, &Tm[16 * i], sizeof p.second.m); i++; }
     i = 0;
-    if (config.optimize_object_poses) for (auto &p : object_to_global) { std::memcpy(p.second.m, &To[16 * i], sizeof p.second.m); i++; }
+    if (config.optimize_object_poses) for (auto &p : object_to_global) { if (!fixed_frames.count(p.first)) std::memcpy(p.second.m, &To[16 * i], sizeof p.second.m); i++; }
     if (config.optimize_cam_intrinsics) {                        // intrinsics_vec2mats (:580-593): the last 9 entries per camera
         size_t vi = io_vec.size() - 9 * C;
         for (auto &p : transforms_to_root_cam) {
@@ -316,6 +333,7 @@ long long MultiCamMapper::remove_outliers(double max_px, Rejection *out) {
     for (auto f = object_to_global.begin(); f != object_to_global.end();) {
         if (left.count(f->first)) { ++f; continue; }
         rj.dropped_frames.push_back(f->first);
+        fixed_frames.erase(f->first);
         frame_cam_markers.erase(f->first); raw_frame_cam_markers.erase(f->first);
         f = object_to_global.erase(f);
     }

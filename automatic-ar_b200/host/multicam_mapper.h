@@ -5,6 +5,7 @@
 #pragma once
 #include <cmath>
 #include <map>
+#include <set>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -73,6 +74,12 @@ public:
     // all their observations stay (listed in `out`).  The handle is dropped: the next solve() creates it anew.  Returns the number removed.
     struct Rejection { long long removed = 0, observations = 0; std::vector<int> dropped_frames, unobserved_cams, unobserved_markers; };
     long long remove_outliers(double max_px, Rejection *out = nullptr);
+    // not in the reference: hold these cameras / markers / frames (ids) fixed in solve().  Their Jacobian columns are explicit zeros
+    // (aar_set_fixed, include/aar_cuda.h) and their Mat44 stay the caller's matrices byte for byte.  The sets persist across handles
+    // (remove_outliers drops the frames it removes); track() ignores them.  An id the mapper does not hold throws std::invalid_argument.
+    void set_fixed_cams(const std::set<int> &ids);
+    void set_fixed_markers(const std::set<int> &ids);
+    void set_fixed_frames(const std::set<int> &ids);
     void track();     // multicam_mapper.cpp:430-443: per-frame 6-dof solve against the fixed rig, every frame of the object at once
 
     bool write_solution_file(const std::string &path);         // byte-exact .solution (multicam_mapper.cpp:1053-1099)
@@ -111,6 +118,7 @@ private:
     void check(int rc, const char *what) const;
 
     Config config;
+    std::set<int> fixed_cams, fixed_markers, fixed_frames;
     bool with_huber = false, corners_undistorted = false, analytic_jacobian = false;
     size_t root_cam = 0, root_marker = 0;
     double marker_size = 0;

@@ -24,7 +24,7 @@ NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a",
 # declared by include/aar_cuda.h — tests check that the library exports every one of them
 EXPORTS = ["aar_lm_default_params", "aar_problem_create", "aar_problem_destroy", "aar_last_error", "aar_num_vars",
            "aar_num_observations", "aar_num_local_observations", "aar_jacobian_nnz", "aar_index_maps", "aar_get_observations",
-           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_lm_solve",
+           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_lm_solve",
            "aar_lm_begin", "aar_lm_iterate", "aar_lm_end", "aar_track_batch", "aar_track_upload", "aar_track_run", "aar_track_download", "aar_track_ms", "aar_shard_plan", "aar_row_map", "aar_comm_unique_id", "aar_comm_init",
            "aar_kernel_launches", "aar_set_profiling", "aar_get_phase_ms", "aar_problem_stats"]
 
@@ -240,6 +240,21 @@ class Problem:
         S = np.zeros((self.n_r, self.n_r)); b = np.zeros(self.n_r); cost = C.c_double(0)
         _chk(lib().aar_reduced_system(self.h, _vp(z), C.c_double(mu), _vp(S), _vp(b), C.byref(cost)), "aar_reduced_system")
         return S, b, cost.value
+
+    def set_fixed(self, cams=None, markers=None, frames=None):
+        """aar_set_fixed: hold cameras / markers / frames fixed in the later solves and reduced systems of this handle.  Boolean arrays by
+        index ([num_cams], [num_markers], [num_frames] of the description); None = none of that kind; all None clears."""
+        keep = []
+
+        def mask(m, n, what):
+            if m is None:
+                return None
+            a = np.asarray(m).reshape(-1)
+            if len(a) != n:
+                raise ValueError(f"set_fixed: {what} has {len(a)} entries, the description {n}")
+            keep.append(np.ascontiguousarray(a != 0, dtype=np.uint8))
+            return _vp(keep[-1])
+        _chk(lib().aar_set_fixed(self.h, mask(cams, self.nC, "cams"), mask(markers, self.nM, "markers"), mask(frames, self.nF, "frames")), "aar_set_fixed")
 
     @staticmethod
     def default_params(**kw):

@@ -160,6 +160,14 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
  * optimize_cam_intrinsics 12 more per camera, in the internal order [fx cx fy cy k1 k2 | p1 p2 k3 . . .] (csrc/aar_intrinsics.cuh). */
 int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, double *b, double *cost);
 
+/* Not in the reference.  Hold poses fixed in every later solve / aar_reduced_system of this handle: their Jacobian columns are
+ * treated as explicit zeros (step exactly 0, excluded from mu0).  Arrays indexed by rank of id: [num_cams], [num_markers],
+ * [num_frames] of the description (global frames; every rank passes the same arrays); nonzero = fixed; NULL = none of that kind;
+ * all NULL clears.  The root camera / marker and entities of a group that is not optimised may be flagged (no effect).
+ * Residuals and cost are unchanged; aar_eval_jacobian, aar_error_report and aar_track_* ignore the mask.  AAR_ERR_INVALID between
+ * aar_lm_begin and aar_lm_end, and for a mask that leaves no free column. */
+int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed);
+
 /* MultiCamMapper::solve() = SparseLevMarq::solve(z, f, J) (multicam_mapper.cpp:419-428,
  * sparselevmarq.h:439-472): z is in/out like io_vec; the loop is device resident. */
 int aar_lm_solve(aar_problem *p, double *z_inout, const aar_lm_params *params, aar_lm_report *report);
