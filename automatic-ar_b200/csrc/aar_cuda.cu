@@ -28,6 +28,7 @@
 #include "aar_kernels.cuh"
 #include "aar_report.cuh"
 #include "aar_fixed.cuh"
+#include "aar_prior.cuh"
 
 using namespace aar;
 
@@ -138,6 +139,9 @@ struct aar_problem {
     DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
     // aar_set_fixed (aar_fixed.cuh): one byte per reduced block and per local frame; without a mask nothing is launched
     bool has_fixed = false; DevBuf<uint8_t> d_blk_fixed, d_frame_fixed;
+    // aar_set_prior (aar_prior.cuh): [zbar 6 | w 6] and a has-prior byte per reduced pose block and per local frame; without priors
+    // nothing is launched
+    bool has_prior = false; DevBuf<double> d_blk_prior, d_frame_prior; DevBuf<uint8_t> d_blk_has_prior, d_frame_has_prior;
     cudaEvent_t ev[16] = {}; double phase_ms[AAR_NUM_PHASES] = {};
 };
 
@@ -221,6 +225,28 @@ int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_ou
         LAUNCH(p, k_residual_an, cdiv(p->dp.N, 256), 256, 0, dq, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
     else if (p->dp.N > 0)
         LAUNCH(p, k_residual, cdiv(p->dp.N, 256), 256, 0, dq, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
+    return AAR_OK;
+}
+
+// Soft priors (aar_prior.cuh): rank 0 alone adds the terms of the camera and marker blocks, every rank those of its frames, so the
+// all-reduces of the reduced system and of the cost count each once.  One thread per (entity, component) in CTAs of 256.
+int prior_blocks(const aar_problem *p) { return p->rank == 0 ? p->nrc + p->nrm : 0; }
+unsigned prior_grid(const aar_problem *p) { return cdiv(6LL * (prior_blocks(p) + p->dp.F), 256); }
+
+// J^T J += diag(w), J^T r += w (z - zbar) at d_z into Hrr / gr / Hf; nothing without priors
+void prior_add(aar_problem *p) {
+    if (!p->has_prior || !prior_grid(p)) return;
+    LAUNCH(p, k_prior_add, prior_grid(p), 256, 0, prior_blocks(p), p->d_blk_prior.p, p->d_blk_has_prior.p, p->dp.F, p->d_frame_prior.p,
+           p->d_frame_has_prior.p, p->dp.col_frame0, p->n_r, p->d_z.p, p->d_Hrr.p, p->d_gr.p, p->d_Hf.p);
+}
+
+// the cost the solver compares at dz into d_red3[0] (zeroed by the caller): the reprojection sum of residual(), then the priors'
+// sum w (z - zbar)^2.  The reprojection hooks (aar_eval_residual, aar_error_report) call residual() alone.
+int solver_cost(aar_problem *p, const double *dz, float huber_delta) {
+    if (int rc = residual(p, dz, huber_delta, nullptr)) return rc;
+    if (p->has_prior && prior_grid(p))
+        LAUNCH(p, k_prior_cost, prior_grid(p), 256, 0, prior_blocks(p), p->d_blk_prior.p, p->d_blk_has_prior.p, p->dp.F, p->d_frame_prior.p,
+               p->d_frame_has_prior.p, p->dp.col_frame0, dz, p->d_red3.p);
     return AAR_OK;
 }
 
@@ -358,7 +384,8 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = fal
         p->exact_reruns++;
         CU(cudaMemsetAsync(p->d_flag.p + 1, 0, sizeof(int), p->stream));
     }
-    hold_fixed(p);
+    prior_add(p);
+    hold_fixed(p);      // after the priors: a held entity's columns are zero in the whole augmented Jacobian
     return AAR_OK;
 }
 
@@ -478,7 +505,7 @@ int lm_try(aar_problem *p, bool graph) {
     if (p->opt_f && p->dp.F > 0)
         LAUNCH(p, k_backsub, std::max(1, std::min(4 * p->num_sms, (int)cdiv(p->dp.F, BS_WARPS))), BS_WARPS * 32, 0, p->dp, p->d_fc.p, p->d_Hf.p, p->d_W.p, p->d_dr.p, p->d_z.p, p->d_zt.p, p->d_red3.p);
     prof_mark(p, 4);
-    residual(p, p->d_zt.p, p->h_st->huber_delta, nullptr);
+    if ((rc = solver_cost(p, p->d_zt.p, p->h_st->huber_delta))) return rc;
     prof_mark(p, 5);
     if ((rc = allreduce(p, p->d_red3.p, 3, ncclSum))) return rc;
     LAUNCH(p, k_lm_decide, 1, 1, 0, p->d_st.p, p->d_red3.p, n_r, p->d_dr.p, Br, p->d_flag.p, (int)graph, p->lm_inner);
@@ -1167,7 +1194,7 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
     CU(cudaSetDevice(p->device));
     int rc = upload_z(p, z, p->d_z.p); if (rc) return rc;
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-    residual(p, p->d_z.p, p->h_st->huber_eval, nullptr);
+    if ((rc = solver_cost(p, p->d_z.p, p->h_st->huber_eval))) return rc;
     if ((rc = jacobian_accumulate(p, p->h_st->huber_eval))) return rc;
     p->h_st->mu = mu; push_state(p);
     const int n_r = p->n_r;
@@ -1201,7 +1228,7 @@ int aar_lm_begin(aar_problem *p, const double *z0, const aar_lm_params *params) 
     CU(cudaMemsetAsync(p->d_flag.p, 0, 4 * sizeof(int), p->stream));
     // SparseLevMarq::init (sparselevmarq.h:237-249)
     CU(cudaMemsetAsync(p->d_red3.p, 0, 8 * sizeof(double), p->stream));
-    residual(p, p->d_z.p, huber0, nullptr);
+    if ((rc = solver_cost(p, p->d_z.p, huber0))) return rc;
     if ((rc = allreduce(p, p->d_red3.p, 1, ncclSum))) return rc;
     CU(cudaMemcpyAsync(p->h_red3, p->d_red3.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     CU(cudaStreamSynchronize(p->stream));
@@ -1287,6 +1314,15 @@ done:
     return ok;
 }
 #undef GR
+
+// the kernels of an LM iteration changed (aar_set_fixed, aar_set_prior): the next aar_lm_iterate captures the graph again
+static void drop_lm_graph(aar_problem *p) {
+    if (p->lm_exec) cudaGraphExecDestroy(p->lm_exec);
+    if (p->lm_graph) cudaGraphDestroy(p->lm_graph);
+    if (p->lm_side) cudaStreamDestroy(p->lm_side);
+    p->lm_exec = nullptr; p->lm_graph = nullptr; p->lm_side = nullptr;
+    p->lm_graph_tried = p->lm_graph_ok = false;
+}
 
 // up to `iters` LM iterations inside the graph; one host synchronisation at the end
 static int lm_graph_run(aar_problem *p, int iters, aar_lm_report *rep) {
@@ -1551,14 +1587,73 @@ int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marke
         CU(cudaMemcpyAsync(p->d_frame_fixed.p, fr.data(), fr.size(), cudaMemcpyHostToDevice, p->stream));
         CU(cudaStreamSynchronize(p->stream));
     }
-    if (any != p->has_fixed) {   // the body of the graph-resident loop gains or loses k_hold_fixed: capture it again on the next aar_lm_iterate
-        if (p->lm_exec) cudaGraphExecDestroy(p->lm_exec);
-        if (p->lm_graph) cudaGraphDestroy(p->lm_graph);
-        if (p->lm_side) cudaStreamDestroy(p->lm_side);
-        p->lm_exec = nullptr; p->lm_graph = nullptr; p->lm_side = nullptr;
-        p->lm_graph_tried = p->lm_graph_ok = false;
-    }
+    if (any != p->has_fixed) drop_lm_graph(p);   // the body of the graph-resident loop gains or loses k_hold_fixed
     p->has_fixed = any;
+    return AAR_OK;
+}
+int aar_set_prior(aar_problem *p, const double *cam_T, const double *cam_w, const double *marker_T, const double *marker_w,
+                  const double *frame_T, const double *frame_w) {
+    if (!p) return AAR_ERR_INVALID;
+    if (p->lm_active) { set_err("aar_set_prior between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
+    const int nb = p->nrc + p->nrm, Fl = p->dp.F;
+    std::vector<double> blk((size_t)std::max(nb, 1) * PRIOR_STRIDE, 0.0), fr((size_t)std::max(Fl, 1) * PRIOR_STRIDE, 0.0);
+    std::vector<uint8_t> blk_has((size_t)std::max(nb, 1), 0), fr_has((size_t)std::max(Fl, 1), 0);
+    bool any = false;
+    // every weight is checked, and the target of every entity with a nonzero weight; then only optimised, non-root entities (and this
+    // rank's frames) are kept.  zbar is the R -> r of aar_mats2evec, so a target equal to the start matrix gives z - zbar = 0 exactly.
+    auto take = [&](const char *what, int n, const double *T, const double *w, auto slot) -> int {
+        if (!w) return AAR_OK;
+        for (int e = 0; e < n; e++) {
+            const double *we = w + 6 * (size_t)e;
+            bool nonzero = false;
+            for (int i = 0; i < 6; i++) {
+                if (!(std::isfinite(we[i]) && we[i] >= 0)) { set_err("aar_set_prior: %s %d: weight %d is %g (must be finite and >= 0)", what, e, i, we[i]); return AAR_ERR_INVALID; }
+                nonzero |= we[i] != 0;
+            }
+            if (!nonzero) continue;
+            const double *Te = T ? T + 16 * (size_t)e : nullptr;
+            bool finite = Te != nullptr;
+            for (int k = 0; k < 12 && finite; k++) finite = std::isfinite(Te[k]);
+            if (!finite) { set_err("aar_set_prior: %s %d has a nonzero weight and a %s target", what, e, Te ? "non-finite" : "missing"); return AAR_ERR_INVALID; }
+            double *dst; uint8_t *has;
+            if (!slot(e, dst, has)) continue;
+            double R[9];
+            for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) R[i * 3 + j] = Te[i * 4 + j];
+            aar_host::rotation_to_vector(R, dst);
+            for (int i = 0; i < 3; i++) dst[3 + i] = Te[i * 4 + 3];
+            for (int i = 0; i < 6; i++) dst[6 + i] = we[i];
+            *has = 1; any = true;
+        }
+        return AAR_OK;
+    };
+    int rc;
+    if ((rc = take("camera", p->C, cam_T, cam_w, [&](int i, double *&d, uint8_t *&h) {
+        if (!p->opt_c || i == p->root_cam) return false;
+        const int b = i - (i > p->root_cam ? 1 : 0); d = &blk[(size_t)b * PRIOR_STRIDE]; h = &blk_has[(size_t)b]; return true; }))) return rc;
+    if ((rc = take("marker", p->M, marker_T, marker_w, [&](int j, double *&d, uint8_t *&h) {
+        if (!p->opt_m || j == p->root_marker) return false;
+        const int b = p->nrc + j - (j > p->root_marker ? 1 : 0); d = &blk[(size_t)b * PRIOR_STRIDE]; h = &blk_has[(size_t)b]; return true; }))) return rc;
+    bool any_frame = false;      // on any rank: every rank of a sharded handle launches the same kernels
+    if ((rc = take("frame", p->F, frame_T, frame_w, [&](int k, double *&d, uint8_t *&h) {
+        if (!p->opt_f) return false;
+        any_frame = true;
+        if (k < p->f_begin || k >= p->f_end) return false;
+        d = &fr[(size_t)(k - p->f_begin) * PRIOR_STRIDE]; h = &fr_has[(size_t)(k - p->f_begin)]; return true; }))) return rc;
+    any |= any_frame;
+    CU(cudaSetDevice(p->device));
+    if (any) {
+        if (!p->d_blk_prior.p) {     // allocated once: the captured graph keeps the pointers
+            CU(p->d_blk_prior.alloc(blk.size())); CU(p->d_frame_prior.alloc(fr.size()));
+            CU(p->d_blk_has_prior.alloc(blk_has.size())); CU(p->d_frame_has_prior.alloc(fr_has.size()));
+        }
+        CU(cudaMemcpyAsync(p->d_blk_prior.p, blk.data(), blk.size() * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_frame_prior.p, fr.data(), fr.size() * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_blk_has_prior.p, blk_has.data(), blk_has.size(), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_frame_has_prior.p, fr_has.data(), fr_has.size(), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaStreamSynchronize(p->stream));
+    }
+    if (any != p->has_prior) drop_lm_graph(p);   // the graph-resident loop gains or loses k_prior_add / k_prior_cost
+    p->has_prior = any;
     return AAR_OK;
 }
 

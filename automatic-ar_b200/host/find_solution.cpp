@@ -2,6 +2,7 @@
 //   find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>]
 //                 [-consensus-max <k>] [-init <initial.solution>] [-analytic] [-reject-outliers <px>]
 //                 [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]
+//                 [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>]
 // Reads <folder>/<cam>/calib.yml and <folder>/aruco.detections, builds the starting point with the Initializer (device: IPPE per
 // detection + consensus; include/aar_init.h), writes initial<suffix>.solution(.yaml), solves on the GPU (include/aar_cuda.h) and
 // writes final<suffix>.solution(.yaml) — the file names of find_solution.cpp:76-100.  Two additions: -consensus-max (SURVEY 8(f) row 3,
@@ -9,7 +10,10 @@
 // instead of the detections) and -analytic (analytic Jacobian, residuals in double: include/aar_analytic.h; not the reference's arithmetic),
 // -reject-outliers <px> (after the solve, remove the detections whose reprojection error is above px and solve again with the same settings;
 // the final file holds the second solve), -fix-cams / -fix-markers / -fix-frames (hold those poses as they are in both solves, e.g. the
-// calibrated cameras of a rig that gains one: MultiCamMapper::set_fixed_*).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
+// calibrated cameras of a rig that gains one: MultiCamMapper::set_fixed_*), -prior-cams / -prior-markers (the soft form: the camera
+// (marker) poses of an earlier calibration are priors with standard deviations sigma_rot in radians and sigma_t in translation units,
+// for the ids both problems hold, in both solves: MultiCamMapper::set_*_priors; the file's root camera (marker) must be the problem's,
+// since the poses are relative to it).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -21,14 +25,16 @@
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]" << std::endl;
+        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...] [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>]" << std::endl;
         return -1;
     }
     const std::string folder = argv[1];
     const double marker_size = std::stod(argv[2]);
     bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
     std::set<int> excluded_cams, fix_cams, fix_markers, fix_frames; std::string init_path;
-    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF } flag = NONE;
+    struct PriorFile { std::string path; double sigma_rot = 0, sigma_t = 0; } prior_cams, prior_markers;
+    PriorFile *prior = nullptr; int prior_arg = 0;             // the -prior-* option being read and how many of its 3 arguments were read
+    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF, PRIOR } flag = NONE;
     for (int i = 3; i < argc; i++) {
         const std::string a = argv[i];
         if (a == "-subseqs") { use_subseqs = true; flag = NONE; }
@@ -42,6 +48,11 @@ int main(int argc, char **argv) {
         else if (a == "-fix-cams") flag = FIXC;
         else if (a == "-fix-markers") flag = FIXM;
         else if (a == "-fix-frames") flag = FIXF;
+        else if (a == "-prior-cams" || a == "-prior-markers") { flag = PRIOR; prior = a == "-prior-cams" ? &prior_cams : &prior_markers; prior_arg = 0; }
+        else if (flag == PRIOR) {
+            if (prior_arg == 0) prior->path = a; else if (prior_arg == 1) prior->sigma_rot = std::stod(a); else prior->sigma_t = std::stod(a);
+            if (++prior_arg == 3) flag = NONE;
+        }
         else if (flag == EXCLUDE) excluded_cams.insert(std::stoi(a));
         else if (flag == FIXC) fix_cams.insert(std::stoi(a));
         else if (flag == FIXM) fix_markers.insert(std::stoi(a));
@@ -89,6 +100,23 @@ int main(int argc, char **argv) {
         if (with_huber) mcm.set_with_huber(true);
         if (analytic) mcm.set_analytic_jacobian(true);
         mcm.set_fixed_cams(fix_cams); mcm.set_fixed_markers(fix_markers); mcm.set_fixed_frames(fix_frames);
+        for (int k = 0; k < 2; k++) {                             // -prior-cams, -prior-markers
+            const PriorFile &pf = k ? prior_markers : prior_cams;
+            if (pf.path.empty()) continue;
+            aar::MultiCamMapper ref;
+            if (!ref.read_solution_file(pf.path)) return 1;
+            const size_t root = k ? ref.get_root_marker() : ref.get_root_cam(), want = k ? mcm.get_root_marker() : mcm.get_root_cam();
+            if (root != want) {
+                std::cerr << "find_solution: the root " << (k ? "marker" : "camera") << " of " << pf.path << " is " << root << ", the problem's is " << want
+                          << ": its poses are relative to another root" << std::endl;
+                return 1;
+            }
+            const std::map<int, aar::Mat44> &from = k ? ref.transforms_to_root_marker : ref.transforms_to_root_cam, &held = k ? mcm.transforms_to_root_marker : mcm.transforms_to_root_cam;
+            std::map<int, aar::MultiCamMapper::PosePrior> priors;
+            for (auto &e : from) if (held.count(e.first)) priors[e.first] = aar::MultiCamMapper::PosePrior{e.second, pf.sigma_rot, pf.sigma_t};
+            if (k) mcm.set_marker_priors(priors); else mcm.set_cam_priors(priors);
+            std::cout << "priors on " << priors.size() << (k ? " markers" : " cameras") << std::endl;
+        }
         auto start = std::chrono::system_clock::now();
         mcm.solve();
         d += std::chrono::system_clock::now() - start;

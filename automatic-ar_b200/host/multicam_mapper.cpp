@@ -228,6 +228,17 @@ void MultiCamMapper::set_fixed_cams(const std::set<int> &ids) { check_ids(ids, t
 void MultiCamMapper::set_fixed_markers(const std::set<int> &ids) { check_ids(ids, transforms_to_root_marker, "markers"); fixed_markers = ids; }
 void MultiCamMapper::set_fixed_frames(const std::set<int> &ids) { check_ids(ids, object_to_global, "frames"); fixed_frames = ids; }
 
+static void check_priors(const std::map<int, MultiCamMapper::PosePrior> &priors, const std::map<int, Mat44> &held, const char *what) {
+    for (auto &p : priors) {
+        const std::string name = std::string("set_") + what + "_priors: ";
+        if (!held.count(p.first)) throw std::invalid_argument(name + "no " + what + " with id " + std::to_string(p.first));
+        if (!(p.second.sigma_rot > 0) || !(p.second.sigma_t > 0)) throw std::invalid_argument(name + "sigma of id " + std::to_string(p.first) + " is not > 0");
+    }
+}
+void MultiCamMapper::set_cam_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, transforms_to_root_cam, "cam"); cam_priors = priors; }
+void MultiCamMapper::set_marker_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, transforms_to_root_marker, "marker"); marker_priors = priors; }
+void MultiCamMapper::set_frame_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, object_to_global, "frame"); frame_priors = priors; }
+
 void MultiCamMapper::solve() {
     if (!handle) make_handle(corners_undistorted);
     {   // aar_set_fixed: one byte per camera / marker / frame in id order; NULL for an empty set, all NULL clears
@@ -238,6 +249,26 @@ void MultiCamMapper::solve() {
         };
         const std::vector<uint8_t> c = mask(fixed_cams, transforms_to_root_cam), m = mask(fixed_markers, transforms_to_root_marker), f = mask(fixed_frames, object_to_global);
         check(aar_set_fixed(handle, c.empty() ? nullptr : c.data(), m.empty() ? nullptr : m.data(), f.empty() ? nullptr : f.data()), "aar_set_fixed");
+    }
+    {   // aar_set_prior: targets [n][16] and weights 1 / sigma^2 [n][6] in id order (0 where an entity has no prior); NULL for an empty map
+        struct Arrays { std::vector<double> T, w; const double *t() const { return w.empty() ? nullptr : T.data(); } const double *wp() const { return w.empty() ? nullptr : w.data(); } };
+        auto arrays = [](const std::map<int, PosePrior> &priors, const std::map<int, Mat44> &held) {
+            Arrays a; if (priors.empty()) return a;
+            a.T.assign(16 * held.size(), 0.0); a.w.assign(6 * held.size(), 0.0);
+            size_t i = 0;
+            for (auto &p : held) {
+                auto it = priors.find(p.first);
+                if (it != priors.end()) {
+                    std::memcpy(&a.T[16 * i], it->second.T.m, sizeof it->second.T.m);
+                    const double wr = 1.0 / (it->second.sigma_rot * it->second.sigma_rot), wt = 1.0 / (it->second.sigma_t * it->second.sigma_t);
+                    for (int k = 0; k < 3; k++) { a.w[6 * i + k] = wr; a.w[6 * i + 3 + k] = wt; }
+                }
+                i++;
+            }
+            return a;
+        };
+        const Arrays c = arrays(cam_priors, transforms_to_root_cam), m = arrays(marker_priors, transforms_to_root_marker), f = arrays(frame_priors, object_to_global);
+        check(aar_set_prior(handle, c.t(), c.wp(), m.t(), m.wp(), f.t(), f.wp()), "aar_set_prior");
     }
     io_vec.assign((size_t)aar_num_vars(handle), 0.0);
     check(aar_mats2evec(handle, io_vec.data()), "aar_mats2evec");
@@ -333,7 +364,7 @@ long long MultiCamMapper::remove_outliers(double max_px, Rejection *out) {
     for (auto f = object_to_global.begin(); f != object_to_global.end();) {
         if (left.count(f->first)) { ++f; continue; }
         rj.dropped_frames.push_back(f->first);
-        fixed_frames.erase(f->first);
+        fixed_frames.erase(f->first); frame_priors.erase(f->first);
         frame_cam_markers.erase(f->first); raw_frame_cam_markers.erase(f->first);
         f = object_to_global.erase(f);
     }

@@ -80,6 +80,14 @@ public:
     void set_fixed_cams(const std::set<int> &ids);
     void set_fixed_markers(const std::set<int> &ids);
     void set_fixed_frames(const std::set<int> &ids);
+    // not in the reference: soft pose priors in solve() (aar_set_prior, include/aar_cuda.h): the pose T is known to sigma_rot (radians,
+    // per rotation-vector component) and sigma_t (the solution's translation units); weights 1 / sigma^2, sigma = inf: no prior on that
+    // part.  The maps replace the earlier ones and persist across handles (remove_outliers drops the frames it removes); track() ignores
+    // them.  An id the mapper does not hold, or a sigma that is not > 0, throws std::invalid_argument.
+    struct PosePrior { Mat44 T; double sigma_rot, sigma_t; };
+    void set_cam_priors(const std::map<int, PosePrior> &priors);
+    void set_marker_priors(const std::map<int, PosePrior> &priors);
+    void set_frame_priors(const std::map<int, PosePrior> &priors);
     void track();     // multicam_mapper.cpp:430-443: per-frame 6-dof solve against the fixed rig, every frame of the object at once
 
     bool write_solution_file(const std::string &path);         // byte-exact .solution (multicam_mapper.cpp:1053-1099)
@@ -119,6 +127,7 @@ private:
 
     Config config;
     std::set<int> fixed_cams, fixed_markers, fixed_frames;
+    std::map<int, PosePrior> cam_priors, marker_priors, frame_priors;
     bool with_huber = false, corners_undistorted = false, analytic_jacobian = false;
     size_t root_cam = 0, root_marker = 0;
     double marker_size = 0;

@@ -24,7 +24,7 @@ NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a",
 # declared by include/aar_cuda.h — tests check that the library exports every one of them
 EXPORTS = ["aar_lm_default_params", "aar_problem_create", "aar_problem_destroy", "aar_last_error", "aar_num_vars",
            "aar_num_observations", "aar_num_local_observations", "aar_jacobian_nnz", "aar_index_maps", "aar_get_observations",
-           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_lm_solve",
+           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_set_prior", "aar_lm_solve",
            "aar_lm_begin", "aar_lm_iterate", "aar_lm_end", "aar_track_batch", "aar_track_upload", "aar_track_run", "aar_track_download", "aar_track_ms", "aar_shard_plan", "aar_row_map", "aar_comm_unique_id", "aar_comm_init",
            "aar_kernel_launches", "aar_set_profiling", "aar_get_phase_ms", "aar_problem_stats"]
 
@@ -255,6 +255,24 @@ class Problem:
             keep.append(np.ascontiguousarray(a != 0, dtype=np.uint8))
             return _vp(keep[-1])
         _chk(lib().aar_set_fixed(self.h, mask(cams, self.nC, "cams"), mask(markers, self.nM, "markers"), mask(frames, self.nF, "frames")), "aar_set_fixed")
+
+    def set_prior(self, cams=None, markers=None, frames=None):
+        """aar_set_prior: soft pose priors in the later solves and reduced systems of this handle.  Each argument is a pair (T [n, 4, 4]
+        targets, w [n, 6] information weights 1/sigma^2 of [r0 r1 r2 t0 t1 t2], 0 = none) by index of the description; None = no prior
+        of that kind; all None clears."""
+        keep = []
+
+        def pair(tw, n, what):
+            if tw is None:
+                return None, None
+            T, w = tw
+            T = np.ascontiguousarray(T, dtype=np.float64); w = np.ascontiguousarray(w, dtype=np.float64)
+            if T.shape != (n, 4, 4) or w.shape != (n, 6):
+                raise ValueError(f"set_prior: {what} needs T [{n}, 4, 4] and w [{n}, 6], got {T.shape} and {w.shape}")
+            keep.extend((T, w))
+            return _vp(T), _vp(w)
+        args = [*pair(cams, self.nC, "cams"), *pair(markers, self.nM, "markers"), *pair(frames, self.nF, "frames")]
+        _chk(lib().aar_set_prior(self.h, *args), "aar_set_prior")
 
     @staticmethod
     def default_params(**kw):

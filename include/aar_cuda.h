@@ -156,7 +156,8 @@ int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out)
 int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t *rowidx, double *vals);
 /* frame-eliminated normal equations of this rank's shard at z for damping mu (parity hook of the
  * Schur stage): S [n_r*n_r] row-major, UPPER block triangle valid, WITHOUT mu on its diagonal;
- * b [n_r]; cost = sum of squared residuals of the shard.  n_r = 6 (cameras - 1) + 6 (markers - 1) of the optimised groups; with
+ * b [n_r]; cost = sum of squared residuals of the shard.  With priors (aar_set_prior) S, b and cost are those of the augmented
+ * problem: the camera / marker terms on rank 0, the frame terms on the rank that holds the frame.  n_r = 6 (cameras - 1) + 6 (markers - 1) of the optimised groups; with
  * optimize_cam_intrinsics 12 more per camera, in the internal order [fx cx fy cy k1 k2 | p1 p2 k3 . . .] (csrc/aar_intrinsics.cuh). */
 int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, double *b, double *cost);
 
@@ -167,6 +168,20 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
  * Residuals and cost are unchanged; aar_eval_jacobian, aar_error_report and aar_track_* ignore the mask.  AAR_ERR_INVALID between
  * aar_lm_begin and aar_lm_end, and for a mask that leaves no free column. */
 int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed);
+
+/* Not in the reference.  Soft priors: six residual rows sqrt(w) (z_e - zbar_e) per entity in every later solve / aar_reduced_system of
+ * this handle; zbar_e from the 4x4 target by the R -> r of aar_mats2evec.  T: [n][16] row-major like desc->cam_T; w: [n][6] information
+ * weights (1/sigma^2) of [r0 r1 r2 t0 t1 t2], >= 0 and finite, 0 = none; w == NULL: no prior of that kind; all NULL clears.  Indexed by
+ * rank of id; frames global like aar_set_fixed.  Root / non-optimised entities are ignored.  AAR_ERR_INVALID between aar_lm_begin and
+ * aar_lm_end, for a negative or non-finite weight, and for a non-finite target of an entity with a nonzero weight.
+ * The cost the solver reports and compares (aar_lm_report, the trace, aar_reduced_system) includes sum w (z - zbar)^2; the stop rule
+ * still divides by the 8 N reprojection rows.  mu0 = tau max diag(J^T J) is taken over the augmented diagonal, so a weight far above
+ * the reprojection diagonal slows the first iterations: for a hard constraint use aar_set_fixed, which also wins over a prior on the
+ * same entity (its prior residual stays in the cost as a constant).  The rotation difference is taken component by component in
+ * rotation-vector space (to first order the geodesic error near the target; no wrap near |r| = pi).  aar_eval_residual,
+ * aar_eval_jacobian, aar_error_report and aar_track_* ignore priors. */
+int aar_set_prior(aar_problem *p, const double *cam_T, const double *cam_w, const double *marker_T, const double *marker_w,
+                  const double *frame_T, const double *frame_w);
 
 /* MultiCamMapper::solve() = SparseLevMarq::solve(z, f, J) (multicam_mapper.cpp:419-428,
  * sparselevmarq.h:439-472): z is in/out like io_vec; the loop is device resident. */
