@@ -29,6 +29,7 @@
 #include "aar_report.cuh"
 #include "aar_fixed.cuh"
 #include "aar_prior.cuh"
+#include "aar_pair_prior.cuh"
 
 using namespace aar;
 
@@ -142,6 +143,8 @@ struct aar_problem {
     // aar_set_prior (aar_prior.cuh): [zbar 6 | w 6] and a has-prior byte per reduced pose block and per local frame; without priors
     // nothing is launched
     bool has_prior = false; DevBuf<double> d_blk_prior, d_frame_prior; DevBuf<uint8_t> d_blk_has_prior, d_frame_has_prior;
+    // aar_set_pair_prior (aar_pair_prior.cuh): one record per stored camera or marker pair; without pairs nothing is launched
+    int n_pair = 0; DevBuf<PairPriorRec> d_pair_prior;
     cudaEvent_t ev[16] = {}; double phase_ms[AAR_NUM_PHASES] = {};
 };
 
@@ -240,13 +243,24 @@ void prior_add(aar_problem *p) {
            p->d_frame_has_prior.p, p->dp.col_frame0, p->n_r, p->d_z.p, p->d_Hrr.p, p->d_gr.p, p->d_Hf.p);
 }
 
+// Relative-pose priors (aar_pair_prior.cuh): pairs of cameras or markers only, so rank 0 alone adds them, like the camera and marker
+// priors; the all-reduces count them once.
+int pair_count(const aar_problem *p) { return p->rank == 0 ? p->n_pair : 0; }
+
+// J^T J and J^T r of the pair rows at d_z into Hrr / gr; nothing without pairs
+void pair_prior_add(aar_problem *p) {
+    if (!pair_count(p)) return;
+    LAUNCH(p, k_pair_prior_add, cdiv(pair_count(p), PP_WARPS), PP_WARPS * 32, 0, pair_count(p), p->d_pair_prior.p, p->n_r, p->d_z.p, p->d_Hrr.p, p->d_gr.p);
+}
+
 // the cost the solver compares at dz into d_red3[0] (zeroed by the caller): the reprojection sum of residual(), then the priors'
-// sum w (z - zbar)^2.  The reprojection hooks (aar_eval_residual, aar_error_report) call residual() alone.
+// sum w (z - zbar)^2 and the pair rows' squared sum.  The reprojection hooks (aar_eval_residual, aar_error_report) call residual() alone.
 int solver_cost(aar_problem *p, const double *dz, float huber_delta) {
     if (int rc = residual(p, dz, huber_delta, nullptr)) return rc;
     if (p->has_prior && prior_grid(p))
         LAUNCH(p, k_prior_cost, prior_grid(p), 256, 0, prior_blocks(p), p->d_blk_prior.p, p->d_blk_has_prior.p, p->dp.F, p->d_frame_prior.p,
                p->d_frame_has_prior.p, p->dp.col_frame0, dz, p->d_red3.p);
+    if (pair_count(p)) LAUNCH(p, k_pair_prior_cost, cdiv(pair_count(p), 256), 256, 0, pair_count(p), p->d_pair_prior.p, dz, p->d_red3.p);
     return AAR_OK;
 }
 
@@ -385,6 +399,7 @@ int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = fal
         CU(cudaMemsetAsync(p->d_flag.p + 1, 0, sizeof(int), p->stream));
     }
     prior_add(p);
+    pair_prior_add(p);
     hold_fixed(p);      // after the priors: a held entity's columns are zero in the whole augmented Jacobian
     return AAR_OK;
 }
@@ -1654,6 +1669,57 @@ int aar_set_prior(aar_problem *p, const double *cam_T, const double *cam_w, cons
     }
     if (any != p->has_prior) drop_lm_graph(p);   // the graph-resident loop gains or loses k_prior_add / k_prior_cost
     p->has_prior = any;
+    return AAR_OK;
+}
+int aar_set_pair_prior(aar_problem *p, int32_t num_cam_pairs, const int32_t *cam_pairs, const double *cam_T, const double *cam_w,
+                       int32_t num_marker_pairs, const int32_t *marker_pairs, const double *marker_T, const double *marker_w) {
+    if (!p) return AAR_ERR_INVALID;
+    if (p->lm_active) { set_err("aar_set_pair_prior between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
+    std::vector<PairPriorRec> recs;
+    // every pair is checked; then a pair is kept when a side has columns and a weight is nonzero (the others add nothing)
+    auto take = [&](const char *what, int count, int n, const int32_t *pairs, const double *T, const double *w, auto col) -> int {
+        if (n < 0) { set_err("aar_set_pair_prior: %d %s pairs", n, what); return AAR_ERR_INVALID; }
+        if (n > 0 && (!pairs || !T || !w)) { set_err("aar_set_pair_prior: %d %s pairs and a NULL array", n, what); return AAR_ERR_INVALID; }
+        for (int k = 0; k < n; k++) {
+            const int a = pairs[2 * (size_t)k], b = pairs[2 * (size_t)k + 1];
+            if (a < 0 || a >= count || b < 0 || b >= count) { set_err("aar_set_pair_prior: %s pair %d (%d, %d): index out of range [0, %d)", what, k, a, b, count); return AAR_ERR_INVALID; }
+            if (a == b) { set_err("aar_set_pair_prior: %s pair %d joins %s %d with itself", what, k, what, a); return AAR_ERR_INVALID; }
+            const double *we = w + 2 * (size_t)k, *Te = T + 16 * (size_t)k;
+            for (int i = 0; i < 2; i++)
+                if (!(std::isfinite(we[i]) && we[i] >= 0)) { set_err("aar_set_pair_prior: %s pair %d: weight %d is %g (must be finite and >= 0)", what, k, i, we[i]); return AAR_ERR_INVALID; }
+            if (we[0] == 0 && we[1] == 0) continue;
+            for (int i = 0; i < 12; i++)
+                if (!std::isfinite(Te[i])) { set_err("aar_set_pair_prior: %s pair %d has a nonzero weight and a non-finite target", what, k); return AAR_ERR_INVALID; }
+            double R[9], orth = 0;
+            for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) R[i * 3 + j] = Te[i * 4 + j];
+            for (int i = 0; i < 3; i++)
+                for (int j = 0; j < 3; j++) orth = std::max(orth, std::fabs(R[i] * R[j] + R[3 + i] * R[3 + j] + R[6 + i] * R[6 + j] - (i == j ? 1.0 : 0.0)));
+            const double det = R[0] * (R[4] * R[8] - R[5] * R[7]) - R[1] * (R[3] * R[8] - R[5] * R[6]) + R[2] * (R[3] * R[7] - R[4] * R[6]);
+            if (!(orth <= 1e-9) || !(det > 0)) { set_err("aar_set_pair_prior: %s pair %d: the target rotation is not a rotation (|R^T R - I| = %g, det R = %g)", what, k, orth, det); return AAR_ERR_INVALID; }
+            PairPriorRec r;
+            r.col_a = (int)col(a); r.col_b = (int)col(b);
+            if (r.col_a < 0 && r.col_b < 0) continue;
+            std::memcpy(r.R, R, sizeof R);
+            for (int i = 0; i < 3; i++) r.t[i] = Te[i * 4 + 3];
+            r.w_rot = we[0]; r.w_t = we[1];
+            recs.push_back(r);
+        }
+        return AAR_OK;
+    };
+    int rc;
+    if ((rc = take("camera", p->C, num_cam_pairs, cam_pairs, cam_T, cam_w, [&](int i) { return col_cam(p, i); }))) return rc;
+    if ((rc = take("marker", p->M, num_marker_pairs, marker_pairs, marker_T, marker_w, [&](int j) { return col_marker(p, j); }))) return rc;
+    CU(cudaSetDevice(p->device));
+    const int n = (int)recs.size();
+    if (n != p->n_pair) {        // the graph-resident loop gains or loses the pair kernels, or their grids change: capture it again
+        drop_lm_graph(p);
+        CU(p->d_pair_prior.alloc(recs.size()));
+        p->n_pair = n;
+    }
+    if (n) {                     // same count: the captured graph keeps the pointer and reads the new values
+        CU(cudaMemcpyAsync(p->d_pair_prior.p, recs.data(), recs.size() * sizeof(PairPriorRec), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaStreamSynchronize(p->stream));
+    }
     return AAR_OK;
 }
 

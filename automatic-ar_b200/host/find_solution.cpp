@@ -3,6 +3,7 @@
 //                 [-consensus-max <k>] [-init <initial.solution>] [-analytic] [-reject-outliers <px>]
 //                 [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]
 //                 [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>]
+//                 [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>]
 // Reads <folder>/<cam>/calib.yml and <folder>/aruco.detections, builds the starting point with the Initializer (device: IPPE per
 // detection + consensus; include/aar_init.h), writes initial<suffix>.solution(.yaml), solves on the GPU (include/aar_cuda.h) and
 // writes final<suffix>.solution(.yaml) — the file names of find_solution.cpp:76-100.  Two additions: -consensus-max (SURVEY 8(f) row 3,
@@ -13,7 +14,11 @@
 // calibrated cameras of a rig that gains one: MultiCamMapper::set_fixed_*), -prior-cams / -prior-markers (the soft form: the camera
 // (marker) poses of an earlier calibration are priors with standard deviations sigma_rot in radians and sigma_t in translation units,
 // for the ids both problems hold, in both solves: MultiCamMapper::set_*_priors; the file's root camera (marker) must be the problem's,
-// since the poses are relative to it).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
+// since the poses are relative to it), -stereo-prior (the relative poses of a stereo-calibration file, MultiCamMapper::read_stereo_calib,
+// are relative-pose priors: for every pair of camera ids i < j that the file and the problem both hold, transforms[i][j] is taken as
+// T_ij = T_i^-1 T_j (j's coordinates into i's) with standard deviations sigma_rot in radians of relative rotation and sigma_t, in both
+// solves: MultiCamMapper::set_cam_pair_priors; the file's root camera is ignored, relative poses do not depend on it; combines with
+// -prior-cams).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -25,15 +30,15 @@
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...] [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>]" << std::endl;
+        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...] [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>] [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>]" << std::endl;
         return -1;
     }
     const std::string folder = argv[1];
     const double marker_size = std::stod(argv[2]);
     bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
     std::set<int> excluded_cams, fix_cams, fix_markers, fix_frames; std::string init_path;
-    struct PriorFile { std::string path; double sigma_rot = 0, sigma_t = 0; } prior_cams, prior_markers;
-    PriorFile *prior = nullptr; int prior_arg = 0;             // the -prior-* option being read and how many of its 3 arguments were read
+    struct PriorFile { std::string path; double sigma_rot = 0, sigma_t = 0; } prior_cams, prior_markers, stereo_prior;
+    PriorFile *prior = nullptr; int prior_arg = 0;             // the -prior-* / -stereo-prior option being read and how many of its 3 arguments were read
     enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF, PRIOR } flag = NONE;
     for (int i = 3; i < argc; i++) {
         const std::string a = argv[i];
@@ -49,6 +54,7 @@ int main(int argc, char **argv) {
         else if (a == "-fix-markers") flag = FIXM;
         else if (a == "-fix-frames") flag = FIXF;
         else if (a == "-prior-cams" || a == "-prior-markers") { flag = PRIOR; prior = a == "-prior-cams" ? &prior_cams : &prior_markers; prior_arg = 0; }
+        else if (a == "-stereo-prior") { flag = PRIOR; prior = &stereo_prior; prior_arg = 0; }
         else if (flag == PRIOR) {
             if (prior_arg == 0) prior->path = a; else if (prior_arg == 1) prior->sigma_rot = std::stod(a); else prior->sigma_t = std::stod(a);
             if (++prior_arg == 3) flag = NONE;
@@ -116,6 +122,19 @@ int main(int argc, char **argv) {
             for (auto &e : from) if (held.count(e.first)) priors[e.first] = aar::MultiCamMapper::PosePrior{e.second, pf.sigma_rot, pf.sigma_t};
             if (k) mcm.set_marker_priors(priors); else mcm.set_cam_priors(priors);
             std::cout << "priors on " << priors.size() << (k ? " markers" : " cameras") << std::endl;
+        }
+        if (!stereo_prior.path.empty()) {                         // -stereo-prior
+            std::map<int, std::map<int, aar::Mat44>> tr;
+            aar::MultiCamMapper::read_stereo_calib(stereo_prior.path, tr);
+            std::map<std::pair<int, int>, aar::MultiCamMapper::PairPrior> pairs;
+            for (auto &a : tr) {
+                if (!mcm.transforms_to_root_cam.count(a.first)) continue;
+                for (auto &b : a.second)
+                    if (a.first < b.first && mcm.transforms_to_root_cam.count(b.first))
+                        pairs[{a.first, b.first}] = aar::MultiCamMapper::PairPrior{b.second, stereo_prior.sigma_rot, stereo_prior.sigma_t};
+            }
+            mcm.set_cam_pair_priors(pairs);
+            std::cout << "pair priors on " << pairs.size() << " camera pairs" << std::endl;
         }
         auto start = std::chrono::system_clock::now();
         mcm.solve();

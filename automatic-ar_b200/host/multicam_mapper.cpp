@@ -239,6 +239,18 @@ void MultiCamMapper::set_cam_priors(const std::map<int, PosePrior> &priors) { ch
 void MultiCamMapper::set_marker_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, transforms_to_root_marker, "marker"); marker_priors = priors; }
 void MultiCamMapper::set_frame_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, object_to_global, "frame"); frame_priors = priors; }
 
+static void check_pair_priors(const std::map<std::pair<int, int>, MultiCamMapper::PairPrior> &priors, const std::map<int, Mat44> &held, const char *what) {
+    for (auto &p : priors) {
+        const std::string name = std::string("set_") + what + "_pair_priors: ", ids = "(" + std::to_string(p.first.first) + ", " + std::to_string(p.first.second) + ")";
+        for (int id : {p.first.first, p.first.second})
+            if (!held.count(id)) throw std::invalid_argument(name + "no " + what + " with id " + std::to_string(id));
+        if (p.first.first == p.first.second) throw std::invalid_argument(name + "pair " + ids + " joins a " + what + " with itself");
+        if (!(p.second.sigma_rot > 0) || !(p.second.sigma_t > 0)) throw std::invalid_argument(name + "sigma of pair " + ids + " is not > 0");
+    }
+}
+void MultiCamMapper::set_cam_pair_priors(const std::map<std::pair<int, int>, PairPrior> &priors) { check_pair_priors(priors, transforms_to_root_cam, "cam"); cam_pair_priors = priors; }
+void MultiCamMapper::set_marker_pair_priors(const std::map<std::pair<int, int>, PairPrior> &priors) { check_pair_priors(priors, transforms_to_root_marker, "marker"); marker_pair_priors = priors; }
+
 void MultiCamMapper::solve() {
     if (!handle) make_handle(corners_undistorted);
     {   // aar_set_fixed: one byte per camera / marker / frame in id order; NULL for an empty set, all NULL clears
@@ -269,6 +281,22 @@ void MultiCamMapper::solve() {
         };
         const Arrays c = arrays(cam_priors, transforms_to_root_cam), m = arrays(marker_priors, transforms_to_root_marker), f = arrays(frame_priors, object_to_global);
         check(aar_set_prior(handle, c.t(), c.wp(), m.t(), m.wp(), f.t(), f.wp()), "aar_set_prior");
+    }
+    {   // aar_set_pair_prior: index pairs [n][2] (ranks of the ids), targets [n][16], weights 1 / sigma^2 [n][2] in map order
+        struct Arrays { std::vector<int32_t> ab; std::vector<double> T, w; };
+        auto arrays = [](const std::map<std::pair<int, int>, PairPrior> &priors, const std::map<int, Mat44> &held) {
+            Arrays a;
+            auto rank = [&](int id) { return (int32_t)std::distance(held.begin(), held.find(id)); };
+            for (auto &p : priors) {
+                a.ab.push_back(rank(p.first.first)); a.ab.push_back(rank(p.first.second));
+                a.T.insert(a.T.end(), p.second.T.m, p.second.T.m + 16);
+                a.w.push_back(1.0 / (p.second.sigma_rot * p.second.sigma_rot)); a.w.push_back(1.0 / (p.second.sigma_t * p.second.sigma_t));
+            }
+            return a;
+        };
+        const Arrays c = arrays(cam_pair_priors, transforms_to_root_cam), m = arrays(marker_pair_priors, transforms_to_root_marker);
+        check(aar_set_pair_prior(handle, (int32_t)cam_pair_priors.size(), c.ab.data(), c.T.data(), c.w.data(),
+                                 (int32_t)marker_pair_priors.size(), m.ab.data(), m.T.data(), m.w.data()), "aar_set_pair_prior");
     }
     io_vec.assign((size_t)aar_num_vars(handle), 0.0);
     check(aar_mats2evec(handle, io_vec.data()), "aar_mats2evec");

@@ -88,6 +88,14 @@ public:
     void set_cam_priors(const std::map<int, PosePrior> &priors);
     void set_marker_priors(const std::map<int, PosePrior> &priors);
     void set_frame_priors(const std::map<int, PosePrior> &priors);
+    // not in the reference: soft relative-pose priors between two cameras or two markers in solve() (aar_set_pair_prior,
+    // include/aar_cuda.h), keyed by the ids (a, b): T is T_ab = T_a^-1 T_b (b's coordinates into a's, e.g. a stereo pair's
+    // calibration), known to sigma_rot (radians of relative rotation) and sigma_t (translation units); weights 1 / sigma^2,
+    // sigma = inf: no prior on that part.  The maps replace the earlier ones and persist across handles; every solve() passes them to
+    // its handle; track() ignores them.  An id the mapper does not hold, a == b, or a sigma that is not > 0 throws std::invalid_argument.
+    struct PairPrior { Mat44 T; double sigma_rot, sigma_t; };
+    void set_cam_pair_priors(const std::map<std::pair<int, int>, PairPrior> &priors);
+    void set_marker_pair_priors(const std::map<std::pair<int, int>, PairPrior> &priors);
     void track();     // multicam_mapper.cpp:430-443: per-frame 6-dof solve against the fixed rig, every frame of the object at once
 
     bool write_solution_file(const std::string &path);         // byte-exact .solution (multicam_mapper.cpp:1053-1099)
@@ -128,6 +136,7 @@ private:
     Config config;
     std::set<int> fixed_cams, fixed_markers, fixed_frames;
     std::map<int, PosePrior> cam_priors, marker_priors, frame_priors;
+    std::map<std::pair<int, int>, PairPrior> cam_pair_priors, marker_pair_priors;
     bool with_huber = false, corners_undistorted = false, analytic_jacobian = false;
     size_t root_cam = 0, root_marker = 0;
     double marker_size = 0;

@@ -24,7 +24,7 @@ NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a",
 # declared by include/aar_cuda.h — tests check that the library exports every one of them
 EXPORTS = ["aar_lm_default_params", "aar_problem_create", "aar_problem_destroy", "aar_last_error", "aar_num_vars",
            "aar_num_observations", "aar_num_local_observations", "aar_jacobian_nnz", "aar_index_maps", "aar_get_observations",
-           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_set_prior", "aar_lm_solve",
+           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_set_prior", "aar_set_pair_prior", "aar_lm_solve",
            "aar_lm_begin", "aar_lm_iterate", "aar_lm_end", "aar_track_batch", "aar_track_upload", "aar_track_run", "aar_track_download", "aar_track_ms", "aar_shard_plan", "aar_row_map", "aar_comm_unique_id", "aar_comm_init",
            "aar_kernel_launches", "aar_set_profiling", "aar_get_phase_ms", "aar_problem_stats"]
 
@@ -273,6 +273,25 @@ class Problem:
             return _vp(T), _vp(w)
         args = [*pair(cams, self.nC, "cams"), *pair(markers, self.nM, "markers"), *pair(frames, self.nF, "frames")]
         _chk(lib().aar_set_prior(self.h, *args), "aar_set_prior")
+
+    def set_pair_prior(self, cams=None, markers=None):
+        """aar_set_pair_prior: soft relative-pose priors between two cameras or two markers in the later solves and reduced systems of
+        this handle.  Each argument is a triple (pairs [n, 2] indices (a, b) of the description, T [n, 4, 4] targets of
+        T_ab = T_a^-1 T_b, w [n, 2] weights w_rot = 1/sigma_rot^2, w_t = 1/sigma_t^2); None = no pairs of that kind; both None clears."""
+        keep = []
+
+        def triple(ptw, what):
+            if ptw is None:
+                return 0, None, None, None
+            P, T, w = ptw
+            P = np.ascontiguousarray(P, dtype=np.int32); T = np.ascontiguousarray(T, dtype=np.float64); w = np.ascontiguousarray(w, dtype=np.float64)
+            n = len(P)
+            if P.shape != (n, 2) or T.shape != (n, 4, 4) or w.shape != (n, 2):
+                raise ValueError(f"set_pair_prior: {what} needs pairs [n, 2], T [n, 4, 4] and w [n, 2], got {P.shape}, {T.shape} and {w.shape}")
+            keep.extend((P, T, w))
+            return n, _vp(P), _vp(T), _vp(w)
+        args = [*triple(cams, "cams"), *triple(markers, "markers")]
+        _chk(lib().aar_set_pair_prior(self.h, *args), "aar_set_pair_prior")
 
     @staticmethod
     def default_params(**kw):

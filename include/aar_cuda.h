@@ -7,7 +7,9 @@
  * (libs/sparselevmarq.h:80, 118).  This header is what a binding of that seam looks like:
  * plain pointers and sizes, opaque handle, int status codes, no exceptions, no C++ / torch types.
  * Every entry point cites the reference interface it replaces.  INTEGRATION.md shows the
- * reference-side stub.
+ * reference-side stub.  Entry points marked "Not in the reference" extend the solve: held poses
+ * (aar_set_fixed), soft pose priors (aar_set_prior) and soft relative-pose priors between two
+ * cameras or two markers (aar_set_pair_prior).
  *
  * Conventions
  *   - all matrices are row-major 4x4 doubles (cv::Mat CV_64F as the reference holds them);
@@ -156,8 +158,8 @@ int aar_error_report(aar_problem *p, const double *z, aar_error_report_out *out)
 int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t *rowidx, double *vals);
 /* frame-eliminated normal equations of this rank's shard at z for damping mu (parity hook of the
  * Schur stage): S [n_r*n_r] row-major, UPPER block triangle valid, WITHOUT mu on its diagonal;
- * b [n_r]; cost = sum of squared residuals of the shard.  With priors (aar_set_prior) S, b and cost are those of the augmented
- * problem: the camera / marker terms on rank 0, the frame terms on the rank that holds the frame.  n_r = 6 (cameras - 1) + 6 (markers - 1) of the optimised groups; with
+ * b [n_r]; cost = sum of squared residuals of the shard.  With priors (aar_set_prior, aar_set_pair_prior) S, b and cost are those of
+ * the augmented problem: the camera / marker and pair terms on rank 0, the frame terms on the rank that holds the frame.  n_r = 6 (cameras - 1) + 6 (markers - 1) of the optimised groups; with
  * optimize_cam_intrinsics 12 more per camera, in the internal order [fx cx fy cy k1 k2 | p1 p2 k3 . . .] (csrc/aar_intrinsics.cuh). */
 int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, double *b, double *cost);
 
@@ -182,6 +184,24 @@ int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marke
  * aar_eval_jacobian, aar_error_report and aar_track_* ignore priors. */
 int aar_set_prior(aar_problem *p, const double *cam_T, const double *cam_w, const double *marker_T, const double *marker_w,
                   const double *frame_T, const double *frame_w);
+
+/* Not in the reference.  Soft relative-pose priors between two cameras or two markers (e.g. a stereo pair calibrated on its own, two
+ * markers on one rigid board): 12 residual rows per pair in every later solve / aar_reduced_system of this handle.  With T_x the
+ * pose the solve optimises (camera -> root camera, marker -> root marker) the pair (a, b) measures T_ab = T_a^-1 T_b (b's coordinates
+ * into a's, the direction of desc->cam_T), R_ab = R_a^T R_b, t_ab = R_a^T (t_b - t_a); the rows are sqrt(w_rot / 2) vec(R_ab - Rbar)
+ * and sqrt(w_t) (t_ab - tbar), their squared sum w_rot (2 - 2 cos theta) + w_t |t_ab - tbar|^2 (theta: the angle of Rbar^T R_ab;
+ * w_rot = 1 / sigma_rot^2 with sigma_rot in radians, w_t = 1 / sigma_t^2).  *_pairs: [n][2] indices (ranks of ids); *_T: [n][16]
+ * row-major targets T_ab; *_w: [n][2] w_rot, w_t.  Both counts 0 clears; every call replaces the earlier pairs.  A pair listed twice
+ * counts twice.  A side without columns (the root) is a constant identity pose; a pair with no columns on either side, or with both
+ * weights 0, is ignored.  AAR_ERR_INVALID between aar_lm_begin and aar_lm_end, for an index out of range, for a == b, for a negative
+ * or non-finite weight, and, for a pair with a nonzero weight, for a non-finite target or a target rotation with |Rbar^T Rbar - I| >
+ * 1e-9 or det Rbar <= 0.  Adds to aar_set_prior, with the same rules: the cost the solver reports and compares includes the pair
+ * terms, mu0 is taken over the augmented diagonal, the stop rule still divides by the 8 N reprojection rows, pair rows are never
+ * Huber-weighted, aar_set_fixed wins over a pair on a held entity, and aar_eval_residual, aar_eval_jacobian, aar_error_report and
+ * aar_track_* ignore pairs.  Changing the number of stored pairs captures the graph-resident loop again; new values alone keep it. */
+int aar_set_pair_prior(aar_problem *p,
+                       int32_t num_cam_pairs, const int32_t *cam_pairs, const double *cam_T, const double *cam_w,
+                       int32_t num_marker_pairs, const int32_t *marker_pairs, const double *marker_T, const double *marker_w);
 
 /* MultiCamMapper::solve() = SparseLevMarq::solve(z, f, J) (multicam_mapper.cpp:419-428,
  * sparselevmarq.h:439-472): z is in/out like io_vec; the loop is device resident. */
