@@ -26,6 +26,7 @@
 #include "../../include/aar_cuda.h"
 #include "aar_host_math.h"
 #include "aar_kernels.cuh"
+#include "aar_lens.cuh"
 #include "aar_report.cuh"
 #include "aar_fixed.cuh"
 #include "aar_prior.cuh"
@@ -109,6 +110,7 @@ struct aar_problem {
     DevBuf<int2> d_pair_fc; DevBuf<double> d_pair_tab; int npairs = 0;
     DevBuf<int4> d_pair_info, d_mrun_info; DevBuf<int> d_perm_fm, d_pair_cam; DevBuf<double> d_cm_rep; int nmruns = 0;     // visiting orders of the tensor-core assembly (aar_assemble.cuh)
     bool analytic = false; DevBuf<double> d_cam_an, d_mk_an, d_fr_an;                 // analytic-Jacobian / full-FP64 variant (aar_analytic.cuh)
+    bool lens = false; DevBuf<double> d_lens, d_lens_tr;                               // lens model (aar_lens.cuh): [C][9] at z / at the trial point
     DevBuf<double> d_trk_cam_inv, d_trk_Y, d_trk_z, d_trk_z0, d_trk_cost; bool trk_have_z0 = false; double track_ms = 0; long long track_runs = 0;
     DevBuf<double> d_fc, d_E, d_xinv;
     DevBuf<int> d_pair_slot_i; DevBuf<double> d_intr_tr, d_Ji;
@@ -140,6 +142,7 @@ struct aar_problem {
     DevBuf<double> d_rep_err, d_rep_sum; DevBuf<unsigned long long> d_rep_cnt, d_rep_max, d_sel; DevBuf<unsigned> d_sel_hist;
     // aar_set_fixed (aar_fixed.cuh): one byte per reduced block and per local frame; without a mask nothing is launched
     bool has_fixed = false; DevBuf<uint8_t> d_blk_fixed, d_frame_fixed;
+    std::vector<uint8_t> fixed_pose_blk, fixed_frame, fixed_intr;   // the masks of aar_set_fixed and aar_set_fixed_intrinsics (empty: none)
     // aar_set_prior (aar_prior.cuh): [zbar 6 | w 6] and a has-prior byte per reduced pose block and per local frame; without priors
     // nothing is launched
     bool has_prior = false; DevBuf<double> d_blk_prior, d_frame_prior; DevBuf<uint8_t> d_blk_has_prior, d_frame_has_prior;
@@ -223,6 +226,13 @@ int residual(aar_problem *p, const double *dz, float huber_delta, double *d_r_ou
     DevProblem dq = p->dp;
     if (unweighted) { dq.huber = 0; dq.st_dev = nullptr; }
     LAUNCH(p, k_expand_trial, cdiv((long long)p->C + p->M + p->dp.F, 128), 128, 0, p->dp, dz);
+    if (p->lens) {
+        if (p->opt_i) LAUNCH(p, k_expand_lens, cdiv(9LL * p->C, 64), 64, 0, p->dp, dz, p->d_lens_tr.p);
+        if (p->dp.N > 0)
+            LAUNCH(p, k_residual_lens, cdiv(p->dp.N, 256), 256, 0, dq, p->opt_i ? p->d_lens_tr.p : p->d_lens.p, p->d_cam_tr.p, p->d_mk_tr.p, p->d_fr_tr.p, huber_delta,
+                   d_r_out, p->d_red3.p);
+        return AAR_OK;
+    }
     if (p->opt_i) LAUNCH(p, k_expand_intr, cdiv(p->C, 64), 64, 0, p->dp, dz, p->d_intr_tr.p);
     if (p->dp.N > 0 && p->analytic)
         LAUNCH(p, k_residual_an, cdiv(p->dp.N, 256), 256, 0, dq, p->d_cam_tr.p, POSE_STRIDE, p->d_mk_tr.p, POSE_STRIDE, p->d_fr_tr.p, POSE_STRIDE, huber_delta, d_r_out, p->d_red3.p);
@@ -327,7 +337,10 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
         if (p->d_cm_rep.n < cm_n * ASM_CM_REPLICAS) CU(p->d_cm_rep.alloc(cm_n * ASM_CM_REPLICAS));
         CU(cudaMemsetAsync(p->d_cm_rep.p, 0, cm_n * ASM_CM_REPLICAS * sizeof(double), p->stream));
     }
-    if (p->analytic) {
+    if (p->lens) {
+        if constexpr (std::is_same<JT, double>::value) LAUNCH(p, k_jac_lens, cdiv(N, 128), 128, 0, p->dp, p->d_lens.p, huber_eval, Jn, p->d_Rv.p);
+        else { set_err("the analytic variant stages its rows in double"); return AAR_ERR_INVALID; }
+    } else if (p->analytic) {
         if constexpr (std::is_same<JT, double>::value) LAUNCH(p, k_jac_analytic, cdiv(N, 128), 128, 0, p->dp, huber_eval, Jn, p->d_Rv.p);
         else { set_err("the analytic variant stages its rows in double"); return AAR_ERR_INVALID; }
     } else
@@ -347,7 +360,11 @@ int launch_jacobian(aar_problem *p, float huber_eval, JT *Jn) {
         const int grid3 = (int)std::min<long long>((long long)std::max(per_sm, 1) * p->num_sms, want);
         LAUNCH(p, k3, grid3, ASM_THREADS, smem3, p->dp, pl, Jn, p->huber ? p->d_Rv.p : nullptr, p->d_W.p, p->d_Hrr.p, p->d_gr.p);
     }
-    if (p->opt_i && p->npairs > 0) {   // intrinsics columns (aar_intrinsics.cuh): one warp per (frame, camera) pair, from the same staged rows
+    if (p->lens && p->opt_i && p->npairs > 0) {   // the nine lens columns (aar_lens.cuh): one warp per (frame, camera) pair
+        if constexpr (std::is_same<JT, double>::value)
+            LAUNCH(p, k_intr_assemble_lens, cdiv(p->npairs, LENS_WARPS), 32 * LENS_WARPS, 0, p->dp, p->d_lens.p, p->d_pair_info.p, p->d_pair_cam.p, p->d_pair_slot_i.p, Jn,
+                   p->huber ? p->d_Rv.p : nullptr, p->d_W.p, p->d_Hrr.p, p->d_gr.p);
+    } else if (p->opt_i && p->npairs > 0) {   // intrinsics columns (aar_intrinsics.cuh): one warp per (frame, camera) pair, from the same staged rows
         auto k4 = k_intr_assemble<JT>;
         LAUNCH(p, k4, cdiv((long long)p->npairs * 32, 128), 128, 0, p->dp, p->d_pair_info.p, p->d_pair_cam.p, p->d_pair_slot_i.p, Jn, p->huber ? p->d_Rv.p : nullptr, s1, s2,
                p->d_W.p, p->d_Hrr.p, p->d_gr.p);
@@ -371,7 +388,8 @@ void hold_fixed(aar_problem *p) {
 int jacobian_accumulate(aar_problem *p, float huber_eval, bool defer_check = false, bool *rows64 = nullptr) {
     const long long jobs = (long long)p->C * NVAR_CAM + (long long)p->M * NVAR_RT + (long long)p->dp.F * NVAR_RT;
     LAUNCH(p, k_expand_jac, cdiv(jobs, 128), 128, 0, p->dp, p->d_z.p, p->d_flag.p);
-    if (p->opt_i) LAUNCH(p, k_expand_intr, cdiv(p->C, 64), 64, 0, p->dp, p->d_z.p, p->d_intr.p);
+    if (p->lens) { if (p->opt_i) LAUNCH(p, k_expand_lens, cdiv(9LL * p->C, 64), 64, 0, p->dp, p->d_z.p, p->d_lens.p); }
+    else if (p->opt_i) LAUNCH(p, k_expand_intr, cdiv(p->C, 64), 64, 0, p->dp, p->d_z.p, p->d_intr.p);
     if (p->analytic) LAUNCH(p, k_expand_analytic, cdiv((long long)p->C + p->M + p->dp.F, 128), 128, 0, p->dp, p->d_z.p);
     else if (p->npairs > 0) LAUNCH(p, k_pair_tab, std::max(1, std::min(p->npairs, 10 * p->num_sms)), PAIR_TAB, 0, p->dp);      // 10 CTAs of 192 threads per SM: one full wave
     const size_t N = (size_t)p->dp.N;
@@ -578,7 +596,11 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
     g_ranks_on_host = std::max(1, d->world_size);
     p->opt_i = d->optimize_cam_intrinsics != 0;
     p->analytic = d->analytic_jacobian != 0;
-    if (p->analytic && p->opt_i) { set_err("analytic_jacobian with optimize_cam_intrinsics: the intrinsics block is built for the central-difference path only"); return AAR_ERR_UNSUPPORTED; }
+    if (d->lens_model > 1) { set_err("lens_model %d: only 0 (undistorted corners, pinhole) and 1 (OpenCV's five-coefficient model on raw corners) exist", (int)d->lens_model); return AAR_ERR_UNSUPPORTED; }
+    p->lens = d->lens_model == 1;
+    if (p->lens && !p->analytic) { set_err("lens_model 1 needs analytic_jacobian = 1: the central-difference path is the reference's pinhole residual"); return AAR_ERR_UNSUPPORTED; }
+    if (p->lens && d->corners_undistorted) { set_err("lens_model 1 needs the raw corners: corners_undistorted = 1 (a .solution file) holds none"); return AAR_ERR_UNSUPPORTED; }
+    if (p->analytic && p->opt_i && !p->lens) { set_err("analytic_jacobian with optimize_cam_intrinsics: the pinhole intrinsics block is built for the central-difference path only (lens_model 1 refines intrinsics in the analytic mode)"); return AAR_ERR_UNSUPPORTED; }
     p->nrc = p->opt_c ? p->C - 1 : 0; p->nrm = p->opt_m ? p->M - 1 : 0; p->nri = p->opt_i ? 2 * p->C : 0; p->n_r = 6 * (p->nrc + p->nrm + p->nri);
     p->n_vars = p->n_r + (p->opt_f ? 6LL * p->F : 0);
     p->n_vars_ext = 6LL * (p->nrc + p->nrm) + (p->opt_f ? 6LL * p->F : 0) + (p->opt_i ? 9LL * p->C : 0);
@@ -657,6 +679,7 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
     const int nblk_r = p->nrc + p->nrm + p->nri;
     std::vector<int> slot_ptr((size_t)Fl + 1, 0), cs_cum((size_t)Fl + 1, 0), ms_cum((size_t)Fl + 1, 0), is_cnt((size_t)Fl + 1, 0), slot_c((size_t)Nl, -1), slot_m((size_t)Nl, -1), slot_i((size_t)Nl, -1);
     const bool slots_c = p->opt_f && p->opt_c, slots_m = p->opt_f && p->opt_m, slots_i = p->opt_f && p->opt_i;   // intrinsics: pseudo-block A of every camera seen, root included
+    const bool slots_ib = slots_i && p->lens;      // the lens model's block B has columns too: its slot follows A's
     const int Tf = host_threads(Nl);
     parallel_for(Fl, Tf, [&](long long f0, long long f1, int) {
         std::vector<long long> stamp((size_t)std::max(nblk_r, 1), -1);
@@ -667,7 +690,7 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
                 const int c = p->g_cam[(size_t)o], m = p->g_marker[(size_t)o];
                 if (slots_c && c != p->root_cam) { const size_t bk = (size_t)(c - (c > p->root_cam ? 1 : 0)); if (stamp[bk] != f) { stamp[bk] = f; ncs++; } }
                 if (slots_m && m != p->root_marker) { const size_t bk = (size_t)(p->nrc + m - (m > p->root_marker ? 1 : 0)); if (stamp[bk] != f) { stamp[bk] = f; nms++; } }
-                if (slots_i) { const size_t bk = (size_t)(p->nrc + p->nrm + 2 * c); if (stamp[bk] != f) { stamp[bk] = f; nis++; } }
+                if (slots_i) { const size_t bk = (size_t)(p->nrc + p->nrm + 2 * c); if (stamp[bk] != f) { stamp[bk] = f; nis += slots_ib ? 2 : 1; } }
             }
             cs_cum[(size_t)f + 1] = ncs; ms_cum[(size_t)f + 1] = nms; is_cnt[(size_t)f + 1] = nis;
         }
@@ -708,7 +731,10 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
             if (slots_i)
                 for (long long o = o0; o < o1; o++) {
                     const int bk = p->nrc + p->nrm + 2 * p->g_cam[(size_t)o];
-                    if (seen[(size_t)bk] < first) { seen[(size_t)bk] = next; slot_block[(size_t)next++] = bk; }
+                    if (seen[(size_t)bk] < first) {
+                        seen[(size_t)bk] = next; slot_block[(size_t)next++] = bk;
+                        if (slots_ib) { seen[(size_t)bk + 1] = next; slot_block[(size_t)next++] = bk + 1; }
+                    }
                     slot_i[(size_t)(o - p->o_begin)] = seen[(size_t)bk];
                 }
             for (int sl = first; sl < next; sl++) { slot_frame[(size_t)sl] = (int)f; frame_block_slot[(size_t)f * nblk_r + slot_block[(size_t)sl]] = sl; }
@@ -818,6 +844,17 @@ static int create_impl(const aar_problem_desc *d, aar_problem **out, bool host_o
 #undef UP
     CU(p->d_und_a.alloc((size_t)Nl)); CU(p->d_und_b.alloc((size_t)Nl));
     CU(p->d_cam_tab.alloc((size_t)p->C * CAM_TAB)); CU(p->d_mk_tab.alloc((size_t)p->M * MK_TAB)); CU(p->d_fr_tab.alloc((size_t)std::max(Fl, 1) * FR_TAB));
+    if (p->lens) {
+        std::vector<double> lens(9 * (size_t)p->C);
+        for (int c = 0; c < p->C; c++) {
+            const double *K = &p->cam_K[9 * (size_t)c], *dd = &p->cam_dist[5 * (size_t)c]; double *l = &lens[9 * (size_t)c];
+            l[0] = K[0]; l[1] = K[2]; l[2] = K[4]; l[3] = K[5]; for (int k = 0; k < 5; k++) l[4 + k] = dd[k];
+        }
+        CU(p->d_lens.alloc(lens.size())); CU(p->d_lens_tr.alloc(lens.size()));
+        CU(cudaMemcpyAsync(p->d_lens.p, lens.data(), lens.size() * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_lens_tr.p, lens.data(), lens.size() * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        CU(cudaStreamSynchronize(p->stream));     // `lens` leaves scope
+    }
     if (p->analytic) { CU(p->d_cam_an.alloc((size_t)p->C * CAM_AN)); CU(p->d_mk_an.alloc((size_t)p->M * RT_AN)); CU(p->d_fr_an.alloc((size_t)std::max(Fl, 1) * RT_AN)); }
     CU(p->d_cam_tr.alloc((size_t)p->C * POSE_STRIDE)); CU(p->d_mk_tr.alloc((size_t)p->M * POSE_STRIDE)); CU(p->d_fr_tr.alloc((size_t)std::max(Fl, 1) * POSE_STRIDE));
     const size_t nz = (size_t)std::max<long long>(p->n_vars, 1);
@@ -1154,15 +1191,17 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
     bool rows64 = false;
     if ((rc = jacobian_accumulate(p, p->h_st->huber_eval, false, &rows64))) return rc;
     const size_t N = (size_t)p->N;
-    std::vector<double> J64(rows64 ? JROW * N : 0), Ji(p->opt_i ? 32 * N : 0);
+    const int ni = p->lens ? 9 : 4;          // intrinsics columns with values: all nine in the lens model, fx cx fy cy in the reference's
+    std::vector<double> J64(rows64 ? JROW * N : 0), Ji(p->opt_i ? (size_t)(8 * ni) * N : 0);
     std::vector<float> J32(rows64 ? 0 : JROW * N);
     if (N > 0) {
         if (rows64) CU(cudaMemcpyAsync(J64.data(), p->d_Jn64.p, JROW * N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
         else CU(cudaMemcpyAsync(J32.data(), p->d_Jn32.p, JROW * N * sizeof(float), cudaMemcpyDeviceToHost, p->stream));
         if (p->opt_i) {     // intrinsics columns: no staged rows, recomputed from the pose and pair tables just expanded
-            if (p->d_Ji.n < 32 * N) CU(p->d_Ji.alloc(32 * N));
-            LAUNCH(p, k_intr_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, p->d_Ji.p);
-            CU(cudaMemcpyAsync(Ji.data(), p->d_Ji.p, 32 * N * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+            if (p->d_Ji.n < Ji.size()) CU(p->d_Ji.alloc(Ji.size()));
+            if (p->lens) LAUNCH(p, k_lens_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, p->d_lens.p, p->d_Ji.p);
+            else LAUNCH(p, k_intr_dump, cdiv(p->dp.N, 128), 128, 0, p->dp, p->d_Ji.p);
+            CU(cudaMemcpyAsync(Ji.data(), p->d_Ji.p, Ji.size() * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
         }
     }
     CU(cudaStreamSynchronize(p->stream));
@@ -1193,11 +1232,11 @@ int aar_eval_jacobian(aar_problem *p, const double *z, int64_t *colptr, int32_t 
     if (p->opt_c) for (int i = 0; i < p->C; i++) if (i != p->root_cam) emit(by_cam[(size_t)i], 0);
     if (p->opt_m) for (int i = 0; i < p->M; i++) if (i != p->root_marker) emit(by_marker[(size_t)i], 6);
     if (p->opt_f) for (int i = 0; i < p->F; i++) emit(by_frame[(size_t)i], 12);
-    if (p->opt_i)                                            // 9 columns per camera, root included; the distortion columns are explicit zeros (mcm.cpp:835-893)
+    if (p->opt_i)                                            // 9 columns per camera, root included; without the lens model the distortion columns are explicit zeros (mcm.cpp:835-893)
         for (int i = 0; i < p->C; i++)
             for (int d = 0; d < 9; d++) {
                 for (long long o : by_cam[(size_t)i])
-                    for (int q = 0; q < 8; q++) { rowidx[nnz] = (int32_t)(8 * o + q); vals[nnz] = d < 4 ? Ji[(size_t)o * 32 + (size_t)d * 8 + q] : 0.0; nnz++; }
+                    for (int q = 0; q < 8; q++) { rowidx[nnz] = (int32_t)(8 * o + q); vals[nnz] = d < ni ? Ji[(size_t)o * 8 * ni + (size_t)d * 8 + q] : 0.0; nnz++; }
                 colptr[++col] = nnz;
             }
     return AAR_OK;
@@ -1568,33 +1607,26 @@ int aar_problem_stats(const aar_problem *p, int64_t *out) {
     out[4] = (p->lm_graph_ok ? 2 : 0) | (p->last_cluster_solve ? 4 : 0) | (p->last_smem_acc ? 8 : 0) | (p->last_cm_rep ? 16 : 0) | ((long long)p->lm_graph_iters << 8); out[5] = p->max_slots; out[6] = p->f_begin; out[7] = p->f_end;
     return AAR_OK;
 }
-int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed) {
-    if (!p) return AAR_ERR_INVALID;
-    if (p->lm_active) { set_err("aar_set_fixed between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
-    // only flags on optimised, non-root entities count; the masks of this rank hold its own frames
+// uploads the union of the pose mask (aar_set_fixed) and the intrinsics flags (aar_set_fixed_intrinsics) for k_hold_fixed
+static int apply_fixed(aar_problem *p, std::vector<uint8_t> pose_blk, std::vector<uint8_t> frame, std::vector<uint8_t> intr) {
     const int nb = p->nrc + p->nrm + p->nri, Fl = p->dp.F;
     std::vector<uint8_t> blk((size_t)std::max(nb, 1), 0), fr((size_t)std::max(Fl, 1), 0);
-    bool any = false; long long free_blocks = p->nri;              // the intrinsics pseudo-blocks are never held fixed
-    if (p->opt_c)
-        for (int i = 0; i < p->C; i++) {
-            if (i == p->root_cam) continue;
-            const bool f = cam_fixed && cam_fixed[i];
-            blk[(size_t)(i - (i > p->root_cam ? 1 : 0))] = f; any |= f; free_blocks += !f;
-        }
-    if (p->opt_m)
-        for (int j = 0; j < p->M; j++) {
-            if (j == p->root_marker) continue;
-            const bool f = marker_fixed && marker_fixed[j];
-            blk[(size_t)(p->nrc + j - (j > p->root_marker ? 1 : 0))] = f; any |= f; free_blocks += !f;
+    bool any = false; long long free_blocks = 0;
+    for (int i = 0; i < p->nrc + p->nrm; i++) { const bool f = !pose_blk.empty() && pose_blk[(size_t)i]; blk[(size_t)i] = f; any |= f; free_blocks += !f; }
+    for (int c = 0; c < p->nri / 2; c++)
+        for (int k = 0; k < 2; k++) {
+            const bool f = !intr.empty() && ((intr[(size_t)c] >> k) & 1);
+            blk[(size_t)(p->nrc + p->nrm + 2 * c + k)] = f; any |= f;
+            free_blocks += !f && (k == 0 || p->lens);        // the reference's block B (distortion, padding) has no live column
         }
     if (p->opt_f)
         for (int k = 0; k < p->F; k++) {
-            const bool f = frame_fixed && frame_fixed[k];
+            const bool f = !frame.empty() && frame[(size_t)k];
             if (k >= p->f_begin && k < p->f_end) fr[(size_t)(k - p->f_begin)] = f;
             any |= f; free_blocks += !f;
         }
     // with every column fixed the step is 0 and the gain 0 / 0
-    if (any && free_blocks == 0) { set_err("aar_set_fixed: the mask leaves no free column to solve for"); return AAR_ERR_INVALID; }
+    if (any && free_blocks == 0) { set_err("the fixed masks leave no free column to solve for"); return AAR_ERR_INVALID; }
     CU(cudaSetDevice(p->device));
     if (any) {
         if (!p->d_blk_fixed.p) { CU(p->d_blk_fixed.alloc(blk.size())); CU(p->d_frame_fixed.alloc(fr.size())); }   // allocated once: the captured graph keeps the pointers
@@ -1604,7 +1636,32 @@ int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marke
     }
     if (any != p->has_fixed) drop_lm_graph(p);   // the body of the graph-resident loop gains or loses k_hold_fixed
     p->has_fixed = any;
+    p->fixed_pose_blk = std::move(pose_blk); p->fixed_frame = std::move(frame); p->fixed_intr = std::move(intr);
     return AAR_OK;
+}
+int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed) {
+    if (!p) return AAR_ERR_INVALID;
+    if (p->lm_active) { set_err("aar_set_fixed between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
+    // only flags on optimised, non-root entities count
+    std::vector<uint8_t> blk((size_t)(p->nrc + p->nrm), 0), fr;
+    if (p->opt_c && cam_fixed)
+        for (int i = 0; i < p->C; i++) if (i != p->root_cam) blk[(size_t)(i - (i > p->root_cam ? 1 : 0))] = cam_fixed[i] != 0;
+    if (p->opt_m && marker_fixed)
+        for (int j = 0; j < p->M; j++) if (j != p->root_marker) blk[(size_t)(p->nrc + j - (j > p->root_marker ? 1 : 0))] = marker_fixed[j] != 0;
+    if (p->opt_f && frame_fixed) fr.assign(frame_fixed, frame_fixed + p->F);
+    if (std::none_of(blk.begin(), blk.end(), [](uint8_t v) { return v != 0; })) blk.clear();
+    return apply_fixed(p, std::move(blk), std::move(fr), p->fixed_intr);
+}
+int aar_set_fixed_intrinsics(aar_problem *p, const uint8_t *cam_flags) {
+    if (!p) return AAR_ERR_INVALID;
+    if (p->lm_active) { set_err("aar_set_fixed_intrinsics between aar_lm_begin and aar_lm_end"); return AAR_ERR_INVALID; }
+    if (!p->opt_i) { set_err("aar_set_fixed_intrinsics: the handle does not optimise the intrinsics"); return AAR_ERR_INVALID; }
+    std::vector<uint8_t> intr;
+    if (cam_flags) {
+        for (int c = 0; c < p->C; c++) if (cam_flags[c] > 3) { set_err("aar_set_fixed_intrinsics: camera %d: flags %d (bit 0 holds fx cx fy cy k1 k2, bit 1 p1 p2 k3)", p->cam_ids[(size_t)c], (int)cam_flags[c]); return AAR_ERR_INVALID; }
+        intr.assign(cam_flags, cam_flags + p->C);
+    }
+    return apply_fixed(p, p->fixed_pose_blk, p->fixed_frame, std::move(intr));
 }
 int aar_set_prior(aar_problem *p, const double *cam_T, const double *cam_w, const double *marker_T, const double *marker_w,
                   const double *frame_T, const double *frame_w) {

@@ -3,7 +3,7 @@
 //                 [-consensus-max <k>] [-init <initial.solution>] [-analytic] [-reject-outliers <px>]
 //                 [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...]
 //                 [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>]
-//                 [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>]
+//                 [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>] [-refine-intrinsics] [-fix-intrinsics <cam_id> ...] [-fix-p1p2k3]
 // Reads <folder>/<cam>/calib.yml and <folder>/aruco.detections, builds the starting point with the Initializer (device: IPPE per
 // detection + consensus; include/aar_init.h), writes initial<suffix>.solution(.yaml), solves on the GPU (include/aar_cuda.h) and
 // writes final<suffix>.solution(.yaml) — the file names of find_solution.cpp:76-100.  Two additions: -consensus-max (SURVEY 8(f) row 3,
@@ -18,7 +18,11 @@
 // are relative-pose priors: for every pair of camera ids i < j that the file and the problem both hold, transforms[i][j] is taken as
 // T_ij = T_i^-1 T_j (j's coordinates into i's) with standard deviations sigma_rot in radians of relative rotation and sigma_t, in both
 // solves: MultiCamMapper::set_cam_pair_priors; the file's root camera is ignored, relative poses do not depend on it; combines with
-// -prior-cams).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
+// -prior-cams), -refine-intrinsics (refine K and the five distortion coefficients of every camera on the raw corners in both solves:
+// MultiCamMapper::set_lens_model, the lens model of the analytic mode; calib.yml's values are the start, and the written corners are
+// undistorted with the refined coefficients; needs the detections, so -init is refused), -fix-intrinsics (with -refine-intrinsics:
+// those cameras keep calib.yml's K and distortion) and -fix-p1p2k3 (with -refine-intrinsics: p1 p2 k3 of every camera stay calib.yml's,
+// for corners that cover too little of the image to observe them).  Unlike the reference (whose option loop starts at argv[4]) options are read from argv[3] on.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -30,16 +34,16 @@
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...] [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>] [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>]" << std::endl;
+        std::cout << "Usage: find_solution <path_to_data_folder> <marker_size> [-subseqs] [-exclude-cams <cam_id> ...] [-with-huber] [-thresh <t>] [-consensus-max <k>] [-init <file>] [-analytic] [-reject-outliers <px>] [-fix-cams <cam_id> ...] [-fix-markers <marker_id> ...] [-fix-frames <frame_id> ...] [-prior-cams <file.solution> <sigma_rot_rad> <sigma_t>] [-prior-markers <file.solution> <sigma_rot_rad> <sigma_t>] [-stereo-prior <stereo_calib_file> <sigma_rot_rad> <sigma_t>] [-refine-intrinsics] [-fix-intrinsics <cam_id> ...] [-fix-p1p2k3]" << std::endl;
         return -1;
     }
     const std::string folder = argv[1];
     const double marker_size = std::stod(argv[2]);
-    bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
-    std::set<int> excluded_cams, fix_cams, fix_markers, fix_frames; std::string init_path;
+    bool use_subseqs = false, with_huber = false, set_threshold = false, analytic = false, refine_intrinsics = false, fix_p1p2k3 = false; double threshold = 2.0; int consensus_max = 0; double reject_px = -1;
+    std::set<int> excluded_cams, fix_cams, fix_markers, fix_frames, fix_intrinsics; std::string init_path;
     struct PriorFile { std::string path; double sigma_rot = 0, sigma_t = 0; } prior_cams, prior_markers, stereo_prior;
     PriorFile *prior = nullptr; int prior_arg = 0;             // the -prior-* / -stereo-prior option being read and how many of its 3 arguments were read
-    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF, PRIOR } flag = NONE;
+    enum { NONE, EXCLUDE, THRESH, CMAX, INIT, REJECT, FIXC, FIXM, FIXF, FIXI, PRIOR } flag = NONE;
     for (int i = 3; i < argc; i++) {
         const std::string a = argv[i];
         if (a == "-subseqs") { use_subseqs = true; flag = NONE; }
@@ -53,6 +57,9 @@ int main(int argc, char **argv) {
         else if (a == "-fix-cams") flag = FIXC;
         else if (a == "-fix-markers") flag = FIXM;
         else if (a == "-fix-frames") flag = FIXF;
+        else if (a == "-refine-intrinsics") { refine_intrinsics = true; flag = NONE; }
+        else if (a == "-fix-intrinsics") flag = FIXI;
+        else if (a == "-fix-p1p2k3") { fix_p1p2k3 = true; flag = NONE; }
         else if (a == "-prior-cams" || a == "-prior-markers") { flag = PRIOR; prior = a == "-prior-cams" ? &prior_cams : &prior_markers; prior_arg = 0; }
         else if (a == "-stereo-prior") { flag = PRIOR; prior = &stereo_prior; prior_arg = 0; }
         else if (flag == PRIOR) {
@@ -63,10 +70,15 @@ int main(int argc, char **argv) {
         else if (flag == FIXC) fix_cams.insert(std::stoi(a));
         else if (flag == FIXM) fix_markers.insert(std::stoi(a));
         else if (flag == FIXF) fix_frames.insert(std::stoi(a));
+        else if (flag == FIXI) fix_intrinsics.insert(std::stoi(a));
         else if (flag == THRESH) { threshold = std::stod(a); flag = NONE; }
         else if (flag == CMAX) { consensus_max = std::stoi(a); flag = NONE; }
         else if (flag == INIT) { init_path = a; flag = NONE; }
         else if (flag == REJECT) { reject_px = std::stod(a); flag = NONE; }
+    }
+    if (refine_intrinsics && !init_path.empty()) {
+        std::cerr << "find_solution: -refine-intrinsics needs the raw detections; a .solution file (-init) holds undistorted corners only" << std::endl;
+        return 1;
     }
     std::string suffix;                                         // find_solution.cpp:76-100
     if (use_subseqs) suffix += "_subseqs";
@@ -105,6 +117,14 @@ int main(int argc, char **argv) {
         mcm.set_optmize_flag_cam_intrinsics(false);              // find_solution.cpp:140
         if (with_huber) mcm.set_with_huber(true);
         if (analytic) mcm.set_analytic_jacobian(true);
+        if (refine_intrinsics) {
+            mcm.set_optmize_flag_cam_intrinsics(true);
+            mcm.set_lens_model(true);
+            std::map<int, uint8_t> held;
+            if (fix_p1p2k3) for (auto &p : mcm.transforms_to_root_cam) held[p.first] = 2;
+            for (int c : fix_intrinsics) held[c] = 3;
+            mcm.set_fixed_intrinsics(held);
+        }
         mcm.set_fixed_cams(fix_cams); mcm.set_fixed_markers(fix_markers); mcm.set_fixed_frames(fix_frames);
         for (int k = 0; k < 2; k++) {                             // -prior-cams, -prior-markers
             const PriorFile &pf = k ? prior_markers : prior_cams;

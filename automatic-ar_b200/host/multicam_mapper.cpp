@@ -165,7 +165,8 @@ void MultiCamMapper::make_handle(bool undist) {
     d.cam_T = Tc.data(); d.marker_T = Tm.data(); d.frame_T = To.data(); d.cam_K = K.data(); d.cam_dist = D.data();
     d.num_detections = (int64_t)df.size(); d.det_frame = df.data(); d.det_cam = dc.data(); d.det_marker = dm.data(); d.det_xy = xy.data();
     d.optimize_cam_poses = config.optimize_cam_poses; d.optimize_marker_poses = config.optimize_marker_poses; d.optimize_object_poses = config.optimize_object_poses;
-    d.optimize_cam_intrinsics = config.optimize_cam_intrinsics; d.with_huber = with_huber; d.corners_undistorted = undist; d.analytic_jacobian = analytic_jacobian;
+    d.optimize_cam_intrinsics = config.optimize_cam_intrinsics; d.with_huber = with_huber; d.corners_undistorted = undist; d.analytic_jacobian = analytic_jacobian || lens_model;
+    d.lens_model = lens_model ? 1 : 0;
     d.J_delta = 1e-3; d.device = 0; d.world_size = 1;
     check(aar_problem_create(&d, &handle), "aar_problem_create");
 }
@@ -235,6 +236,18 @@ static void check_priors(const std::map<int, MultiCamMapper::PosePrior> &priors,
         if (!(p.second.sigma_rot > 0) || !(p.second.sigma_t > 0)) throw std::invalid_argument(name + "sigma of id " + std::to_string(p.first) + " is not > 0");
     }
 }
+void MultiCamMapper::set_lens_model(bool v) {
+    if (v && raw_frame_cam_markers.empty()) throw std::logic_error("set_lens_model: the mapper holds no raw corners (a .solution file stores undistorted ones)");
+    lens_model = v; drop_handle();
+}
+void MultiCamMapper::set_fixed_intrinsics(const std::map<int, uint8_t> &flags) {
+    for (auto &p : flags) {
+        if (!transforms_to_root_cam.count(p.first)) throw std::invalid_argument("set_fixed_intrinsics: no cams with id " + std::to_string(p.first));
+        if (p.second > 3) throw std::invalid_argument("set_fixed_intrinsics: flags " + std::to_string((int)p.second) + " of camera " + std::to_string(p.first) + " (bit 0: fx cx fy cy k1 k2, bit 1: p1 p2 k3)");
+    }
+    fixed_intrinsics = flags;
+}
+
 void MultiCamMapper::set_cam_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, transforms_to_root_cam, "cam"); cam_priors = priors; }
 void MultiCamMapper::set_marker_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, transforms_to_root_marker, "marker"); marker_priors = priors; }
 void MultiCamMapper::set_frame_priors(const std::map<int, PosePrior> &priors) { check_priors(priors, object_to_global, "frame"); frame_priors = priors; }
@@ -261,6 +274,11 @@ void MultiCamMapper::solve() {
         };
         const std::vector<uint8_t> c = mask(fixed_cams, transforms_to_root_cam), m = mask(fixed_markers, transforms_to_root_marker), f = mask(fixed_frames, object_to_global);
         check(aar_set_fixed(handle, c.empty() ? nullptr : c.data(), m.empty() ? nullptr : m.data(), f.empty() ? nullptr : f.data()), "aar_set_fixed");
+        if (config.optimize_cam_intrinsics) {                   // aar_set_fixed_intrinsics: flags per camera in id order, NULL for none
+            std::vector<uint8_t> fi;
+            if (!fixed_intrinsics.empty()) for (auto &p : transforms_to_root_cam) { auto it = fixed_intrinsics.find(p.first); fi.push_back(it == fixed_intrinsics.end() ? 0 : it->second); }
+            check(aar_set_fixed_intrinsics(handle, fi.empty() ? nullptr : fi.data()), "aar_set_fixed_intrinsics");
+        }
     }
     {   // aar_set_prior: targets [n][16] and weights 1 / sigma^2 [n][6] in id order (0 where an entity has no prior); NULL for an empty map
         struct Arrays { std::vector<double> T, w; const double *t() const { return w.empty() ? nullptr : T.data(); } const double *wp() const { return w.empty() ? nullptr : w.data(); } };
@@ -323,9 +341,20 @@ void MultiCamMapper::solve() {
         size_t vi = io_vec.size() - 9 * C;
         for (auto &p : transforms_to_root_cam) {
             CamConfig &cc = cam_configs[p.first];
-            cc.K[0] = io_vec[vi]; cc.K[2] = io_vec[vi + 1]; cc.K[4] = io_vec[vi + 2]; cc.K[5] = io_vec[vi + 3];
-            for (int k = 0; k < 5; k++) cc.dist[k] = io_vec[vi + 4 + k];
+            auto it = fixed_intrinsics.find(p.first);
+            const int held = it == fixed_intrinsics.end() ? 0 : it->second;     // held parts keep the caller's bytes
+            if (!(held & 1)) { cc.K[0] = io_vec[vi]; cc.K[2] = io_vec[vi + 1]; cc.K[4] = io_vec[vi + 2]; cc.K[5] = io_vec[vi + 3]; cc.dist[0] = io_vec[vi + 4]; cc.dist[1] = io_vec[vi + 5]; }
+            if (!(held & 2)) { cc.dist[2] = io_vec[vi + 6]; cc.dist[3] = io_vec[vi + 7]; cc.dist[4] = io_vec[vi + 8]; }
             vi += 9;
+        }
+        if (lens_model) {
+            // the undistorted copy of the corners follows the refined coefficients: a handle built from the raw corners with them
+            // runs remove_distortions again (it also serves the next solve, which starts from the refined intrinsics)
+            const std::vector<double> z = io_vec;
+            frame_cam_markers = raw_frame_cam_markers;
+            make_handle(false);
+            pull_undistorted();
+            io_vec = z;
         }
     }
 }

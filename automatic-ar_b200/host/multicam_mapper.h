@@ -54,6 +54,16 @@ public:
     void set_with_huber(bool v) { with_huber = v; drop_handle(); }
     // not in the reference: analytic Jacobian + residuals kept in double (include/aar_analytic.h, SURVEY 8(f) row 4); pose blocks only
     void set_analytic_jacobian(bool v) { analytic_jacobian = v; drop_handle(); }
+    // not in the reference: the lens model of the analytic mode (aar_problem_desc::lens_model, DESIGN.md §6g): residuals on the raw
+    // corners through OpenCV's five-coefficient projection, so that solve() with optimize_cam_intrinsics refines K and the distortion.
+    // Implies the analytic Jacobian.  Needs the raw corners of init(): after read_solution_file (undistorted corners only) it throws
+    // std::logic_error.  After a solve that refined the intrinsics, frame_cam_markers holds the raw corners undistorted with the
+    // refined coefficients, so that a written .solution is self-consistent.
+    void set_lens_model(bool v);
+    // not in the reference: hold the intrinsics of these cameras (ids) in solve() when optimize_cam_intrinsics: bit 0 holds
+    // fx cx fy cy k1 k2, bit 1 holds p1 p2 k3 (aar_set_fixed_intrinsics, include/aar_cuda.h); held values stay the caller's bytes.
+    // Replaces the earlier map; an id the mapper does not hold or a flag above 3 throws std::invalid_argument.
+    void set_fixed_intrinsics(const std::map<int, uint8_t> &flags);
     void set_config(const Config &c) { config = c; drop_handle(); }
     size_t get_num_vars(const Config &conf) const;
 
@@ -137,7 +147,8 @@ private:
     std::set<int> fixed_cams, fixed_markers, fixed_frames;
     std::map<int, PosePrior> cam_priors, marker_priors, frame_priors;
     std::map<std::pair<int, int>, PairPrior> cam_pair_priors, marker_pair_priors;
-    bool with_huber = false, corners_undistorted = false, analytic_jacobian = false;
+    std::map<int, uint8_t> fixed_intrinsics;
+    bool with_huber = false, corners_undistorted = false, analytic_jacobian = false, lens_model = false;
     size_t root_cam = 0, root_marker = 0;
     double marker_size = 0;
     aar_problem *handle = nullptr;

@@ -24,7 +24,7 @@ NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a",
 # declared by include/aar_cuda.h — tests check that the library exports every one of them
 EXPORTS = ["aar_lm_default_params", "aar_problem_create", "aar_problem_destroy", "aar_last_error", "aar_num_vars",
            "aar_num_observations", "aar_num_local_observations", "aar_jacobian_nnz", "aar_index_maps", "aar_get_observations",
-           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_set_prior", "aar_set_pair_prior", "aar_lm_solve",
+           "aar_mats2evec", "aar_evec2mats", "aar_eval_residual", "aar_error_report", "aar_eval_jacobian", "aar_reduced_system", "aar_set_fixed", "aar_set_fixed_intrinsics", "aar_set_prior", "aar_set_pair_prior", "aar_lm_solve",
            "aar_lm_begin", "aar_lm_iterate", "aar_lm_end", "aar_track_batch", "aar_track_upload", "aar_track_run", "aar_track_download", "aar_track_ms", "aar_shard_plan", "aar_row_map", "aar_comm_unique_id", "aar_comm_init",
            "aar_kernel_launches", "aar_set_profiling", "aar_get_phase_ms", "aar_problem_stats"]
 
@@ -54,7 +54,7 @@ class Desc(C.Structure):
                 ("cam_T", C.c_void_p), ("marker_T", C.c_void_p), ("frame_T", C.c_void_p), ("cam_K", C.c_void_p), ("cam_dist", C.c_void_p),
                 ("num_detections", C.c_int64), ("det_frame", C.c_void_p), ("det_cam", C.c_void_p), ("det_marker", C.c_void_p), ("det_xy", C.c_void_p),
                 ("optimize_cam_poses", C.c_uint8), ("optimize_marker_poses", C.c_uint8), ("optimize_object_poses", C.c_uint8),
-                ("optimize_cam_intrinsics", C.c_uint8), ("with_huber", C.c_uint8), ("corners_undistorted", C.c_uint8), ("analytic_jacobian", C.c_uint8), ("reserved", C.c_uint8 * 1),
+                ("optimize_cam_intrinsics", C.c_uint8), ("with_huber", C.c_uint8), ("corners_undistorted", C.c_uint8), ("analytic_jacobian", C.c_uint8), ("lens_model", C.c_uint8),
                 ("J_delta", C.c_double), ("device", C.c_int32), ("stream", C.c_void_p), ("rank", C.c_int32), ("world_size", C.c_int32)]
 
 
@@ -130,7 +130,8 @@ class Problem:
         return dict(frame_idx=of, cam_idx=oc, marker_idx=om, has_jac=oj)
 
     @staticmethod
-    def _desc(rig, use_init, cams, markers, objects, with_huber, device, stream, rank, world_size, J_delta, intrinsics=False, analytic=False):
+    def _desc(rig, use_init, cams, markers, objects, with_huber, device, stream, rank, world_size, J_delta, intrinsics=False, analytic=False, lens=False,
+              corners_undistorted=False):
         k = {}
         k["cam_ids"] = np.ascontiguousarray(rig.cam_ids, np.int32); k["marker_ids"] = np.ascontiguousarray(rig.marker_ids, np.int32)
         k["frame_ids"] = np.ascontiguousarray(rig.frame_ids, np.int32)
@@ -149,15 +150,19 @@ class Problem:
         d.det_frame, d.det_cam, d.det_marker, d.det_xy = _vp(k["det_frame"]), _vp(k["det_cam"]), _vp(k["det_marker"]), _vp(k["det_xy"])
         d.optimize_cam_poses, d.optimize_marker_poses, d.optimize_object_poses, d.optimize_cam_intrinsics = int(cams), int(markers), int(objects), int(intrinsics)
         d.with_huber = int(with_huber); d.J_delta = J_delta; d.device = device
-        d.analytic_jacobian = int(analytic)
+        d.analytic_jacobian = int(analytic); d.lens_model = int(lens); d.corners_undistorted = int(corners_undistorted)
         d.stream = C.c_void_p(stream) if stream else None
         d.rank, d.world_size = rank, world_size
         return d, k
 
     def __init__(self, rig, use_init=True, cams=True, markers=True, objects=True, with_huber=False, device=0, stream=None,
-                 rank=0, world_size=1, J_delta=0.0, intrinsics=False, analytic=False):
+                 rank=0, world_size=1, J_delta=0.0, intrinsics=False, analytic=False, lens=False, corners_undistorted=False):
+        """lens=True: the lens model of the analytic mode (aar_problem_desc::lens_model = 1): residuals on the raw corners against OpenCV's
+        five-coefficient projection; implies analytic=True.  With intrinsics=True it refines K and the distortion of every camera."""
         L = lib()
-        d, self._keep = self._desc(rig, use_init, cams, markers, objects, with_huber, device, stream, rank, world_size, J_delta, intrinsics, analytic)
+        analytic = analytic or lens
+        d, self._keep = self._desc(rig, use_init, cams, markers, objects, with_huber, device, stream, rank, world_size, J_delta, intrinsics, analytic, lens,
+                                   corners_undistorted)
         self.h = C.c_void_p()
         _chk(L.aar_problem_create(C.byref(d), C.byref(self.h)), "aar_problem_create")
         self.nC, self.nM, self.nF = d.num_cams, d.num_markers, d.num_frames
@@ -255,6 +260,16 @@ class Problem:
             keep.append(np.ascontiguousarray(a != 0, dtype=np.uint8))
             return _vp(keep[-1])
         _chk(lib().aar_set_fixed(self.h, mask(cams, self.nC, "cams"), mask(markers, self.nM, "markers"), mask(frames, self.nF, "frames")), "aar_set_fixed")
+
+    def set_fixed_intrinsics(self, flags=None):
+        """aar_set_fixed_intrinsics: per camera index, bit 0 holds [fx cx fy cy k1 k2], bit 1 holds [p1 p2 k3]; None clears."""
+        if flags is None:
+            _chk(lib().aar_set_fixed_intrinsics(self.h, None), "aar_set_fixed_intrinsics")
+            return
+        a = np.ascontiguousarray(np.asarray(flags).reshape(-1), dtype=np.uint8)
+        if len(a) != self.nC:
+            raise ValueError(f"set_fixed_intrinsics: {len(a)} entries, the description has {self.nC} cameras")
+        _chk(lib().aar_set_fixed_intrinsics(self.h, _vp(a)), "aar_set_fixed_intrinsics")
 
     def set_prior(self, cams=None, markers=None, frames=None):
         """aar_set_prior: soft pose priors in the later solves and reduced systems of this handle.  Each argument is a pair (T [n, 4, 4]

@@ -121,4 +121,89 @@ AAR_HD void aar_an_observation(const double *Ri, const double *ti, const double 
     }
 }
 
+/* sink of aar_an_observation_lens that keeps no intrinsics columns */
+struct aar_an_null_intr_sink {
+    AAR_HD void put(int, const double *, const double *) {}
+};
+
+/* The lens-model variant (aar_problem_desc::lens_model = 1): the same chain and pose columns, but the residual is taken on the RAW
+ * corner against OpenCV's projectPoints with five distortion coefficients:
+ *     x' = Xc.x / Xc.z, y' = Xc.y / Xc.z, r2 = x'^2 + y'^2, rad = 1 + ((k3 r2 + k2) r2 + k1) r2
+ *     x'' = x' rad + 2 p1 x'y' + p2 (r2 + 2 x'^2),  y'' = y' rad + p1 (r2 + 2 y'^2) + 2 p2 x'y'
+ *     p = (fx x'' + cx, fy y'' + cy)
+ *   lens            [fx cx fy cy k1 k2 p1 p2 k3] (the io_vec order of one camera's intrinsics)
+ *   raw             detected corners x0 y0 .. x3 y3, corner order as in aar_an_observation
+ *   sink.put(col, corner, jx, jy)      the 18 pose columns, as in aar_an_observation (through the 2x2 distortion Jacobian)
+ *   isink.put(corner, jx, jy)          jx[9], jy[9]: d e_x / d lens_k and d e_y / d lens_k of that corner, k in the order of `lens`
+ * With all five coefficients 0 the residual and the pose columns are those of aar_an_observation with und = raw. */
+template <class Sink, class ISink>
+AAR_HD void aar_an_observation_lens(const double *Ri, const double *ti, const double *dRc, const double *tc,
+                                    const double *Ro, const double *to, const double *dRo,
+                                    const double *Rm, const double *tm, const double *dRm,
+                                    const double *lens, double h, const float *raw,
+                                    bool act_c, bool act_m, bool act_f, double *e, Sink &sink, ISink &isink) {
+    const double fx = lens[0], cx = lens[1], fy = lens[2], cy = lens[3], k1 = lens[4], k2 = lens[5], p1 = lens[6], p2 = lens[7], k3 = lens[8];
+    double R1[9];
+    if (act_m)
+        for (int i = 0; i < 3; i++)
+            for (int j = 0; j < 3; j++) R1[i * 3 + j] = (Ri[i * 3 + 0] * Ro[0 * 3 + j] + Ri[i * 3 + 1] * Ro[1 * 3 + j]) + Ri[i * 3 + 2] * Ro[2 * 3 + j];
+    for (int i = 0; i < 4; i++) {
+        const double x = (i == 1 || i == 2) ? h : -h, y = (i < 2) ? h : -h;
+        double Xm[3], Xo[3], Xc[3];
+        for (int j = 0; j < 3; j++) Xm[j] = (Rm[j * 3 + 0] * x + Rm[j * 3 + 1] * y) + tm[j];
+        for (int j = 0; j < 3; j++) Xo[j] = ((Ro[j * 3 + 0] * Xm[0] + Ro[j * 3 + 1] * Xm[1]) + Ro[j * 3 + 2] * Xm[2]) + to[j];
+        for (int j = 0; j < 3; j++) Xc[j] = ((Ri[j * 3 + 0] * Xo[0] + Ri[j * 3 + 1] * Xo[1]) + Ri[j * 3 + 2] * Xo[2]) + ti[j];
+        const double iz = 1.0 / Xc[2], ux = Xc[0] * iz, uy = Xc[1] * iz;
+        const double r2 = ux * ux + uy * uy, xy2 = 2.0 * (ux * uy), tx = r2 + 2.0 * (ux * ux), ty = r2 + 2.0 * (uy * uy);
+        const double rad = 1.0 + ((k3 * r2 + k2) * r2 + k1) * r2;
+        const double xd = (ux * rad + p1 * xy2) + p2 * tx, yd = (uy * rad + p1 * ty) + p2 * xy2;
+        e[2 * i] = (double)raw[2 * i] - (fx * xd + cx);
+        e[2 * i + 1] = (double)raw[2 * i + 1] - (fy * yd + cy);
+        /* D = d(x'', y'') / d(x', y'), scaled by the focal lengths and 1 / Z: a displacement g of Xc moves (x', y') by
+         * iz (g0 - x' g2, g1 - y' g2) and the projection by A (g0 - x' g2, g1 - y' g2), A = diag(fx, fy) D iz */
+        const double drad = 2.0 * ((3.0 * k3 * r2 + 2.0 * k2) * r2 + k1);          /* d rad / d(r2) times 2 */
+        const double D00 = (rad + ux * ux * drad) + (2.0 * p1 * uy + 6.0 * p2 * ux);
+        const double D01 = ux * uy * drad + (2.0 * p1 * ux + 2.0 * p2 * uy);
+        const double D11 = (rad + uy * uy * drad) + (6.0 * p1 * uy + 2.0 * p2 * ux);
+        const double a = fx * iz, b = fy * iz;
+        const double A00 = a * D00, A01 = a * D01, A10 = b * D01, A11 = b * D11;
+#define AAR_AN_PUT(col, g0, g1, g2)                                                                      \
+        do { const double q0 = (g0) - ux * (g2), q1 = (g1) - uy * (g2);                                  \
+             sink.put((col), i, -(A00 * q0 + A01 * q1), -(A11 * q1 + A10 * q0)); } while (0)
+        if (act_c) {
+            const double d0 = Xo[0] - tc[0], d1 = Xo[1] - tc[1], d2 = Xo[2] - tc[2];
+            for (int k = 0; k < 3; k++) {
+                const double *D = dRc + 9 * k;
+                const double g0 = (D[0] * d0 + D[3] * d1) + D[6] * d2, g1 = (D[1] * d0 + D[4] * d1) + D[7] * d2, g2 = (D[2] * d0 + D[5] * d1) + D[8] * d2;
+                AAR_AN_PUT(k, g0, g1, g2);
+            }
+            for (int k = 0; k < 3; k++) AAR_AN_PUT(3 + k, -Ri[0 * 3 + k], -Ri[1 * 3 + k], -Ri[2 * 3 + k]);
+        }
+        if (act_m) {
+            for (int k = 0; k < 3; k++) {
+                const double *D = dRm + 9 * k;
+                const double w0 = D[0] * x + D[1] * y, w1 = D[3] * x + D[4] * y, w2 = D[6] * x + D[7] * y;
+                const double g0 = (R1[0] * w0 + R1[1] * w1) + R1[2] * w2, g1 = (R1[3] * w0 + R1[4] * w1) + R1[5] * w2, g2 = (R1[6] * w0 + R1[7] * w1) + R1[8] * w2;
+                AAR_AN_PUT(6 + k, g0, g1, g2);
+            }
+            for (int k = 0; k < 3; k++) AAR_AN_PUT(9 + k, R1[0 * 3 + k], R1[1 * 3 + k], R1[2 * 3 + k]);
+        }
+        if (act_f) {
+            for (int k = 0; k < 3; k++) {
+                const double *D = dRo + 9 * k;
+                const double w0 = (D[0] * Xm[0] + D[1] * Xm[1]) + D[2] * Xm[2], w1 = (D[3] * Xm[0] + D[4] * Xm[1]) + D[5] * Xm[2], w2 = (D[6] * Xm[0] + D[7] * Xm[1]) + D[8] * Xm[2];
+                const double g0 = (Ri[0] * w0 + Ri[1] * w1) + Ri[2] * w2, g1 = (Ri[3] * w0 + Ri[4] * w1) + Ri[5] * w2, g2 = (Ri[6] * w0 + Ri[7] * w1) + Ri[8] * w2;
+                AAR_AN_PUT(12 + k, g0, g1, g2);
+            }
+            for (int k = 0; k < 3; k++) AAR_AN_PUT(15 + k, Ri[0 * 3 + k], Ri[1 * 3 + k], Ri[2 * 3 + k]);
+        }
+#undef AAR_AN_PUT
+        /* intrinsics columns of e = raw - p: minus the derivatives of p */
+        const double r4 = r2 * r2, r6 = r4 * r2;
+        const double jx[9] = {-xd, -1.0, 0.0, 0.0, -(fx * (ux * r2)), -(fx * (ux * r4)), -(fx * xy2), -(fx * tx), -(fx * (ux * r6))};
+        const double jy[9] = {0.0, 0.0, -yd, -1.0, -(fy * (uy * r2)), -(fy * (uy * r4)), -(fy * ty), -(fy * xy2), -(fy * (uy * r6))};
+        isink.put(i, jx, jy);
+    }
+}
+
 #endif /* AAR_ANALYTIC_H */

@@ -8,8 +8,9 @@
  * plain pointers and sizes, opaque handle, int status codes, no exceptions, no C++ / torch types.
  * Every entry point cites the reference interface it replaces.  INTEGRATION.md shows the
  * reference-side stub.  Entry points marked "Not in the reference" extend the solve: held poses
- * (aar_set_fixed), soft pose priors (aar_set_prior) and soft relative-pose priors between two
- * cameras or two markers (aar_set_pair_prior).
+ * (aar_set_fixed), held intrinsics (aar_set_fixed_intrinsics), soft pose priors (aar_set_prior) and
+ * soft relative-pose priors between two cameras or two markers (aar_set_pair_prior); so does the lens
+ * model of aar_problem_desc::lens_model.
  *
  * Conventions
  *   - all matrices are row-major 4x4 doubles (cv::Mat CV_64F as the reference holds them);
@@ -61,8 +62,14 @@ typedef struct {
                                                        * no remove_distortions pass, and the Jacobian's "raw" corners are these corners too */
     uint8_t analytic_jacobian;                        /* 0: the reference's central differences on float32-rounded projections (parity path).
                                                        * 1: analytic Jacobian, residuals kept in double (include/aar_analytic.h) — NOT the reference's
-                                                       *    arithmetic; pose blocks only (with optimize_cam_intrinsics: AAR_ERR_UNSUPPORTED); track ignores it */
-    uint8_t reserved[1];
+                                                       *    arithmetic; with lens_model 0, pose blocks only (with optimize_cam_intrinsics:
+                                                       *    AAR_ERR_UNSUPPORTED); track ignores it */
+    uint8_t lens_model;                               /* Not in the reference.  0: the corners undistorted once at create with cam_dist (above).
+                                                       * 1: residual raw - projectPoints(Xc; K, k1 k2 p1 p2 k3) on the detected corners, no undistortion
+                                                       *    in the residual (aar_an_observation_lens, include/aar_analytic.h); K and dist from the
+                                                       *    iterate when optimize_cam_intrinsics (all nine columns live), else from cam_K / cam_dist.
+                                                       *    Needs analytic_jacobian = 1 and corners_undistorted = 0; other values: AAR_ERR_UNSUPPORTED.
+                                                       *    aar_eval_residual, aar_error_report and aar_eval_jacobian follow it; aar_track_* ignore it. */
     double J_delta;                                   /* multicam_mapper.h:189, 0 -> 1e-3 */
     /* placement */
     int32_t device;                                   /* CUDA device ordinal */
@@ -170,6 +177,13 @@ int aar_reduced_system(aar_problem *p, const double *z, double mu, double *S, do
  * Residuals and cost are unchanged; aar_eval_jacobian, aar_error_report and aar_track_* ignore the mask.  AAR_ERR_INVALID between
  * aar_lm_begin and aar_lm_end, and for a mask that leaves no free column. */
 int aar_set_fixed(aar_problem *p, const uint8_t *cam_fixed, const uint8_t *marker_fixed, const uint8_t *frame_fixed);
+
+/* Not in the reference.  Hold intrinsics of chosen cameras fixed in every later solve / aar_reduced_system of a handle with
+ * optimize_cam_intrinsics, like aar_set_fixed holds poses: cam_flags [num_cams] indexed by rank of id, bit 0 holds
+ * [fx cx fy cy k1 k2], bit 1 holds [p1 p2 k3]; NULL clears.  Combines with the aar_set_fixed mask.  AAR_ERR_INVALID between
+ * aar_lm_begin and aar_lm_end, without optimize_cam_intrinsics, for a flag with bits above 1, and for a combined mask that leaves no
+ * free column (without lens_model, [p1 p2 k3] is never a free column: the reference's distortion columns are explicit zeros). */
+int aar_set_fixed_intrinsics(aar_problem *p, const uint8_t *cam_flags);
 
 /* Not in the reference.  Soft priors: six residual rows sqrt(w) (z_e - zbar_e) per entity in every later solve / aar_reduced_system of
  * this handle; zbar_e from the 4x4 target by the R -> r of aar_mats2evec.  T: [n][16] row-major like desc->cam_T; w: [n][6] information
